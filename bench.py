@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the SSD gridworld step path (BASELINE.json: Harvest agent-steps/sec incl. obs).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one MapEnv.step over the whole batch of synthetic-action environments resident on a
@@ -17,6 +17,10 @@ D2H observations + rewards inside the timed region) next to a measured host-copy
 BASELINE.json configurations (Cleanup, the tiled 10-agent stress map, the strong split of 65 536 envs over the GPUs);
 `cpu_baseline` / `--impl reference` time the C port of the reference's step on the host cores, and
 `cpu_baseline.python_reference` the reference's own unmodified Python step, one process per core.
+
+`--dump-outputs DIR` writes what the last timed step returned (rank 0): DIR/obs.npy and DIR/reward.npy, float32, for a
+fixed seeded sample of the envs.  The inputs depend on the arguments only, so two builds run with the same arguments can be
+compared output for output.
 """
 import argparse
 import json
@@ -58,7 +62,27 @@ def parse_args():
     ap.add_argument("--no-sweep", action="store_true", help="skip the batch-size x view-radius sweep (BASELINE.json configs[4])")
     ap.add_argument("--sweep-steps", type=int, default=60)
     ap.add_argument("--no-chain", action="store_true", help="stream-ordered steps only (no programmatic dependent launch)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the observations and rewards of the last timed step to DIR as "
+                                                          "float32 .npy files (a fixed seeded sample of the envs, at most 64 MB)")
     return ap.parse_args()
+
+
+DUMP_ENVS = 1024        # envs in a --dump-outputs sample: 1024 x 5 agents x 15x15x3 observations are 14 MB as float32
+DUMP_BYTES = 60 << 20   # cap for larger agent counts and views
+
+
+def dump_index(num_envs, values_per_env):
+    """Sorted env rows of the --dump-outputs sample; depends on the batch shape only."""
+    import numpy as np
+    k = max(1, min(num_envs, DUMP_ENVS, DUMP_BYTES // (4 * values_per_env)))
+    return np.sort(np.random.RandomState(0).choice(num_envs, k, replace=False))
+
+
+def dump_outputs(out_dir, **arrays):
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float32))
 
 
 def workload(args):
@@ -128,7 +152,7 @@ class ClockSampler(object):
 
 
 # ---------------------------------------------------------------------------------- CPU baselines
-def cpu_port_rate(args, seconds_target, steps=None, warmup=2):
+def cpu_port_rate(args, seconds_target, steps=None, warmup=2, dump_dir=None):
     """Times oracle/ssd_oracle.c (the CPU port of the reference's step path) on the host cores on a
     bounded sample of the same workload.  Returns (agent-steps/s, cores, sample description, ms/step)."""
     import numpy as np
@@ -146,11 +170,14 @@ def cpu_port_rate(args, seconds_target, steps=None, warmup=2):
         env.step(ring[i % 16], obs_out=buf)
     n, t0 = 0, time.perf_counter()
     while True:
-        env.step(ring[n % 16], obs_out=buf)
+        _, rew = env.step(ring[n % 16], obs_out=buf)
         n += 1
         dt = time.perf_counter() - t0
         if (steps is not None and n >= steps) or (steps is None and dt >= seconds_target):
             break
+    if dump_dir:
+        idx = dump_index(B, buf[0].size + cfg.num_agents)
+        dump_outputs(dump_dir, obs=buf[idx], reward=rew[idx])
     rate = n * B * cfg.num_agents / dt
     sample = ("%d envs x %d steps of the same workload (%sEnv, %d agents, %dx%dx3 obs, uniform random actions), "
               "oracle/ssd_oracle.c, %d pthreads" % (B, n, args.game.capitalize(), cfg.num_agents, cfg.view_width, cfg.view_width, cores))
@@ -195,8 +222,8 @@ def python_reference_rate(args):
                       % (args.game.capitalize(), args.agents, args.view, args.pyref_steps, cores - 1)}
 
 
-def cpu_baseline(args, seconds_target=12.0, steps=None, warmup=2):
-    rate, cores, sample, ms = cpu_port_rate(args, seconds_target, steps=steps, warmup=warmup)
+def cpu_baseline(args, seconds_target=12.0, steps=None, warmup=2, dump_dir=None):
+    rate, cores, sample, ms = cpu_port_rate(args, seconds_target, steps=steps, warmup=warmup, dump_dir=dump_dir)
     base = {"value": rate, "unit": UNIT, "cores": cores, "kind": "port", "sample": sample}
     try:
         base["python_reference"] = python_reference_rate(args)
@@ -211,7 +238,7 @@ def run_reference(args, rank):
     own Python step, one process per core, is reported inside cpu_baseline.python_reference.  Never touches libssd_b200.so."""
     if rank != 0:
         return
-    base, ms = cpu_baseline(args, steps=args.steps, warmup=max(args.warmup, 1))
+    base, ms = cpu_baseline(args, steps=args.steps, warmup=max(args.warmup, 1), dump_dir=args.dump_outputs)
     rate = base["value"]
     line = {"impl": "reference", "metric": METRIC, "value": rate, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
             "warmup": args.warmup, "ms_per_step": ms, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
@@ -348,6 +375,9 @@ def run_ours(args, rank, world, local_rank):
         ms, ms_max = run.timed(args.steps)
         launches = env.launch_count - launches0  # kernels of the timed region: one fused step kernel per step (+ 2 per episode reset)
         n_timed = clk.mark()
+        if args.dump_outputs and rank == 0:  # now: the clocks loop below steps on in the same buffers
+            sel = torch.from_numpy(dump_index(B, run.obs[0].numel() + N)).to(dev)
+            dump_outputs(args.dump_outputs, obs=run.obs[sel].cpu().numpy(), reward=run.rew[sel].cpu().numpy())
         # K steps can be shorter than one nvidia-smi poll: keep the same kernel running for >= 1.5 s so that the clocks line
         # describes the GPU under this load (not part of any reported time)
         t_end = time.perf_counter() + 1.5

@@ -17,15 +17,19 @@ Every fixture stores the initial state, the actions, and after EVERY step the re
 grid, positions, orientations, rewards and uint8 observations (the float64 observation is
 (u8 - 128.0) / 255.0 exactly; ref_harness.obs_u8 asserts that).
 
-The two 64-env fixtures (BASELINE.json configs[1] and configs[3], SURVEY.md 8d) are "seeded tapes": instead
-of ~10 MB of incompressible uniform doubles and shuffled waste orders they store the MT19937 states of
-np.random / random right after reset(); tests/golden_util.py regenerates the tape from them (the draw
-counts per step are stored, and this script asserts that the regenerated tape equals the recorded one).
-Observations are kept every `obs_every`-th step, everything else every step.
+The Cleanup tapes (seeded=True) are "seeded tapes": instead of megabytes of incompressible uniform doubles and
+shuffled waste orders they store the MT19937 states of np.random / random right after reset();
+tests/golden_util.py regenerates the tape from them (the draw counts per step are stored, and this script
+asserts that the regenerated tape equals the recorded one).  Where an env never shuffles its waste list within
+the recorded steps, the recording does not determine the state of `random`; any state replays the same tape.
+Observations are kept every `obs_every`-th step, everything else every step.  Fixtures are LZMA-compressed
+.npz files (np.load reads them), so that each stays below 1 MB.
 """
+import io
 import os
 import random
 import sys
+import zipfile
 
 import numpy as np
 
@@ -175,7 +179,11 @@ def record(name, kind, amap, N, n_envs, steps, view=7, mode="tape", p_clean=0.0,
         keep = np.array(sorted(set(range(0, T, obs_every)) | {T - 1}), np.int32)
         out["obs_steps"], out["obs"] = keep, out["obs"][keep]
     path = os.path.join(OUT, name + ".npz")
-    np.savez_compressed(path, **out)
+    with zipfile.ZipFile(path, "w", zipfile.ZIP_LZMA) as zf:
+        for k, a in out.items():
+            buf = io.BytesIO()
+            np.lib.format.write_array(buf, np.asanyarray(a), allow_pickle=False)
+            zf.writestr(k + ".npy", buf.getvalue())
     print("%-28s %7.1f KB  %s" % (name, os.path.getsize(path) / 1024.0, events))
 
 
@@ -187,8 +195,8 @@ def main():
         _rec = record
         record = lambda name, *a, **k: _rec(name, *a, **k) if name in only else None
     record("harvest_tape", KIND_HARVEST, HARVEST_MAP, 5, 8, 150, p_fire=0.1)
-    record("cleanup_tape", KIND_CLEANUP, CLEANUP_MAP, 5, 8, 250, p_clean=0.4, p_fire=0.05)
-    record("cleanup10_tiled_tape", KIND_CLEANUP, tiled, 10, 4, 80, p_clean=0.3, p_fire=0.25, seed0=50)
+    record("cleanup_tape", KIND_CLEANUP, CLEANUP_MAP, 5, 8, 250, p_clean=0.4, p_fire=0.05, seeded=True)
+    record("cleanup10_tiled_tape", KIND_CLEANUP, tiled, 10, 4, 80, p_clean=0.3, p_fire=0.25, seed0=50, seeded=True)
     record("harvest_dense_tape", KIND_HARVEST, DENSE_MAP, 8, 6, 300, p_absent=0.1, shuffle_order=True, seed0=20)
     record("harvest_r5_tape", KIND_HARVEST, HARVEST_MAP, 5, 2, 40, view=5, p_fire=0.15, seed0=30)
     record("harvest_r10_tape", KIND_HARVEST, HARVEST_MAP, 5, 2, 40, view=10, p_fire=0.15, seed0=32)
