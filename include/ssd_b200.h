@@ -216,6 +216,21 @@ int ssd_policy_set_head(ssd_policy_t p, int units, int num_outputs, const float*
                         const float* logits_w, const float* logits_b, const float* value_w, const float* value_b);
 int ssd_policy_lstm_heads(ssd_policy_t p, const float* features, const float* h_in, const float* c_in, float* h_out, float* c_out, float* logits,
                           float* value, int8_t* actions, int64_t num_agents, uint64_t seed, uint32_t counter, void* stream);
+/* One network per agent id, as the reference's training scripts build them (a policy per 'agent-i', policy_mapping_fn
+ * mapping agent i to it): num_policies = P weight sets, 1..SSD_MAX_AGENTS.  Every weight pointer points to P consecutive
+ * arrays, each in the layout above.  Agent m = b*P + p of the [B][P][15][15][3] observation tensor (num_agents = B*P) is
+ * evaluated with weight set p; features, logits, value and actions stay agent-major ([M][...], M = B*P), and the Philox
+ * counter words of the sampler are the agent-major index m, so P copies of one weight set give exactly the outputs of the
+ * shared network.  ssd_policy_set_head_n must be given the P of ssd_policy_create_n; on a handle with P > 1,
+ * ssd_policy_features and ssd_policy_lstm_heads return SSD_ERR_INVALID unless num_agents % P == 0.
+ * The TILED recurrent state of such a handle is grouped per policy: P*G groups, G = ceil(B/128), shape [P*G][8][128][16];
+ * state group p*G + g holds policy p and envs b in [128 g, 128 g + 128): element (agent m = b*P + p, unit u) at
+ * (((p*G + b/128) * 8 + u/16) * 128 + b % 128) * 16 + u % 16.  P = 1 is the shared network (ssd_policy_create /
+ * ssd_policy_set_head are that case). */
+int ssd_policy_create_n(int view_radius, int device, int num_policies, const float* conv_w, const float* conv_b, const float* fc1_w,
+                        const float* fc1_b, const float* fc2_w, const float* fc2_b, ssd_policy_t* out);
+int ssd_policy_set_head_n(ssd_policy_t p, int num_policies, int units, int num_outputs, const float* lstm_w, const float* lstm_u,
+                          const float* lstm_b, const float* logits_w, const float* logits_b, const float* value_w, const float* value_b);
 /* The unfused alternative for other cell sizes: LSTM cell update after the gate GEMM (conv_to_fcnet_v2.py:68-80; Keras gate order i, f, c~, o; sigmoid recurrent
  * activation): gates dev bf16[num_agents][4*units] = x W + h U without the bias, bias dev f32[4*units],
  * c_prev / c_out / h_out dev f32[num_agents][units] (c_out may alias c_prev), h_bf16_out dev bf16[num_agents][units]

@@ -22,7 +22,7 @@ SYMBOLS = ("ssd_last_error", "ssd_abi_version", "ssd_create", "ssd_destroy", "ss
            "ssd_get_state", "ssd_reset", "ssd_reset_rows", "ssd_step", "ssd_rollout", "ssd_step_phases", "ssd_get_beams", "ssd_render", "ssd_render_map", "ssd_step_host",
            "ssd_set_option", "ssd_stats", "ssd_launch_count", "ssd_philox_selftest",
            "ssd_policy_create", "ssd_policy_features", "ssd_policy_destroy", "ssd_policy_lstm_cell",
-           "ssd_policy_set_head", "ssd_policy_lstm_heads")
+           "ssd_policy_set_head", "ssd_policy_lstm_heads", "ssd_policy_create_n", "ssd_policy_set_head_n")
 
 
 class SsdConfig(C.Structure):
@@ -89,6 +89,8 @@ def _load():
         "ssd_policy_lstm_cell": (i32, [vp, vp, vp, vp, vp, vp, i64, i32, vp]),
         "ssd_policy_set_head": (i32, [vp, i32, i32, vp, vp, vp, vp, vp, vp, vp]),
         "ssd_policy_lstm_heads": (i32, [vp, vp, vp, vp, vp, vp, vp, vp, vp, i64, C.c_uint64, C.c_uint32, vp]),
+        "ssd_policy_create_n": (i32, [i32, i32, i32, vp, vp, vp, vp, vp, vp, C.POINTER(vp)]),
+        "ssd_policy_set_head_n": (i32, [vp, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)

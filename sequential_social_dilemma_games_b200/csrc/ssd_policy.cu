@@ -52,7 +52,6 @@ constexpr int N1 = 80;                        // 13 * 6 = 78 conv outputs of one
 constexpr int K2 = 80, N2 = FEAT;             // one row block of Dense(32)
 constexpr int K3 = FEAT, N3 = FEAT;
 constexpr int RING = 6;                       // image-row operand blocks in flight (tensor memory)
-constexpr int WRING = 6;                      // Dense weight blocks in flight (shared memory)
 constexpr int kProducerWarps = 4, kMmaWarp = 4, kDrainWarp0 = 5, kDrainWarps = 8, kLoadWarp = kDrainWarp0 + kDrainWarps, kThreads = 32 * (kLoadWarp + 1);
 // tensor memory (512 columns x 128 lanes x 32 bit): accumulators, and the A operands -- a lane is an agent, a column two fp16
 constexpr int kTmemCols = 512;
@@ -71,17 +70,28 @@ constexpr int kB3Bytes = (K3 / 8) * N3 * 16;              // 2 048
 constexpr int kConstFloats = N1 + N2 + N3;                // cb[80], b1[32], b2[32]
 constexpr int kHeadBytes = kB1Bytes + kB3Bytes + kConstFloats * 4;   // resident part of the blob: 25 664
 constexpr int kBlobBytes = kHeadBytes + CO * kB2Bytes;    // + the 13 row blocks of Dense(32), streamed: 92 224
-constexpr int kObsStride = 86528;                         // 128 * 675 = 86 400 + slack for the padded taps of the last agent (128-byte multiple)
-constexpr int kOffObs = 0;
-constexpr int kOffB1 = 2 * kObsStride, kOffB3 = kOffB1 + kB1Bytes, kOffConst = kOffB3 + kB3Bytes;
-constexpr int kOffW1 = kOffB1 + kHeadBytes;
-constexpr int kOffBar = kOffW1 + WRING * kB2Bytes;
+constexpr int kObsSlot = 704;                             // per-agent variant: one agent's 16-byte-aligned span (<= 690 bytes) + reads past it
 enum { BAR_OBS = 0, BAR_OBS_FREE = 2, BAR_ROW_FULL = 4, BAR_D1_FREE = 10, BAR_C_FULL = 12, BAR_W1_FULL = 14, BAR_X3 = 20, BAR_D3 = 21, BAR_STEP = 22,
        BAR_COUNT = 30 };
 constexpr int STEPS = 8;                      // ring of "first block of MMA step s has completed" barriers
-constexpr int kSmemBytes = kOffBar + BAR_COUNT * 8;
-static_assert(kHeadBytes % 16 == 0 && kOffB1 % 128 == 0 && kOffW1 % 16 == 0 && kOffBar % 8 == 0, "alignment");
-static_assert(kSmemBytes <= 227 * 1024, "one CTA per SM");
+// Shared-memory layout of the two variants of the kernel.  Shared weights: a group is 128 consecutive agents, one contiguous
+// run of 86 400 bytes.  Per-agent weights: a group is 128 agents of one policy, rows P * 675 bytes apart, each gathered into
+// a 704-byte slot; the two observation buffers grow by 7 168 bytes, which the weight ring pays for with one block (6 -> 5:
+// 5 KB; the blocks come from L2 and the ring still runs five output rows ahead of their use).
+template <bool kPerAgent>
+struct TrunkSmem {
+    static constexpr int WRING = kPerAgent ? 5 : 6;         // Dense weight blocks in flight (shared memory)
+    static constexpr int kSlot = kPerAgent ? kObsSlot : IMG; // bytes from one agent's observation to the next
+    static constexpr int kObsStride = kPerAgent ? GA * kObsSlot : 86528;  // 128 * 675 = 86 400 + slack for the padded taps of the last agent
+    static constexpr int kOffObs = 0;
+    static constexpr int kOffB1 = 2 * kObsStride, kOffB3 = kOffB1 + kB1Bytes, kOffConst = kOffB3 + kB3Bytes;
+    static constexpr int kOffW1 = kOffB1 + kHeadBytes;
+    static constexpr int kOffBar = kOffW1 + WRING * kB2Bytes;
+    static constexpr int kSmemBytes = kOffBar + BAR_COUNT * 8;
+    static_assert(kHeadBytes % 16 == 0 && kOffB1 % 128 == 0 && kOffW1 % 16 == 0 && kOffBar % 8 == 0, "alignment");
+    static_assert(kSmemBytes <= 227 * 1024, "one CTA per SM");
+    static_assert(BAR_W1_FULL + WRING <= BAR_X3, "weight-ring barriers");
+};
 
 // The CTA works through its groups g = blockIdx.x, blockIdx.x + gridDim.x, ... as ONE sequence of output rows
 // T = 13 * (group ordinal) + i and image rows R = 15 * (group ordinal) + r; three roles run that sequence concurrently:
@@ -101,15 +111,29 @@ static_assert(kSmemBytes <= 227 * 1024, "one CTA per SM");
 // D2 complete -- hangs on ONE tcgen05.commit per step into a ring of eight step barriers (a commit costs the issuing
 // thread ~40 cycles, five per step were 15 % of the kernel): whoever needs "the first block of step x is complete" waits
 // barrier x % 8 on parity (x / 8) & 1; no waiter is ever more than six steps from the MMA thread, so phases cannot alias.
+//
+// kPerAgent: agent m = b * P + p of the [B, P] batch is evaluated with weight set p (blob + p * kBlobBytes).  A UMMA tile
+// cannot change its B operand per row, so CTA c serves policy c % P only -- groups g = c / P, c / P + cpp, ... of the agents
+// (b, p), b in [128 g, 128 g + 128) -- and loads that policy's resident weights once, as the shared kernel does.
+template <bool kPerAgent>
 __global__ void __launch_bounds__(kThreads, 1) policy_features_kernel(const uint8_t* __restrict__ obs, long long M, const uint8_t* __restrict__ blob,
-                                                                     float* __restrict__ out) {
+                                                                     float* __restrict__ out, int num_policies, int ctas_per_policy) {
+    using L = TrunkSmem<kPerAgent>;
+    constexpr int WRING = L::WRING, kObsStride = L::kObsStride, kOffObs = L::kOffObs, kOffB1 = L::kOffB1, kOffB3 = L::kOffB3;
+    constexpr int kOffConst = L::kOffConst, kOffW1 = L::kOffW1, kOffBar = L::kOffBar;
     extern __shared__ __align__(128) uint8_t smem[];
     __shared__ uint32_t s_tmem;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     uint64_t* bars = reinterpret_cast<uint64_t*>(smem + kOffBar);
     const float* s_const = reinterpret_cast<const float*>(smem + kOffConst);
-    const long long n_groups = (M + GA - 1) / GA;
-    const uint32_t n_my = blockIdx.x < n_groups ? static_cast<uint32_t>((n_groups - blockIdx.x + gridDim.x - 1) / gridDim.x) : 0;  // groups of this CTA
+    const int np = kPerAgent ? num_policies : 1;
+    const int pol = kPerAgent ? static_cast<int>(blockIdx.x) % np : 0;                       // this CTA's weight set
+    const long long cta = kPerAgent ? blockIdx.x / np : blockIdx.x;                          // its index among the CTAs of that policy
+    const long long stride = kPerAgent ? ctas_per_policy : gridDim.x;
+    const long long rows = kPerAgent ? M / np : M;                                           // agents per policy
+    if (kPerAgent) blob += static_cast<long long>(pol) * kBlobBytes;
+    const long long n_groups = (rows + GA - 1) / GA;
+    const uint32_t n_my = cta < n_groups ? static_cast<uint32_t>((n_groups - cta + stride - 1) / stride) : 0;  // groups of this CTA
     const uint32_t NT = n_my * CO;
 
     if (tid == 0) {
@@ -151,7 +175,9 @@ __global__ void __launch_bounds__(kThreads, 1) policy_features_kernel(const uint
         for (uint32_t gi = 0; gi < n_my; ++gi) {
             warp_wait(bars + BAR_OBS + (gi & 1), (gi >> 1) & 1);
             SSD_PT(0);
-            const uint8_t* img = smem + kOffObs + (gi & 1) * kObsStride + t * IMG;
+            const uint8_t* img = smem + kOffObs + (gi & 1) * kObsStride + t * L::kSlot;
+            if (kPerAgent)  // the slot starts at the 16-byte boundary below the agent's row (obs is 16-byte aligned)
+                img += (static_cast<uint32_t>(((cta + gi * stride) * GA + t) * np + pol) * IMG) & 15u;
 #pragma unroll 1
             for (int r = 0; r < V; ++r, ++R) {
                 const uint32_t slot = R % RING;
@@ -293,34 +319,74 @@ __global__ void __launch_bounds__(kThreads, 1) policy_features_kernel(const uint
             SSD_PT_FLUSH(1);
         }
     } else if (warp == kLoadWarp) {
-        // ------------------------------------------------------------------ loader (one elected thread): TMA bulk copies only
-        if (n_my > 0 && elect_one()) {
-            auto load_obs = [&](uint32_t gi) {  // the group's rem * 675 contiguous bytes (a group starts 16-byte aligned)
-                const long long a0 = (blockIdx.x + static_cast<long long>(gi) * gridDim.x) * GA;
-                const int rem = static_cast<int>(M - a0 < GA ? M - a0 : GA);
-                const uint8_t* src = obs + a0 * IMG;
+        // ------------------------------------------------------------------ loader: TMA bulk copies only.  Shared weights: one
+        // elected thread.  Per-agent weights: the whole warp -- a group is 128 copies, which one thread issued too slowly to keep
+        // the weight ring fed -- with lane 0 polling the barriers for the warp and issuing the weight blocks.
+        if (n_my > 0 && (kPerAgent || elect_one())) {
+            const bool lead = !kPerAgent || lane == 0;
+            auto ready = [&](uint64_t* b, uint32_t parity) {  // per-agent: lane 0's view, the same for the whole warp
+                if (!kPerAgent) return mbar_try_wait(b, parity);
+                return __shfl_sync(0xffffffffu, lane == 0 ? static_cast<int>(mbar_try_wait(b, parity)) : 0, 0) != 0;
+            };
+            auto load_obs = [&](uint32_t gi) {
+                const long long a0 = (cta + static_cast<long long>(gi) * stride) * GA;
+                const int rem = static_cast<int>(rows - a0 < GA ? rows - a0 : GA);
                 uint8_t* dst = smem + kOffObs + (gi & 1) * kObsStride;
-                const uint32_t bytes = static_cast<uint32_t>(rem) * IMG, b16 = bytes & ~15u;
-                for (uint32_t i = b16; i < bytes; ++i) dst[i] = src[i];
-                mbar_expect_tx(bars + BAR_OBS + (gi & 1), b16);
-                bulk_g2s(dst, src, b16, bars + BAR_OBS + (gi & 1));
+                uint64_t* bar = bars + BAR_OBS + (gi & 1);
+                if (!kPerAgent) {  // the group's rem * 675 contiguous bytes (a group starts 16-byte aligned)
+                    const uint8_t* src = obs + a0 * IMG;
+                    const uint32_t bytes = static_cast<uint32_t>(rem) * IMG, b16 = bytes & ~15u;
+                    for (uint32_t i = b16; i < bytes; ++i) dst[i] = src[i];
+                    mbar_expect_tx(bar, b16);
+                    bulk_g2s(dst, src, b16, bar);
+                } else {  // gather: per agent the 16-byte-aligned span around its row, into its slot; nothing past the tensor's end
+                    const long long end = M * IMG, end16 = end & ~15ll;
+                    auto span = [&](int t, long long& s0) {
+                        const long long s = ((a0 + t) * np + pol) * IMG, s1 = (s + IMG + 15) & ~15ll;
+                        s0 = s & ~15ll;
+                        return static_cast<uint32_t>((s1 < end16 ? s1 : end16) - s0);
+                    };
+                    uint32_t bytes = 0;
+                    for (int t = lane; t < rem; t += 32) {
+                        long long s0;
+                        bytes += span(t, s0);
+                        if (s0 + span(t, s0) == end16)  // the last agent of the tensor: its bytes past the last 16-byte boundary by hand
+                            for (long long i = end16; i < end; ++i) dst[t * L::kSlot + (i - s0)] = obs[i];
+                    }
+                    bytes = __reduce_add_sync(0xffffffffu, bytes);
+                    __syncwarp();
+                    if (lane == 0) mbar_expect_tx(bar, bytes);  // before any copy can complete; releases the tail bytes
+                    __syncwarp();
+                    for (int t = lane; t < rem; t += 32) {
+                        long long s0;
+                        const uint32_t n = span(t, s0);
+                        bulk_g2s(dst + t * L::kSlot, obs + s0, n, bar);
+                    }
+                }
             };
             load_obs(0);
             if (n_my > 1) load_obs(1);
             uint32_t next_obs = 2;  // next group whose bytes want a buffer: group next_obs - 2 must have been consumed
 #pragma unroll 1
-            for (uint32_t T = 0; T < NT; ++T) {  // Dense(32) weight block of output row T, six rows ahead of its use
-                const uint32_t ws = T % WRING;
-                while (T >= WRING && !mbar_try_wait(bars + BAR_STEP + (T - 4) % STEPS, ((T - 4) / STEPS) & 1)) {  // Dense partial of row T - 6
-                    if (next_obs < n_my && mbar_try_wait(bars + BAR_OBS_FREE + (next_obs & 1), ((next_obs - 2) >> 1) & 1)) load_obs(next_obs++);
+            for (uint32_t T = 0; T < NT; ++T) {  // Dense(32) weight block of output row T, WRING rows ahead of its use
+                const uint32_t ws = T % WRING, tf = T - WRING + 2;  // step tf issued the Dense partial of row T - WRING
+                while (T >= WRING && !ready(bars + BAR_STEP + tf % STEPS, (tf / STEPS) & 1)) {
+                    if (next_obs < n_my && ready(bars + BAR_OBS_FREE + (next_obs & 1), ((next_obs - 2) >> 1) & 1)) load_obs(next_obs++);
                     __nanosleep(200);
                 }
-                mbar_expect_tx(bars + BAR_W1_FULL + ws, kB2Bytes);
-                bulk_g2s(smem + kOffW1 + ws * kB2Bytes, blob + kHeadBytes + (T % CO) * kB2Bytes, kB2Bytes, bars + BAR_W1_FULL + ws);
-                if (next_obs < n_my && mbar_try_wait(bars + BAR_OBS_FREE + (next_obs & 1), ((next_obs - 2) >> 1) & 1)) load_obs(next_obs++);
+                if (lead) {
+                    mbar_expect_tx(bars + BAR_W1_FULL + ws, kB2Bytes);
+                    bulk_g2s(smem + kOffW1 + ws * kB2Bytes, blob + kHeadBytes + (T % CO) * kB2Bytes, kB2Bytes, bars + BAR_W1_FULL + ws);
+                }
+                if (next_obs < n_my && ready(bars + BAR_OBS_FREE + (next_obs & 1), ((next_obs - 2) >> 1) & 1)) load_obs(next_obs++);
             }
             while (next_obs < n_my) {
-                wait_sleep(bars + BAR_OBS_FREE + (next_obs & 1), ((next_obs - 2) >> 1) & 1);
+                if (kPerAgent) {
+                    while (!ready(bars + BAR_OBS_FREE + (next_obs & 1), ((next_obs - 2) >> 1) & 1)) {
+                    }
+                } else {
+                    wait_sleep(bars + BAR_OBS_FREE + (next_obs & 1), ((next_obs - 2) >> 1) & 1);
+                }
                 load_obs(next_obs++);
             }
         }
@@ -356,9 +422,9 @@ __global__ void __launch_bounds__(kThreads, 1) policy_features_kernel(const uint
             tmem_ld16(trow + kColD3 + 16 * half, acc);
             tmem_ld_wait();
             tc_fence_before();
-            const long long a0 = (blockIdx.x + static_cast<long long>(gi) * gridDim.x) * GA;
-            if (a0 + row < M) {
-                float4* dst = reinterpret_cast<float4*>(out + (a0 + row) * FEAT + 16 * half);
+            const long long a0 = (cta + static_cast<long long>(gi) * stride) * GA;
+            if (a0 + row < rows) {
+                float4* dst = reinterpret_cast<float4*>(out + ((a0 + row) * np + pol) * FEAT + 16 * half);
                 const float* b2 = s_const + N1 + N2 + 16 * half;
 #pragma unroll
                 for (int c = 0; c < 16; c += 4)
@@ -468,49 +534,64 @@ __global__ void __launch_bounds__(256) lstm_cell_kernel(const uint4* __restrict_
 #pragma GCC visibility push(default)
 extern "C" {
 
-int ssd_policy_create(int view_radius, int device, const float* conv_w, const float* conv_b, const float* fc1_w, const float* fc1_b,
-                      const float* fc2_w, const float* fc2_b, ssd_policy_t* out) {
+int ssd_policy_create_n(int view_radius, int device, int num_policies, const float* conv_w, const float* conv_b, const float* fc1_w,
+                        const float* fc1_b, const float* fc2_w, const float* fc2_b, ssd_policy_t* out) {
     using namespace ssd::policy;
     if (!out) return ssd::set_error(SSD_ERR_INVALID, "null argument");
     *out = nullptr;
     if (!conv_w || !conv_b || !fc1_w || !fc1_b || !fc2_w || !fc2_b) return ssd::set_error(SSD_ERR_INVALID, "null weight pointer");
+    if (num_policies < 1 || num_policies > SSD_MAX_AGENTS) return ssd::set_error(SSD_ERR_INVALID, "num_policies must be 1..SSD_MAX_AGENTS");
     if (2 * view_radius + 1 != V) return ssd::set_error(SSD_ERR_UNSUPPORTED, "the feature kernel is built for 15x15 observations (view radius 7)");
-    std::vector<uint8_t> blob(kBlobBytes, 0);
-    __half* b1 = reinterpret_cast<__half*>(blob.data());                          // resident: conv, fc2, constants
-    __half* b3 = reinterpret_cast<__half*>(blob.data() + kB1Bytes);
-    float* cst = reinterpret_cast<float*>(blob.data() + kB1Bytes + kB3Bytes);
-    __half* b2 = reinterpret_cast<__half*>(blob.data() + kHeadBytes);             // streamed: the 13 row blocks of Dense(32)
+    const size_t blob_bytes = static_cast<size_t>(num_policies) * kBlobBytes;
+    std::vector<uint8_t> blobs(blob_bytes, 0);
     auto at = [](int rows, int n, int k) { return ((k >> 3) * rows + n) * 8 + (k & 7); };  // canonical K-major, no swizzle
-    // banded conv weights: conv_w[di][dj][c][f] (Keras kernel layout) at tap k = 48 di + 3 (j + dj) + c of column n = 6 j + f
-    for (int j = 0; j < CO; ++j)
-        for (int f = 0; f < NF; ++f) {
-            double sum16 = 0.0;
-            for (int di = 0; di < 3; ++di)
-                for (int dj = 0; dj < 3; ++dj)
-                    for (int c = 0; c < 3; ++c) {
-                        const __half h = __float2half_rn(conv_w[((di * 3 + dj) * 3 + c) * NF + f]);
-                        b1[at(N1, j * NF + f, di * ROWK + (j + dj) * 3 + c)] = h;
-                        sum16 += static_cast<double>(__half2float(h));
-                    }
-            // relu(conv((x - 128) / 255) + b) with the operand holding 1024 + x
-            cst[j * NF + f] = static_cast<float>(static_cast<double>(conv_b[f]) - (1024.0 + 128.0) * sum16 / 255.0);
-        }
-    for (int i = 0; i < CO; ++i)  // Dense(32) kernel [1014][32], inputs flattened (i, j, f)
-        for (int k = 0; k < CO * NF; ++k)
-            for (int n = 0; n < N2; ++n) b2[i * (K2 * N2) + at(N2, n, k)] = __float2half_rn(fc1_w[(i * CO * NF + k) * N2 + n]);
-    for (int k = 0; k < K3; ++k)
-        for (int n = 0; n < N3; ++n) b3[at(N3, n, k)] = __float2half_rn(fc2_w[k * N3 + n]);
-    for (int n = 0; n < N2; ++n) cst[N1 + n] = fc1_b[n];
-    for (int n = 0; n < N3; ++n) cst[N1 + N2 + n] = fc2_b[n];
+    for (int q = 0; q < num_policies; ++q) {  // weight set q: arrays q of the num_policies consecutive ones behind each pointer
+        uint8_t* blob = blobs.data() + static_cast<size_t>(q) * kBlobBytes;
+        const float* cw = conv_w + q * (9 * 3 * NF);
+        const float* cbias = conv_b + q * NF;
+        const float* w1 = fc1_w + static_cast<size_t>(q) * (CO * CO * NF * N2);
+        const float* b1v = fc1_b + q * N2;
+        const float* w2 = fc2_w + q * (K3 * N3);
+        const float* b2v = fc2_b + q * N3;
+        __half* b1 = reinterpret_cast<__half*>(blob);                          // resident: conv, fc2, constants
+        __half* b3 = reinterpret_cast<__half*>(blob + kB1Bytes);
+        float* cst = reinterpret_cast<float*>(blob + kB1Bytes + kB3Bytes);
+        __half* b2 = reinterpret_cast<__half*>(blob + kHeadBytes);             // streamed: the 13 row blocks of Dense(32)
+        // banded conv weights: conv_w[di][dj][c][f] (Keras kernel layout) at tap k = 48 di + 3 (j + dj) + c of column n = 6 j + f
+        for (int j = 0; j < CO; ++j)
+            for (int f = 0; f < NF; ++f) {
+                double sum16 = 0.0;
+                for (int di = 0; di < 3; ++di)
+                    for (int dj = 0; dj < 3; ++dj)
+                        for (int c = 0; c < 3; ++c) {
+                            const __half h = __float2half_rn(cw[((di * 3 + dj) * 3 + c) * NF + f]);
+                            b1[at(N1, j * NF + f, di * ROWK + (j + dj) * 3 + c)] = h;
+                            sum16 += static_cast<double>(__half2float(h));
+                        }
+                // relu(conv((x - 128) / 255) + b) with the operand holding 1024 + x
+                cst[j * NF + f] = static_cast<float>(static_cast<double>(cbias[f]) - (1024.0 + 128.0) * sum16 / 255.0);
+            }
+        for (int i = 0; i < CO; ++i)  // Dense(32) kernel [1014][32], inputs flattened (i, j, f)
+            for (int k = 0; k < CO * NF; ++k)
+                for (int n = 0; n < N2; ++n) b2[i * (K2 * N2) + at(N2, n, k)] = __float2half_rn(w1[(i * CO * NF + k) * N2 + n]);
+        for (int k = 0; k < K3; ++k)
+            for (int n = 0; n < N3; ++n) b3[at(N3, n, k)] = __float2half_rn(w2[k * N3 + n]);
+        for (int n = 0; n < N2; ++n) cst[N1 + n] = b1v[n];
+        for (int n = 0; n < N3; ++n) cst[N1 + N2 + n] = b2v[n];
+    }
 
     SsdPolicy* p = new (std::nothrow) SsdPolicy();
     if (!p) return ssd::set_error(SSD_ERR_INVALID, "out of host memory");
     p->device = device;
+    p->num_policies = num_policies;
     cudaError_t e = cudaSetDevice(device);
     if (e == cudaSuccess) e = cudaDeviceGetAttribute(&p->sms, cudaDevAttrMultiProcessorCount, device);
-    if (e == cudaSuccess) e = cudaMalloc(&p->d_blob, kBlobBytes);
-    if (e == cudaSuccess) e = cudaMemcpy(p->d_blob, blob.data(), kBlobBytes, cudaMemcpyHostToDevice);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(policy_features_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
+    if (e == cudaSuccess) e = cudaMalloc(&p->d_blob, blob_bytes);
+    if (e == cudaSuccess) e = cudaMemcpy(p->d_blob, blobs.data(), blob_bytes, cudaMemcpyHostToDevice);
+    if (e == cudaSuccess && num_policies == 1)
+        e = cudaFuncSetAttribute(policy_features_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TrunkSmem<false>::kSmemBytes);
+    if (e == cudaSuccess && num_policies > 1)
+        e = cudaFuncSetAttribute(policy_features_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TrunkSmem<true>::kSmemBytes);
     if (e != cudaSuccess) {
         if (p->d_blob) cudaFree(p->d_blob);
         delete p;
@@ -520,16 +601,30 @@ int ssd_policy_create(int view_radius, int device, const float* conv_w, const fl
     return SSD_OK;
 }
 
+int ssd_policy_create(int view_radius, int device, const float* conv_w, const float* conv_b, const float* fc1_w, const float* fc1_b,
+                      const float* fc2_w, const float* fc2_b, ssd_policy_t* out) {
+    return ssd_policy_create_n(view_radius, device, 1, conv_w, conv_b, fc1_w, fc1_b, fc2_w, fc2_b, out);
+}
+
 int ssd_policy_features(ssd_policy_t p, const uint8_t* obs, int64_t num_agents, float* features, void* stream) {
     using namespace ssd::policy;
     if (!p || !obs || !features || num_agents < 0) return ssd::set_error(SSD_ERR_INVALID, "bad argument");
     if (reinterpret_cast<uintptr_t>(obs) % 16 != 0 || reinterpret_cast<uintptr_t>(features) % 16 != 0)
         return ssd::set_error(SSD_ERR_INVALID, "obs and features must be 16-byte aligned");
+    const int np = p->num_policies;
+    if (num_agents % np != 0) return ssd::set_error(SSD_ERR_INVALID, "num_agents must be a multiple of num_policies");
     if (num_agents == 0) return SSD_OK;
     if (cudaSetDevice(p->device) != cudaSuccess) return ssd::set_error(SSD_ERR_CUDA, "cudaSetDevice failed");  // the blob and the stream live there
-    const long long groups = (num_agents + GA - 1) / GA;
-    const int grid = static_cast<int>(groups < p->sms ? groups : p->sms);
-    policy_features_kernel<<<grid, kThreads, kSmemBytes, static_cast<cudaStream_t>(stream)>>>(obs, num_agents, p->d_blob, features);
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (np == 1) {
+        const long long groups = (num_agents + GA - 1) / GA;
+        const int grid = static_cast<int>(groups < p->sms ? groups : p->sms);
+        policy_features_kernel<false><<<grid, kThreads, TrunkSmem<false>::kSmemBytes, st>>>(obs, num_agents, p->d_blob, features, 1, grid);
+    } else {  // P * floor(#SMs / P) CTAs at most, each serving one policy
+        const long long groups = (num_agents / np + GA - 1) / GA;
+        const int per = static_cast<int>(groups < p->sms / np ? groups : p->sms / np);
+        policy_features_kernel<true><<<np * per, kThreads, TrunkSmem<true>::kSmemBytes, st>>>(obs, num_agents, p->d_blob, features, np, per);
+    }
     const cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return ssd::set_error(SSD_ERR_CUDA, cudaGetErrorString(e));
     return SSD_OK;

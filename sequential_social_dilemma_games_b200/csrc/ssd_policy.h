@@ -8,4 +8,5 @@ struct SsdPolicy {
     uint8_t* d_blob = nullptr;       // packed trunk weights
     uint8_t* d_head_blob = nullptr;  // packed LSTM / head weights (ssd_policy_set_head)
     int units = 0, num_outputs = 0;
+    int num_policies = 1;            // weight sets: agent m = b * P + p uses set p (ssd_policy_create_n)
 };

@@ -65,15 +65,26 @@ __device__ __forceinline__ float tanh_fast(float x) {
 }
 __device__ __forceinline__ float sigmoid_fast(float x) { return fmaf(tanh_fast(0.5f * x), 0.5f, 0.5f); }
 
+// kPerAgent: agent m = b * P + p uses weight set p (blob + p * kBlobBytes).  As in the trunk, CTA c serves policy c % P only
+// (groups g = c / P, c / P + cpp, ... of the agents (b, p), b in [128 g, 128 g + 128)), so its [W; U] is loaded once; features
+// are read as 128-byte rows P * 128 bytes apart, outputs are written to agent-major rows, and the recurrent state of that
+// group is state group p * ceil(B / 128) + g.  The sampler keys Philox by the agent-major index m in both variants.
+template <bool kPerAgent>
 __global__ void __launch_bounds__(kThreads, 1)
 lstm_heads_kernel(const float* __restrict__ feat, const float* h_in, const float* c_in, float* h_out, float* c_out, float* __restrict__ logits,
                   float* __restrict__ value, int8_t* __restrict__ actions, long long M, int num_outputs, const uint8_t* __restrict__ blob,
-                  uint32_t seed_lo, uint32_t seed_hi, uint32_t counter) {
+                  uint32_t seed_lo, uint32_t seed_hi, uint32_t counter, int num_policies, int ctas_per_policy) {
     extern __shared__ __align__(128) uint8_t smem[];
     __shared__ uint32_t s_tmem;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     uint64_t* bar = reinterpret_cast<uint64_t*>(smem + kOffBar);
     const float* s_bias = reinterpret_cast<const float*>(smem + kOffConst);
+    const int np = kPerAgent ? num_policies : 1;
+    const int pol = kPerAgent ? static_cast<int>(blockIdx.x) % np : 0;                       // this CTA's weight set
+    const long long cta = kPerAgent ? blockIdx.x / np : blockIdx.x;                          // its index among the CTAs of that policy
+    const long long stride = kPerAgent ? ctas_per_policy : gridDim.x;
+    const long long rows = kPerAgent ? M / np : M;                                           // agents per policy
+    if (kPerAgent) blob += static_cast<long long>(pol) * kBlobBytes;
     if (tid == 0) mbar_init(bar, 1);
     if (warp == 0) tmem_alloc(&s_tmem, 512);
     for (int i = tid; i < (kBlobBytes >> 4); i += kThreads) reinterpret_cast<uint4*>(smem)[i] = reinterpret_cast<const uint4*>(blob)[i];
@@ -86,11 +97,11 @@ lstm_heads_kernel(const float* __restrict__ feat, const float* h_in, const float
     constexpr uint32_t kIG = umma_idesc(GA, 256), kIH = umma_idesc(GA, NH);
     uint32_t parity = 0;
 
-    const long long n_groups = (M + GA - 1) / GA;
+    const long long n_groups = (rows + GA - 1) / GA;
     SSD_HT_DECL;
-    for (long long g = blockIdx.x; g < n_groups; g += gridDim.x) {
-        const long long a0 = g * GA;
-        const int rem = static_cast<int>(M - a0 < GA ? M - a0 : GA);
+    for (long long g = cta; g < n_groups; g += stride) {
+        const long long a0 = g * GA, sg = pol * n_groups + g;   // first agent row of the group in its policy; its state group
+        const int rem = static_cast<int>(rows - a0 < GA ? rows - a0 : GA);
         {   // A = fp16([features | h]).  HBM is read in long contiguous runs (features: a 128-byte row per eight lanes; h: the tiled
             // state, 64 bytes per lane, 2 KB per warp -- a thread walking a row-major row in 32-byte steps reached 2.3 TB/s).
             // All loads before the stores: the compiler keeps a global load below a store through a generic pointer.
@@ -101,11 +112,11 @@ lstm_heads_kernel(const float* __restrict__ feat, const float* h_in, const float
 #pragma unroll
             for (int ps = 0; ps < 4; ++ps) {
                 const int row = ps * 32 + r8;
-                vx[ps] = row < rem ? __ldcs(reinterpret_cast<const float4*>(feat + (a0 + row) * KX) + seg) : z;
+                vx[ps] = row < rem ? __ldcs(reinterpret_cast<const float4*>(feat + ((a0 + row) * np + pol) * KX) + seg) : z;
             }
 #pragma unroll
             for (int b = 0; b < 4; ++b) {
-                const float4* src = reinterpret_cast<const float4*>(h_in + ((g * (U / 16) + hb0 + b) * GA + hrow) * 16);
+                const float4* src = reinterpret_cast<const float4*>(h_in + ((sg * (U / 16) + hb0 + b) * GA + hrow) * 16);
 #pragma unroll
                 for (int j = 0; j < 4; ++j) vh[b][j] = hrow < rem ? __ldcs(src + j) : z;
             }
@@ -143,7 +154,7 @@ lstm_heads_kernel(const float* __restrict__ feat, const float* h_in, const float
             const int q = warp & 3, row = q * 32 + lane, uh = warp >> 2;
             const uint32_t trow = tmem + (static_cast<uint32_t>(q * 32) << 16);
             const bool live = row < rem;
-            const long long tile0 = ((g * (U / 16) + uh * 4) * GA + row) * 16;   // this agent's 16 floats of unit block 4 uh; + GA * 16 per block
+            const long long tile0 = ((sg * (U / 16) + uh * 4) * GA + row) * 16;   // this agent's 16 floats of unit block 4 uh; + GA * 16 per block
             float4 cn[4];   // the next 16 units of c, fetched one iteration ahead
 #pragma unroll
             for (int e = 0; e < 4; ++e) cn[e] = live ? __ldcs(reinterpret_cast<const float4*>(c_in + tile0) + e) : make_float4(0.f, 0.f, 0.f, 0.f);
@@ -205,7 +216,7 @@ lstm_heads_kernel(const float* __restrict__ feat, const float* h_in, const float
             tmem_ld16(tmem + (static_cast<uint32_t>(warp * 32) << 16), y);
             tmem_ld_wait();
             if (row < rem) {
-                const long long m = a0 + row;
+                const long long m = (a0 + row) * np + pol;
                 const float* hb = s_bias + NG;
                 float best = -3.0e38f;
                 int arg = 0;
@@ -226,7 +237,14 @@ lstm_heads_kernel(const float* __restrict__ feat, const float* h_in, const float
                 // y[] is indexed statically: read the value column with a select chain
                 float v = 0.f;
 #pragma unroll
-                for (int a = 0; a < NH; ++a) if (a == num_outputs) v = __uint_as_float(y[a]) + hb[a];
+                for (int a = 0; a < NH; ++a) {
+                    if (!kPerAgent) {
+                        if (a == num_outputs) v = __uint_as_float(y[a]) + hb[a];
+                    } else {  // an explicit selp: ptxas turned the chain into y[num_outputs] through a stack copy of y[] here
+                        asm("{\n\t.reg .pred q;\n\tsetp.eq.s32 q, %2, %3;\n\tselp.f32 %0, %1, %0, q;\n\t}\n"
+                            : "+f"(v) : "f"(__uint_as_float(y[a]) + hb[a]), "r"(a), "r"(num_outputs));
+                    }
+                }
                 value[m] = v;
                 if (actions != nullptr) actions[m] = static_cast<int8_t>(arg);
             }
@@ -247,36 +265,55 @@ lstm_heads_kernel(const float* __restrict__ feat, const float* h_in, const float
 #pragma GCC visibility push(default)
 extern "C" {
 
-int ssd_policy_set_head(ssd_policy_t p, int units, int num_outputs, const float* lstm_w, const float* lstm_u, const float* lstm_b,
-                        const float* logits_w, const float* logits_b, const float* value_w, const float* value_b) {
+int ssd_policy_set_head_n(ssd_policy_t p, int num_policies, int units, int num_outputs, const float* lstm_w, const float* lstm_u,
+                          const float* lstm_b, const float* logits_w, const float* logits_b, const float* value_w, const float* value_b) {
     using namespace ssd::policy_head;
     if (!p || !lstm_w || !lstm_u || !lstm_b || !logits_w || !logits_b || !value_w || !value_b) return ssd::set_error(SSD_ERR_INVALID, "null argument");
+    if (num_policies < 1 || num_policies > SSD_MAX_AGENTS) return ssd::set_error(SSD_ERR_INVALID, "num_policies must be 1..SSD_MAX_AGENTS");
+    if (num_policies != p->num_policies) return ssd::set_error(SSD_ERR_INVALID, "the head must have as many weight sets as the trunk");
     if (units != U) return ssd::set_error(SSD_ERR_UNSUPPORTED, "the fused LSTM kernel is built for cell_size 128 (conv_to_fcnet_v2.py's custom_options)");
     if (num_outputs < 1 || num_outputs > NH - 1) return ssd::set_error(SSD_ERR_UNSUPPORTED, "1..15 policy outputs");
-    std::vector<uint8_t> blob(kBlobBytes, 0);
-    __half* b = reinterpret_cast<__half*>(blob.data() + kOffB);
-    __half* bh = reinterpret_cast<__half*>(blob.data() + kOffBH);
-    float* cst = reinterpret_cast<float*>(blob.data() + kOffConst);
+    const size_t blob_bytes = static_cast<size_t>(num_policies) * kBlobBytes;
+    std::vector<uint8_t> blobs(blob_bytes, 0);
     auto at = [](int rows, int n, int k) { return ((k >> 3) * rows + n) * 8 + (k & 7); };  // canonical K-major, no swizzle
-    for (int n = 0; n < NG; ++n) {   // Keras LSTM: kernel [32][4u], recurrent kernel [u][4u], gates i, f, c~, o
-        for (int k = 0; k < KX; ++k) b[at(NG, n, k)] = __float2half_rn(lstm_w[k * NG + n]);
-        for (int k = 0; k < U; ++k) b[at(NG, n, KX + k)] = __float2half_rn(lstm_u[k * NG + n]);
-        cst[n] = lstm_b[n];
+    for (int q = 0; q < num_policies; ++q) {  // weight set q: arrays q of the num_policies consecutive ones behind each pointer
+        uint8_t* blob = blobs.data() + static_cast<size_t>(q) * kBlobBytes;
+        const float* lw = lstm_w + static_cast<size_t>(q) * KX * NG;
+        const float* lu = lstm_u + static_cast<size_t>(q) * U * NG;
+        const float* lb = lstm_b + q * NG;
+        const float* ow = logits_w + q * U * num_outputs;
+        const float* ob = logits_b + q * num_outputs;
+        const float* vw = value_w + q * U;
+        const float* vb = value_b + q;
+        __half* b = reinterpret_cast<__half*>(blob + kOffB);
+        __half* bh = reinterpret_cast<__half*>(blob + kOffBH);
+        float* cst = reinterpret_cast<float*>(blob + kOffConst);
+        for (int n = 0; n < NG; ++n) {   // Keras LSTM: kernel [32][4u], recurrent kernel [u][4u], gates i, f, c~, o
+            for (int k = 0; k < KX; ++k) b[at(NG, n, k)] = __float2half_rn(lw[k * NG + n]);
+            for (int k = 0; k < U; ++k) b[at(NG, n, KX + k)] = __float2half_rn(lu[k * NG + n]);
+            cst[n] = lb[n];
+        }
+        for (int k = 0; k < U; ++k) {
+            for (int n = 0; n < num_outputs; ++n) bh[at(NH, n, k)] = __float2half_rn(ow[k * num_outputs + n]);
+            bh[at(NH, num_outputs, k)] = __float2half_rn(vw[k]);
+        }
+        for (int n = 0; n < num_outputs; ++n) cst[NG + n] = ob[n];
+        cst[NG + num_outputs] = vb[0];
     }
-    for (int k = 0; k < U; ++k) {
-        for (int n = 0; n < num_outputs; ++n) bh[at(NH, n, k)] = __float2half_rn(logits_w[k * num_outputs + n]);
-        bh[at(NH, num_outputs, k)] = __float2half_rn(value_w[k]);
-    }
-    for (int n = 0; n < num_outputs; ++n) cst[NG + n] = logits_b[n];
-    cst[NG + num_outputs] = value_b[0];
     cudaError_t e = cudaSetDevice(p->device);
-    if (e == cudaSuccess && !p->d_head_blob) e = cudaMalloc(&p->d_head_blob, kBlobBytes);
-    if (e == cudaSuccess) e = cudaMemcpy(p->d_head_blob, blob.data(), kBlobBytes, cudaMemcpyHostToDevice);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(lstm_heads_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
+    if (e == cudaSuccess && !p->d_head_blob) e = cudaMalloc(&p->d_head_blob, blob_bytes);
+    if (e == cudaSuccess) e = cudaMemcpy(p->d_head_blob, blobs.data(), blob_bytes, cudaMemcpyHostToDevice);
+    if (e == cudaSuccess && num_policies == 1) e = cudaFuncSetAttribute(lstm_heads_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
+    if (e == cudaSuccess && num_policies > 1) e = cudaFuncSetAttribute(lstm_heads_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
     if (e != cudaSuccess) return ssd::set_error(SSD_ERR_CUDA, cudaGetErrorString(e));
     p->units = units;
     p->num_outputs = num_outputs;
     return SSD_OK;
+}
+
+int ssd_policy_set_head(ssd_policy_t p, int units, int num_outputs, const float* lstm_w, const float* lstm_u, const float* lstm_b,
+                        const float* logits_w, const float* logits_b, const float* value_w, const float* value_b) {
+    return ssd_policy_set_head_n(p, 1, units, num_outputs, lstm_w, lstm_u, lstm_b, logits_w, logits_b, value_w, value_b);
 }
 
 int ssd_policy_lstm_heads(ssd_policy_t p, const float* features, const float* h_in, const float* c_in, float* h_out, float* c_out, float* logits,
@@ -287,13 +324,23 @@ int ssd_policy_lstm_heads(ssd_policy_t p, const float* features, const float* h_
     const void* ptrs[5] = {features, h_in, c_in, h_out, c_out};
     for (const void* q : ptrs)
         if (reinterpret_cast<uintptr_t>(q) % 16 != 0) return ssd::set_error(SSD_ERR_INVALID, "features and state pointers must be 16-byte aligned");
+    const int np = p->num_policies;
+    if (num_agents % np != 0) return ssd::set_error(SSD_ERR_INVALID, "num_agents must be a multiple of num_policies");
     if (num_agents == 0) return SSD_OK;
     if (cudaSetDevice(p->device) != cudaSuccess) return ssd::set_error(SSD_ERR_CUDA, "cudaSetDevice failed");  // the blob and the stream live there
-    const long long groups = (num_agents + GA - 1) / GA;
-    const int grid = static_cast<int>(groups < p->sms ? groups : p->sms);
-    lstm_heads_kernel<<<grid, kThreads, kSmemBytes, static_cast<cudaStream_t>(stream)>>>(
-        features, h_in, c_in, h_out, c_out, logits, value, actions, num_agents, p->num_outputs, p->d_head_blob, static_cast<uint32_t>(seed),
-        static_cast<uint32_t>(seed >> 32), counter);
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const uint32_t s_lo = static_cast<uint32_t>(seed), s_hi = static_cast<uint32_t>(seed >> 32);
+    if (np == 1) {
+        const long long groups = (num_agents + GA - 1) / GA;
+        const int grid = static_cast<int>(groups < p->sms ? groups : p->sms);
+        lstm_heads_kernel<false><<<grid, kThreads, kSmemBytes, st>>>(features, h_in, c_in, h_out, c_out, logits, value, actions, num_agents,
+                                                                    p->num_outputs, p->d_head_blob, s_lo, s_hi, counter, 1, grid);
+    } else {  // P * floor(#SMs / P) CTAs at most, each serving one policy
+        const long long groups = (num_agents / np + GA - 1) / GA;
+        const int per = static_cast<int>(groups < p->sms / np ? groups : p->sms / np);
+        lstm_heads_kernel<true><<<np * per, kThreads, kSmemBytes, st>>>(features, h_in, c_in, h_out, c_out, logits, value, actions, num_agents,
+                                                                       p->num_outputs, p->d_head_blob, s_lo, s_hi, counter, np, per);
+    }
     const cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return ssd::set_error(SSD_ERR_CUDA, cudaGetErrorString(e));
     return SSD_OK;

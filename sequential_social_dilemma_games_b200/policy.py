@@ -14,7 +14,12 @@ models/conv_to_fcnet_v2.py (ConvToFCNetv2) evaluated on uint8 observations that 
 The recurrent state (h, c) of the fused route lives in HBM in the kernel's tiled layout, shape [ceil(M/128), 8, 128, 16]
 (group of 128 agents, block of 16 units, agent, unit): a warp of the cell update then moves 2 KB contiguous per access.  Treat
 it as opaque between steps (as RLlib does with state_out -> state_in); `state_rows` / `state_from_rows` convert to and from
-[M, cell_size].  Weights are numpy fp32 arrays in the Keras layouts (conv kernel [kh, kw, in, out], dense kernels [in, out], LSTM kernel
+[M, cell_size].
+
+One network per agent id -- the reference's training scripts (run_scripts/train_baseline.py, train_moa.py) build a policy per
+'agent-i' and map agent i to it -- is `ConvToFCNet([weights_0, ..., weights_{P-1}])`: agent (b, p) of a [B, P, 15, 15, 3]
+observation tensor is evaluated with weights_p by the same two kernels (one CTA serves one policy), outputs stay agent-major,
+and the tiled state is grouped per policy, [P * ceil(B/128), 8, 128, 16].  Weights are numpy fp32 arrays in the Keras layouts (conv kernel [kh, kw, in, out], dense kernels [in, out], LSTM kernel
 [in, 4u] / recurrent kernel [u, 4u] / bias [4u] with gates ordered i, f, c, o), so a checkpoint of the reference model
 loads without transposition.  There is no CPU path: the trunk raises without the CUDA library.
 """
@@ -57,7 +62,11 @@ def random_weights(num_outputs, cell_size=128, seed=0):
 
 
 class ConvToFCNet(object):
-    """Forward pass of ConvToFCNetv2 for a batch of agents; `obs` is the uint8 tensor of the step path."""
+    """Forward pass of ConvToFCNetv2 for a batch of agents; `obs` is the uint8 tensor of the step path.
+
+    `weights` is one dict (one network shared by all agents) or a list of P dicts, weights[p] being the policy of 'agent-p':
+    agent m = b * P + p of the flattened [B, P, ...] batch is then evaluated with weights[p].  P > 1 needs the fused head
+    (cell_size 128, 1..15 outputs)."""
 
     def __init__(self, weights, device="cuda:0"):
         self.device = torch.device(device)
@@ -65,26 +74,41 @@ class ConvToFCNet(object):
             raise _lib.SsdError("the policy trunk runs on a CUDA device only")
         if self.device.index is None:  # 'cuda' means the current device, not device 0
             self.device = torch.device("cuda", torch.cuda.current_device())
-        w = {k: np.ascontiguousarray(v, dtype=np.float32) for k, v in weights.items()}
+        sets = list(weights) if isinstance(weights, (list, tuple)) else [weights]
+        if not sets:
+            raise ValueError("no weight sets")
+        sets = [{k: np.ascontiguousarray(v, dtype=np.float32) for k, v in ws.items()} for ws in sets]
+        w = sets[0]
         for name, shape in (("conv_w", (3, 3, 3, CONV_FILTERS)), ("conv_b", (CONV_FILTERS,)), ("fc1_w", (FLAT, FEATURES)),
                             ("fc1_b", (FEATURES,)), ("fc2_w", (FEATURES, FEATURES)), ("fc2_b", (FEATURES,))):
             if w[name].shape != shape:
                 raise ValueError("%s has shape %s, expected %s" % (name, w[name].shape, shape))
-        self.weights = w
-        self._h = C.c_void_p()
-        ptr = lambda a: a.ctypes.data_as(C.c_void_p)
-        _lib.check(_lib.lib.ssd_policy_create(VIEW_RADIUS, self.device.index, ptr(w["conv_w"]), ptr(w["conv_b"]), ptr(w["fc1_w"]),
-                                              ptr(w["fc1_b"]), ptr(w["fc2_w"]), ptr(w["fc2_b"]), C.byref(self._h)))
+        for p, ws in enumerate(sets[1:], 1):
+            if sorted(ws) != sorted(w) or any(ws[k].shape != w[k].shape for k in w):
+                raise ValueError("weights[%d] does not have the names and shapes of weights[0]" % p)
+        self.num_policies = P = len(sets)
+        self.weights = w if P == 1 and not isinstance(weights, (list, tuple)) else sets
         self.cell_size = w["lstm_u"].shape[0] if "lstm_u" in w else 0
         self.num_outputs = w["logits_w"].shape[1] if "logits_w" in w else 0
+        fused = self.cell_size == 128 and 1 <= self.num_outputs <= 15
+        if P > 1 and not fused:
+            raise ValueError("a network per agent needs the fused head: cell_size 128 and 1..15 outputs (got %d, %d)"
+                             % (self.cell_size, self.num_outputs))
+        if P > 1:   # P consecutive arrays behind every weight pointer
+            w = {k: np.ascontiguousarray(np.stack([ws[k] for ws in sets])) for k in w}
+        self._h = C.c_void_p()
+        ptr = lambda a: a.ctypes.data_as(C.c_void_p)
+        _lib.check(_lib.lib.ssd_policy_create_n(VIEW_RADIUS, self.device.index, P, ptr(w["conv_w"]), ptr(w["conv_b"]), ptr(w["fc1_w"]),
+                                                ptr(w["fc1_b"]), ptr(w["fc2_w"]), ptr(w["fc2_b"]), C.byref(self._h)))
         self._head = {}
         self._fused_head = False
         self._sample_seed, self._sample_counter = 0, 0
-        if self.cell_size == 128 and 1 <= self.num_outputs <= 15:
-            _lib.check(_lib.lib.ssd_policy_set_head(self._h, self.cell_size, self.num_outputs, ptr(w["lstm_w"]), ptr(w["lstm_u"]), ptr(w["lstm_b"]),
-                                                    ptr(w["logits_w"]), ptr(w["logits_b"]), ptr(w["value_w"]), ptr(w["value_b"])))
+        if fused:
+            _lib.check(_lib.lib.ssd_policy_set_head_n(self._h, P, self.cell_size, self.num_outputs, ptr(w["lstm_w"]), ptr(w["lstm_u"]),
+                                                      ptr(w["lstm_b"]), ptr(w["logits_w"]), ptr(w["logits_b"]), ptr(w["value_w"]),
+                                                      ptr(w["value_b"])))
             self._fused_head = True
-        if self.cell_size:
+        if self.cell_size and P == 1:
             if self.cell_size % 8:
                 raise ValueError("cell_size must be a multiple of 8")
             dev = lambda k, dt: torch.from_numpy(w[k]).to(self.device, dtype=dt).contiguous()
@@ -103,10 +127,22 @@ class ConvToFCNet(object):
         except Exception:
             pass
 
+    def _groups(self, m):
+        """Number of 128-agent state groups of m agents: P * ceil(m / P / 128)."""
+        P = self.num_policies
+        if m % P:
+            raise ValueError("%d agents do not split into %d per-agent policies" % (m, P))
+        return P * ((m // P + 127) // 128)
+
     def features(self, obs, out=None):
-        """uint8 [..., 15, 15, 3] on the device -> float32 [M, 32] (M = product of the leading dims)."""
+        """uint8 [..., 15, 15, 3] on the device -> float32 [M, 32] (M = product of the leading dims).  A network per agent
+        takes [B, P, 15, 15, 3] or [B * P, 15, 15, 3]; rows stay agent-major."""
         if obs.dtype != torch.uint8 or obs.device != self.device or tuple(obs.shape[-3:]) != (OBS_SIDE, OBS_SIDE, 3):
             raise ValueError("obs must be a uint8 [..., %d, %d, 3] tensor on %s" % (OBS_SIDE, OBS_SIDE, self.device))
+        P = self.num_policies
+        if P > 1 and not (obs.dim() == 4 and obs.shape[0] % P == 0 or obs.dim() == 5 and obs.shape[1] == P):
+            raise ValueError("a network of %d per-agent policies takes obs [B, %d, %d, %d, 3] or [B * %d, %d, %d, 3], not %s"
+                             % (P, P, OBS_SIDE, OBS_SIDE, P, OBS_SIDE, OBS_SIDE, tuple(obs.shape)))
         obs = obs.contiguous()
         m = obs.numel() // (OBS_SIDE * OBS_SIDE * 3)
         if out is None:
@@ -117,26 +153,30 @@ class ConvToFCNet(object):
 
     def initial_state(self, m):
         """Zero (h, c) for m agents, in the layout `forward` / `act` carry (tiled for the fused route, [m, cell_size] otherwise)."""
-        shape = ((m + 127) // 128, self.cell_size // 16, 128, 16) if self._fused_head else (m, self.cell_size)
+        shape = (self._groups(m), self.cell_size // 16, 128, 16) if self._fused_head else (m, self.cell_size)
         z = torch.zeros(shape, dtype=torch.float32, device=self.device)
         return z, z.clone()
 
-    @staticmethod
-    def state_rows(state, m):
-        """Tiled state [G, 8, 128, 16] -> [m, cell_size] (a copy)."""
+    def state_rows(self, state, m):
+        """Tiled state [G, 8, 128, 16] -> agent-major [m, cell_size] (a copy)."""
         if state.dim() == 2:
             return state[:m]
         g, b, r, e = state.shape
-        return state.permute(0, 2, 1, 3).reshape(g * r, b * e)[:m].contiguous()
+        rows = state.permute(0, 2, 1, 3).reshape(g * r, b * e)
+        P = self.num_policies
+        if P == 1:
+            return rows[:m].contiguous()
+        self._groups(m)
+        return rows.reshape(P, g // P * r, b * e)[:, :m // P].transpose(0, 1).reshape(m, b * e)   # (p, b) -> agent b * P + p
 
-    @staticmethod
-    def state_from_rows(rows):
-        """[m, cell_size] -> tiled state [ceil(m/128), cell_size/16, 128, 16], zero padded."""
+    def state_from_rows(self, rows):
+        """Agent-major [m, cell_size] -> tiled state [G, cell_size/16, 128, 16] (G = ceil(m/128), per policy for P > 1), zero padded."""
         m, u = rows.shape
-        g = (m + 127) // 128
-        full = torch.zeros((g * 128, u), dtype=rows.dtype, device=rows.device)
-        full[:m] = rows
-        return full.reshape(g, 128, u // 16, 16).permute(0, 2, 1, 3).contiguous()
+        P = self.num_policies
+        g = self._groups(m) // P
+        full = torch.zeros((P, g * 128, u), dtype=rows.dtype, device=rows.device)
+        full[:, :m // P] = rows.reshape(m // P, P, u).transpose(0, 1)
+        return full.reshape(P * g, 128, u // 16, 16).permute(0, 2, 1, 3).contiguous()
 
     def seed_sampling(self, seed):
         """Key of the Philox streams `act` samples from (counter = number of `act` calls since)."""
@@ -145,7 +185,7 @@ class ConvToFCNet(object):
     def _fused(self, obs, h, c, sample):
         x = self.features(obs)
         m = x.shape[0]
-        if h.dim() != 4 or h.shape[0] * 128 < m:
+        if h.dim() != 4 or (h.shape[0] * 128 < m if self.num_policies == 1 else h.shape[0] != self._groups(m)):
             raise ValueError("the fused route carries (h, c) in the tiled layout of initial_state / state_from_rows")
         h, c = h.contiguous(), c.contiguous()
         h_new, c_new = torch.empty_like(h), torch.empty_like(c)
@@ -168,7 +208,10 @@ class ConvToFCNet(object):
 
     def forward_unfused(self, obs, h, c):
         """The same forward pass with library GEMMs: the trunk kernel, the gate GEMMs (cuBLAS, bf16 x bf16 -> fp32 accumulate), the
-        one-pass cell update, the head GEMMs.  Any cell size that is a multiple of 8; (h, c) are [M, cell_size] here."""
+        one-pass cell update, the head GEMMs.  Any cell size that is a multiple of 8; (h, c) are [M, cell_size] here.  Shared
+        weights only."""
+        if self.num_policies > 1:
+            raise ValueError("forward_unfused runs one shared network; a network per agent runs on the fused route (forward / act)")
         hd = self._head
         x16 = self.features(obs).to(torch.bfloat16)
         gates = torch.mm(x16, hd["lstm_w"]).addmm_(h.to(torch.bfloat16), hd["lstm_u"])   # bf16 [M, 4u], bias added in the cell kernel
