@@ -231,6 +231,32 @@ int ssd_policy_create_n(int view_radius, int device, int num_policies, const flo
                         const float* fc1_b, const float* fc2_w, const float* fc2_b, ssd_policy_t* out);
 int ssd_policy_set_head_n(ssd_policy_t p, int num_policies, int units, int num_outputs, const float* lstm_w, const float* lstm_u,
                           const float* lstm_b, const float* logits_w, const float* logits_b, const float* value_w, const float* value_b);
+/* A policy pool: num_policies = K weight sets, 1..255, loaded once; every call takes a device u8 policy id per agent, and the
+ * ids may change from call to call (several runs or seeds on one GPU, cross-play teams, population play, scripted agents).
+ * ssd_policy_create_pool loads trunk and head together: every weight pointer points to K consecutive arrays in the layouts of
+ * ssd_policy_create / ssd_policy_set_head; the fused head is required.  K outside 1..255 or a null pointer returns
+ * SSD_ERR_INVALID; view_radius != 7, units != 128 or num_outputs outside 1..15 SSD_ERR_UNSUPPORTED; nothing is allocated then.
+ * ssd_policy_pool_features / ssd_policy_pool_lstm_heads take the arguments of ssd_policy_features / ssd_policy_lstm_heads plus
+ * policy_ids dev u8[num_agents], agent-major like obs: agent m is evaluated with weight set policy_ids[m].
+ *   - An id >= K means "no pool policy": nothing is written for that agent -- none of its rows of features, logits, value,
+ *     actions, h_out or c_out -- so a caller can drive it with its own code (as ssd_reset_rows ignores out-of-range rows).
+ *   - The recurrent state is in the TILED layout of the shared network, [ceil(M/128)][8][128][16] (element (agent m, unit u) at
+ *     ((m / 128 * 8 + u / 16) * 128 + m % 128) * 16 + u % 16): it does not depend on the ids, so they may change between two
+ *     steps of a live state.  An agent's rows of h_out / c_out are written only when it has a pool policy.
+ *   - Sampling keys Philox by (seed; m, counter) as ssd_policy_lstm_heads does: weight set k gives agent m exactly the action
+ *     a shared network with set k draws for m.
+ * Each call first groups the agents by id on the device (no host synchronisation) into scratch that belongs to the handle
+ * and grows on demand, so calls on one pool handle must be ordered (one stream).  Pool handles are rejected by
+ * ssd_policy_features / ssd_policy_lstm_heads / ssd_policy_set_head(_n), other handles by the pool entry points
+ * (SSD_ERR_INVALID).  At most 2^31 - 1 agents per call. */
+int ssd_policy_create_pool(int view_radius, int device, int num_policies, int units, int num_outputs, const float* conv_w, const float* conv_b,
+                           const float* fc1_w, const float* fc1_b, const float* fc2_w, const float* fc2_b, const float* lstm_w, const float* lstm_u,
+                           const float* lstm_b, const float* logits_w, const float* logits_b, const float* value_w, const float* value_b,
+                           ssd_policy_t* out);
+int ssd_policy_pool_features(ssd_policy_t p, const uint8_t* obs, const uint8_t* policy_ids, int64_t num_agents, float* features, void* stream);
+int ssd_policy_pool_lstm_heads(ssd_policy_t p, const float* features, const uint8_t* policy_ids, const float* h_in, const float* c_in, float* h_out,
+                               float* c_out, float* logits, float* value, int8_t* actions, int64_t num_agents, uint64_t seed, uint32_t counter,
+                               void* stream);
 /* The unfused alternative for other cell sizes: LSTM cell update after the gate GEMM (conv_to_fcnet_v2.py:68-80; Keras gate order i, f, c~, o; sigmoid recurrent
  * activation): gates dev bf16[num_agents][4*units] = x W + h U without the bias, bias dev f32[4*units],
  * c_prev / c_out / h_out dev f32[num_agents][units] (c_out may alias c_prev), h_bf16_out dev bf16[num_agents][units]

@@ -22,7 +22,8 @@ SYMBOLS = ("ssd_last_error", "ssd_abi_version", "ssd_create", "ssd_destroy", "ss
            "ssd_get_state", "ssd_reset", "ssd_reset_rows", "ssd_step", "ssd_rollout", "ssd_step_phases", "ssd_get_beams", "ssd_render", "ssd_render_map", "ssd_step_host",
            "ssd_set_option", "ssd_stats", "ssd_launch_count", "ssd_philox_selftest",
            "ssd_policy_create", "ssd_policy_features", "ssd_policy_destroy", "ssd_policy_lstm_cell",
-           "ssd_policy_set_head", "ssd_policy_lstm_heads", "ssd_policy_create_n", "ssd_policy_set_head_n")
+           "ssd_policy_set_head", "ssd_policy_lstm_heads", "ssd_policy_create_n", "ssd_policy_set_head_n",
+           "ssd_policy_create_pool", "ssd_policy_pool_features", "ssd_policy_pool_lstm_heads")
 
 
 class SsdConfig(C.Structure):
@@ -91,6 +92,9 @@ def _load():
         "ssd_policy_lstm_heads": (i32, [vp, vp, vp, vp, vp, vp, vp, vp, vp, i64, C.c_uint64, C.c_uint32, vp]),
         "ssd_policy_create_n": (i32, [i32, i32, i32, vp, vp, vp, vp, vp, vp, C.POINTER(vp)]),
         "ssd_policy_set_head_n": (i32, [vp, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp]),
+        "ssd_policy_create_pool": (i32, [i32, i32, i32, i32, i32] + [vp] * 13 + [C.POINTER(vp)]),
+        "ssd_policy_pool_features": (i32, [vp, vp, vp, i64, vp, vp]),
+        "ssd_policy_pool_lstm_heads": (i32, [vp] + [vp] * 9 + [i64, C.c_uint64, C.c_uint32, vp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)

@@ -115,9 +115,20 @@ struct TrunkSmem {
 // kPerAgent: agent m = b * P + p of the [B, P] batch is evaluated with weight set p (blob + p * kBlobBytes).  A UMMA tile
 // cannot change its B operand per row, so CTA c serves policy c % P only -- groups g = c / P, c / P + cpp, ... of the agents
 // (b, p), b in [128 g, 128 g + 128) -- and loads that policy's resident weights once, as the shared kernel does.
-template <bool kPerAgent>
+//
+// WeightMap::Pool: a group is one tile of the assignment (ssd_policy_pool.cu): agents perm[first, first + count) of one
+// policy, gathered and written back as the per-agent variant does, at rows perm[i].  CTA c takes tiles
+// [c T / G, (c + 1) T / G) and runs them as segments of consecutive tiles of one policy.  Each segment is the pipeline above
+// from a clean start: at a switch of policy every role has finished the previous segment (its last fc2 committed, its
+// features written), the CTA synchronises, re-initialises the barriers and loads the new policy's resident block.  The
+// Dense(32) blocks stream from the segment's blob.  Tiles are in policy order, so a CTA switches at most once per policy
+// boundary inside its range.
+template <WeightMap kMap>
 __global__ void __launch_bounds__(kThreads, 1) policy_features_kernel(const uint8_t* __restrict__ obs, long long M, const uint8_t* __restrict__ blob,
-                                                                     float* __restrict__ out, int num_policies, int ctas_per_policy) {
+                                                                     float* __restrict__ out, int num_policies, int ctas_per_policy,
+                                                                     const uint32_t* __restrict__ perm, const PoolTile* __restrict__ tiles,
+                                                                     const uint32_t* __restrict__ num_tiles) {
+    constexpr bool kPerAgent = kMap != WeightMap::Shared, kPool = kMap == WeightMap::Pool;
     using L = TrunkSmem<kPerAgent>;
     constexpr int WRING = L::WRING, kObsStride = L::kObsStride, kOffObs = L::kOffObs, kOffB1 = L::kOffB1, kOffB3 = L::kOffB3;
     constexpr int kOffConst = L::kOffConst, kOffW1 = L::kOffW1, kOffBar = L::kOffBar;
@@ -131,11 +142,35 @@ __global__ void __launch_bounds__(kThreads, 1) policy_features_kernel(const uint
     const long long cta = kPerAgent ? blockIdx.x / np : blockIdx.x;                          // its index among the CTAs of that policy
     const long long stride = kPerAgent ? ctas_per_policy : gridDim.x;
     const long long rows = kPerAgent ? M / np : M;                                           // agents per policy
-    if (kPerAgent) blob += static_cast<long long>(pol) * kBlobBytes;
+    const uint8_t* const blob0 = blob;
+    if (kPerAgent && !kPool) blob += static_cast<long long>(pol) * kBlobBytes;
     const long long n_groups = (rows + GA - 1) / GA;
-    const uint32_t n_my = cta < n_groups ? static_cast<uint32_t>((n_groups - cta + stride - 1) / stride) : 0;  // groups of this CTA
+    long long seg_end = 0, tile_end = 0;   // pool: the CTA's tiles not yet run are [seg_end, tile_end)
+    if (kPool) {
+        const long long nt = *num_tiles;
+        seg_end = nt * blockIdx.x / gridDim.x;
+        tile_end = nt * (blockIdx.x + 1) / gridDim.x;
+    }
+    int seg = 0;
+    uint32_t tmem_base = 0;
+    do {   // pool: one pass per segment; otherwise one pass
+    long long tb = seg_end;   // pool: the segment's first tile = group 0
+    if (kPool && seg_end < tile_end) {
+        tb = seg_end;
+        const int k = tiles[tb].policy;
+        while (++seg_end < tile_end && tiles[seg_end].policy == k) {
+        }
+        blob = blob0 + static_cast<long long>(k) * kBlobBytes;
+    }
+    const uint32_t n_my = kPool ? static_cast<uint32_t>(seg_end - tb)
+                                : cta < n_groups ? static_cast<uint32_t>((n_groups - cta + stride - 1) / stride) : 0;  // groups of this CTA
     const uint32_t NT = n_my * CO;
 
+    if (kPool && seg > 0) {   // every role is done with the previous segment: its barriers can start over
+        tc_fence_after();
+        if (tid == 0)
+            for (int b = 0; b < BAR_COUNT; ++b) asm volatile("mbarrier.inval.shared::cta.b64 [%0];" ::"r"(smem_u32(bars + b)) : "memory");
+    }
     if (tid == 0) {
         for (int b = 0; b < BAR_COUNT; ++b) {
             const int count = (b >= BAR_OBS_FREE && b < BAR_D1_FREE) ? kProducerWarps      // one arrival per producer warp
@@ -144,7 +179,7 @@ __global__ void __launch_bounds__(kThreads, 1) policy_features_kernel(const uint
         }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
-    if (warp == kMmaWarp) {  // all of the SM's tensor memory (one CTA per SM)
+    if (seg == 0 && warp == kMmaWarp) {  // all of the SM's tensor memory (one CTA per SM)
         asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&s_tmem)), "r"(kTmemCols) : "memory");
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
     }
@@ -155,6 +190,7 @@ __global__ void __launch_bounds__(kThreads, 1) policy_features_kernel(const uint
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem = s_tmem;
+    tmem_base = tmem;
 
     if (warp < kProducerWarps) {
         // ------------------------------------------------------------------ producers
@@ -176,7 +212,10 @@ __global__ void __launch_bounds__(kThreads, 1) policy_features_kernel(const uint
             warp_wait(bars + BAR_OBS + (gi & 1), (gi >> 1) & 1);
             SSD_PT(0);
             const uint8_t* img = smem + kOffObs + (gi & 1) * kObsStride + t * L::kSlot;
-            if (kPerAgent)  // the slot starts at the 16-byte boundary below the agent's row (obs is 16-byte aligned)
+            if (kPool) {
+                const PoolTile tile = tiles[tb + gi];
+                img += t < tile.count ? (perm[tile.first + t] * static_cast<uint32_t>(IMG)) & 15u : 0u;
+            } else if (kPerAgent)  // the slot starts at the 16-byte boundary below the agent's row (obs is 16-byte aligned)
                 img += (static_cast<uint32_t>(((cta + gi * stride) * GA + t) * np + pol) * IMG) & 15u;
 #pragma unroll 1
             for (int r = 0; r < V; ++r, ++R) {
@@ -330,7 +369,8 @@ __global__ void __launch_bounds__(kThreads, 1) policy_features_kernel(const uint
             };
             auto load_obs = [&](uint32_t gi) {
                 const long long a0 = (cta + static_cast<long long>(gi) * stride) * GA;
-                const int rem = static_cast<int>(rows - a0 < GA ? rows - a0 : GA);
+                const PoolTile tile = kPool ? tiles[tb + gi] : PoolTile{};
+                const int rem = kPool ? tile.count : static_cast<int>(rows - a0 < GA ? rows - a0 : GA);
                 uint8_t* dst = smem + kOffObs + (gi & 1) * kObsStride;
                 uint64_t* bar = bars + BAR_OBS + (gi & 1);
                 if (!kPerAgent) {  // the group's rem * 675 contiguous bytes (a group starts 16-byte aligned)
@@ -342,7 +382,7 @@ __global__ void __launch_bounds__(kThreads, 1) policy_features_kernel(const uint
                 } else {  // gather: per agent the 16-byte-aligned span around its row, into its slot; nothing past the tensor's end
                     const long long end = M * IMG, end16 = end & ~15ll;
                     auto span = [&](int t, long long& s0) {
-                        const long long s = ((a0 + t) * np + pol) * IMG, s1 = (s + IMG + 15) & ~15ll;
+                        const long long s = (kPool ? static_cast<long long>(perm[tile.first + t]) : (a0 + t) * np + pol) * IMG, s1 = (s + IMG + 15) & ~15ll;
                         s0 = s & ~15ll;
                         return static_cast<uint32_t>((s1 < end16 ? s1 : end16) - s0);
                     };
@@ -423,8 +463,9 @@ __global__ void __launch_bounds__(kThreads, 1) policy_features_kernel(const uint
             tmem_ld_wait();
             tc_fence_before();
             const long long a0 = (cta + static_cast<long long>(gi) * stride) * GA;
-            if (a0 + row < rows) {
-                float4* dst = reinterpret_cast<float4*>(out + ((a0 + row) * np + pol) * FEAT + 16 * half);
+            const PoolTile tile = kPool ? tiles[tb + gi] : PoolTile{};
+            if (kPool ? row < tile.count : a0 + row < rows) {
+                float4* dst = reinterpret_cast<float4*>(out + (kPool ? static_cast<long long>(perm[tile.first + row]) : (a0 + row) * np + pol) * FEAT + 16 * half);
                 const float* b2 = s_const + N1 + N2 + 16 * half;
 #pragma unroll
                 for (int c = 0; c < 16; c += 4)
@@ -477,9 +518,15 @@ __global__ void __launch_bounds__(kThreads, 1) policy_features_kernel(const uint
         }
         if (tid == 32 * kDrainWarp0) SSD_PT_FLUSH(2);
     }
+    if (kPool) {
+        tc_fence_before();
+        __syncthreads();
+    }
+    ++seg;
+    } while (kPool && seg_end < tile_end);
     tc_fence_before();
     __syncthreads();
-    if (warp == kMmaWarp) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(kTmemCols) : "memory");
+    if (warp == kMmaWarp) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(kTmemCols) : "memory");
 }
 
 // LSTM cell update after the gate GEMM (conv_to_fcnet_v2.py:68-80, Keras gate order i, f, c~, o):
@@ -527,20 +574,13 @@ __global__ void __launch_bounds__(256) lstm_cell_kernel(const uint4* __restrict_
     h16_out[idx] = make_uint4(p[0], p[1], p[2], p[3]);
 }
 
-}  // namespace policy
-}  // namespace ssd
-
-
-#pragma GCC visibility push(default)
-extern "C" {
-
-int ssd_policy_create_n(int view_radius, int device, int num_policies, const float* conv_w, const float* conv_b, const float* fc1_w,
-                        const float* fc1_b, const float* fc2_w, const float* fc2_b, ssd_policy_t* out) {
-    using namespace ssd::policy;
+// Packs num_policies trunk weight sets (Keras layouts, consecutive behind each pointer) into a new handle; the caller has
+// checked num_policies against its map's limit.
+int create_trunk(int view_radius, int device, int num_policies, WeightMap map, const float* conv_w, const float* conv_b, const float* fc1_w,
+                 const float* fc1_b, const float* fc2_w, const float* fc2_b, SsdPolicy** out) {
     if (!out) return ssd::set_error(SSD_ERR_INVALID, "null argument");
     *out = nullptr;
     if (!conv_w || !conv_b || !fc1_w || !fc1_b || !fc2_w || !fc2_b) return ssd::set_error(SSD_ERR_INVALID, "null weight pointer");
-    if (num_policies < 1 || num_policies > SSD_MAX_AGENTS) return ssd::set_error(SSD_ERR_INVALID, "num_policies must be 1..SSD_MAX_AGENTS");
     if (2 * view_radius + 1 != V) return ssd::set_error(SSD_ERR_UNSUPPORTED, "the feature kernel is built for 15x15 observations (view radius 7)");
     const size_t blob_bytes = static_cast<size_t>(num_policies) * kBlobBytes;
     std::vector<uint8_t> blobs(blob_bytes, 0);
@@ -584,14 +624,17 @@ int ssd_policy_create_n(int view_radius, int device, int num_policies, const flo
     if (!p) return ssd::set_error(SSD_ERR_INVALID, "out of host memory");
     p->device = device;
     p->num_policies = num_policies;
+    p->pool = map == WeightMap::Pool;
     cudaError_t e = cudaSetDevice(device);
     if (e == cudaSuccess) e = cudaDeviceGetAttribute(&p->sms, cudaDevAttrMultiProcessorCount, device);
     if (e == cudaSuccess) e = cudaMalloc(&p->d_blob, blob_bytes);
     if (e == cudaSuccess) e = cudaMemcpy(p->d_blob, blobs.data(), blob_bytes, cudaMemcpyHostToDevice);
-    if (e == cudaSuccess && num_policies == 1)
-        e = cudaFuncSetAttribute(policy_features_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TrunkSmem<false>::kSmemBytes);
-    if (e == cudaSuccess && num_policies > 1)
-        e = cudaFuncSetAttribute(policy_features_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TrunkSmem<true>::kSmemBytes);
+    if (e == cudaSuccess && map == WeightMap::Pool)
+        e = cudaFuncSetAttribute(policy_features_kernel<WeightMap::Pool>, cudaFuncAttributeMaxDynamicSharedMemorySize, TrunkSmem<true>::kSmemBytes);
+    else if (e == cudaSuccess && num_policies == 1)
+        e = cudaFuncSetAttribute(policy_features_kernel<WeightMap::Shared>, cudaFuncAttributeMaxDynamicSharedMemorySize, TrunkSmem<false>::kSmemBytes);
+    else if (e == cudaSuccess)
+        e = cudaFuncSetAttribute(policy_features_kernel<WeightMap::PerAgent>, cudaFuncAttributeMaxDynamicSharedMemorySize, TrunkSmem<true>::kSmemBytes);
     if (e != cudaSuccess) {
         if (p->d_blob) cudaFree(p->d_blob);
         delete p;
@@ -601,6 +644,20 @@ int ssd_policy_create_n(int view_radius, int device, int num_policies, const flo
     return SSD_OK;
 }
 
+
+}  // namespace policy
+}  // namespace ssd
+
+
+#pragma GCC visibility push(default)
+extern "C" {
+
+int ssd_policy_create_n(int view_radius, int device, int num_policies, const float* conv_w, const float* conv_b, const float* fc1_w,
+                        const float* fc1_b, const float* fc2_w, const float* fc2_b, ssd_policy_t* out) {
+    if (out) *out = nullptr;
+    if (num_policies < 1 || num_policies > SSD_MAX_AGENTS) return ssd::set_error(SSD_ERR_INVALID, "num_policies must be 1..SSD_MAX_AGENTS");
+    return ssd::policy::create_trunk(view_radius, device, num_policies, WeightMap::PerAgent, conv_w, conv_b, fc1_w, fc1_b, fc2_w, fc2_b, out);
+}
 int ssd_policy_create(int view_radius, int device, const float* conv_w, const float* conv_b, const float* fc1_w, const float* fc1_b,
                       const float* fc2_w, const float* fc2_b, ssd_policy_t* out) {
     return ssd_policy_create_n(view_radius, device, 1, conv_w, conv_b, fc1_w, fc1_b, fc2_w, fc2_b, out);
@@ -611,6 +668,7 @@ int ssd_policy_features(ssd_policy_t p, const uint8_t* obs, int64_t num_agents, 
     if (!p || !obs || !features || num_agents < 0) return ssd::set_error(SSD_ERR_INVALID, "bad argument");
     if (reinterpret_cast<uintptr_t>(obs) % 16 != 0 || reinterpret_cast<uintptr_t>(features) % 16 != 0)
         return ssd::set_error(SSD_ERR_INVALID, "obs and features must be 16-byte aligned");
+    if (p->pool) return ssd::set_error(SSD_ERR_INVALID, "a policy pool handle takes ssd_policy_pool_features");
     const int np = p->num_policies;
     if (num_agents % np != 0) return ssd::set_error(SSD_ERR_INVALID, "num_agents must be a multiple of num_policies");
     if (num_agents == 0) return SSD_OK;
@@ -619,12 +677,33 @@ int ssd_policy_features(ssd_policy_t p, const uint8_t* obs, int64_t num_agents, 
     if (np == 1) {
         const long long groups = (num_agents + GA - 1) / GA;
         const int grid = static_cast<int>(groups < p->sms ? groups : p->sms);
-        policy_features_kernel<false><<<grid, kThreads, TrunkSmem<false>::kSmemBytes, st>>>(obs, num_agents, p->d_blob, features, 1, grid);
+        policy_features_kernel<WeightMap::Shared><<<grid, kThreads, TrunkSmem<false>::kSmemBytes, st>>>(obs, num_agents, p->d_blob, features, 1, grid,
+                                                                                                      nullptr, nullptr, nullptr);
     } else {  // P * floor(#SMs / P) CTAs at most, each serving one policy
         const long long groups = (num_agents / np + GA - 1) / GA;
         const int per = static_cast<int>(groups < p->sms / np ? groups : p->sms / np);
-        policy_features_kernel<true><<<np * per, kThreads, TrunkSmem<true>::kSmemBytes, st>>>(obs, num_agents, p->d_blob, features, np, per);
+        policy_features_kernel<WeightMap::PerAgent><<<np * per, kThreads, TrunkSmem<true>::kSmemBytes, st>>>(obs, num_agents, p->d_blob, features, np, per,
+                                                                                                           nullptr, nullptr, nullptr);
     }
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return ssd::set_error(SSD_ERR_CUDA, cudaGetErrorString(e));
+    return SSD_OK;
+}
+
+int ssd_policy_pool_features(ssd_policy_t p, const uint8_t* obs, const uint8_t* policy_ids, int64_t num_agents, float* features, void* stream) {
+    using namespace ssd::policy;
+    if (!p || !obs || !policy_ids || !features || num_agents < 0) return ssd::set_error(SSD_ERR_INVALID, "bad argument");
+    if (!p->pool) return ssd::set_error(SSD_ERR_INVALID, "not a policy pool handle (ssd_policy_create_pool)");
+    if (reinterpret_cast<uintptr_t>(obs) % 16 != 0 || reinterpret_cast<uintptr_t>(features) % 16 != 0)
+        return ssd::set_error(SSD_ERR_INVALID, "obs and features must be 16-byte aligned");
+    if (num_agents == 0) return SSD_OK;
+    const int rc = ssd::policy_pool::assign(p, policy_ids, num_agents, stream);   // sets the device
+    if (rc != SSD_OK) return rc;
+    // a persistent grid over the tile table, whose length only the device knows
+    const long long tiles = ssd::policy_pool::max_tiles(num_agents, p->num_policies);
+    const int grid = static_cast<int>(tiles < p->sms ? tiles : p->sms);
+    policy_features_kernel<WeightMap::Pool><<<grid, kThreads, TrunkSmem<true>::kSmemBytes, static_cast<cudaStream_t>(stream)>>>(
+        obs, num_agents, p->d_blob, features, p->num_policies, grid, p->d_perm, p->d_tiles, p->d_counts + 512);
     const cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return ssd::set_error(SSD_ERR_CUDA, cudaGetErrorString(e));
     return SSD_OK;
@@ -653,6 +732,9 @@ void ssd_policy_destroy(ssd_policy_t p) {
     cudaSetDevice(p->device);
     cudaFree(p->d_blob);
     if (p->d_head_blob) cudaFree(p->d_head_blob);
+    if (p->d_counts) cudaFree(p->d_counts);
+    if (p->d_perm) cudaFree(p->d_perm);
+    if (p->d_tiles) cudaFree(p->d_tiles);
     delete p;
 }
 

@@ -68,12 +68,19 @@ __device__ __forceinline__ float sigmoid_fast(float x) { return fmaf(tanh_fast(0
 // kPerAgent: agent m = b * P + p uses weight set p (blob + p * kBlobBytes).  As in the trunk, CTA c serves policy c % P only
 // (groups g = c / P, c / P + cpp, ... of the agents (b, p), b in [128 g, 128 g + 128)), so its [W; U] is loaded once; features
 // are read as 128-byte rows P * 128 bytes apart, outputs are written to agent-major rows, and the recurrent state of that
-// group is state group p * ceil(B / 128) + g.  The sampler keys Philox by the agent-major index m in both variants.
-template <bool kPerAgent>
+// group is state group p * ceil(B / 128) + g.  The sampler keys Philox by the agent-major index m in all variants.
+//
+// WeightMap::Pool: a group is one tile of the assignment (ssd_policy_pool.cu), agents perm[first, first + count) of one policy;
+// CTA c takes tiles [c T / G, (c + 1) T / G) and reloads the resident weights when the policy changes (the tiles are in
+// policy order).  Feature rows are gathered by perm, h and c are read and written per agent in the agent-major tiled layout
+// (64-byte pieces, one per 16 units), outputs go to row m.
+template <WeightMap kMap>
 __global__ void __launch_bounds__(kThreads, 1)
 lstm_heads_kernel(const float* __restrict__ feat, const float* h_in, const float* c_in, float* h_out, float* c_out, float* __restrict__ logits,
                   float* __restrict__ value, int8_t* __restrict__ actions, long long M, int num_outputs, const uint8_t* __restrict__ blob,
-                  uint32_t seed_lo, uint32_t seed_hi, uint32_t counter, int num_policies, int ctas_per_policy) {
+                  uint32_t seed_lo, uint32_t seed_hi, uint32_t counter, int num_policies, int ctas_per_policy, const uint32_t* __restrict__ perm,
+                  const PoolTile* __restrict__ tiles, const uint32_t* __restrict__ num_tiles) {
+    constexpr bool kPerAgent = kMap != WeightMap::Shared, kPool = kMap == WeightMap::Pool;
     extern __shared__ __align__(128) uint8_t smem[];
     __shared__ uint32_t s_tmem;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -81,10 +88,19 @@ lstm_heads_kernel(const float* __restrict__ feat, const float* h_in, const float
     const float* s_bias = reinterpret_cast<const float*>(smem + kOffConst);
     const int np = kPerAgent ? num_policies : 1;
     const int pol = kPerAgent ? static_cast<int>(blockIdx.x) % np : 0;                       // this CTA's weight set
-    const long long cta = kPerAgent ? blockIdx.x / np : blockIdx.x;                          // its index among the CTAs of that policy
-    const long long stride = kPerAgent ? ctas_per_policy : gridDim.x;
+    const long long nt = kPool ? *num_tiles : 0;
+    const long long cta = kPool ? nt * blockIdx.x / gridDim.x                                // pool: its first tile
+                                : kPerAgent ? blockIdx.x / np : blockIdx.x;                  // its index among the CTAs of that policy
+    const long long stride = kPool ? 1 : kPerAgent ? ctas_per_policy : gridDim.x;
     const long long rows = kPerAgent ? M / np : M;                                           // agents per policy
-    if (kPerAgent) blob += static_cast<long long>(pol) * kBlobBytes;
+    const uint8_t* const blob0 = blob;
+    int cur = 0;   // pool: the weight set in shared memory
+    if (kPool) {
+        cur = cta < nt * (blockIdx.x + 1) / gridDim.x ? tiles[cta].policy : 0;
+        blob += static_cast<long long>(cur) * kBlobBytes;
+    } else if (kPerAgent) {
+        blob += static_cast<long long>(pol) * kBlobBytes;
+    }
     if (tid == 0) mbar_init(bar, 1);
     if (warp == 0) tmem_alloc(&s_tmem, 512);
     for (int i = tid; i < (kBlobBytes >> 4); i += kThreads) reinterpret_cast<uint4*>(smem)[i] = reinterpret_cast<const uint4*>(blob)[i];
@@ -97,11 +113,22 @@ lstm_heads_kernel(const float* __restrict__ feat, const float* h_in, const float
     constexpr uint32_t kIG = umma_idesc(GA, 256), kIH = umma_idesc(GA, NH);
     uint32_t parity = 0;
 
-    const long long n_groups = (rows + GA - 1) / GA;
+    const long long n_groups = kPool ? nt * (blockIdx.x + 1) / gridDim.x : (rows + GA - 1) / GA;   // pool: the end of its tiles
     SSD_HT_DECL;
     for (long long g = cta; g < n_groups; g += stride) {
         const long long a0 = g * GA, sg = pol * n_groups + g;   // first agent row of the group in its policy; its state group
-        const int rem = static_cast<int>(rows - a0 < GA ? rows - a0 : GA);
+        const PoolTile tile = kPool ? tiles[g] : PoolTile{};
+        if (kPool && tile.policy != cur) {   // the previous group is complete (the barrier at the end of the loop)
+            cur = tile.policy;
+            const uint4* src = reinterpret_cast<const uint4*>(blob0 + static_cast<long long>(cur) * kBlobBytes);
+            for (int i = tid; i < (kBlobBytes >> 4); i += kThreads) reinterpret_cast<uint4*>(smem)[i] = src[i];
+            fence_async_smem();
+            __syncthreads();
+        }
+        // pool: agent of row r of the tile, its offset in the agent-major tiled state (element (m, u) at (that + u / 16 * 128) * 16 + u % 16)
+        auto agent = [&](int r) { return static_cast<long long>(perm[tile.first + r]); };
+        auto state_row = [](long long m) { return (m >> 7) * (U / 16) * GA + (m & (GA - 1)); };
+        const int rem = kPool ? tile.count : static_cast<int>(rows - a0 < GA ? rows - a0 : GA);
         {   // A = fp16([features | h]).  HBM is read in long contiguous runs (features: a 128-byte row per eight lanes; h: the tiled
             // state, 64 bytes per lane, 2 KB per warp -- a thread walking a row-major row in 32-byte steps reached 2.3 TB/s).
             // All loads before the stores: the compiler keeps a global load below a store through a generic pointer.
@@ -112,11 +139,12 @@ lstm_heads_kernel(const float* __restrict__ feat, const float* h_in, const float
 #pragma unroll
             for (int ps = 0; ps < 4; ++ps) {
                 const int row = ps * 32 + r8;
-                vx[ps] = row < rem ? __ldcs(reinterpret_cast<const float4*>(feat + ((a0 + row) * np + pol) * KX) + seg) : z;
+                vx[ps] = row < rem ? __ldcs(reinterpret_cast<const float4*>(feat + (kPool ? agent(row) : (a0 + row) * np + pol) * KX) + seg) : z;
             }
+            const long long hbase = kPool && hrow < rem ? state_row(agent(hrow)) : 0;
 #pragma unroll
             for (int b = 0; b < 4; ++b) {
-                const float4* src = reinterpret_cast<const float4*>(h_in + ((sg * (U / 16) + hb0 + b) * GA + hrow) * 16);
+                const float4* src = reinterpret_cast<const float4*>(h_in + (kPool ? (hbase + (hb0 + b) * GA) * 16 : ((sg * (U / 16) + hb0 + b) * GA + hrow) * 16));
 #pragma unroll
                 for (int j = 0; j < 4; ++j) vh[b][j] = hrow < rem ? __ldcs(src + j) : z;
             }
@@ -154,7 +182,8 @@ lstm_heads_kernel(const float* __restrict__ feat, const float* h_in, const float
             const int q = warp & 3, row = q * 32 + lane, uh = warp >> 2;
             const uint32_t trow = tmem + (static_cast<uint32_t>(q * 32) << 16);
             const bool live = row < rem;
-            const long long tile0 = ((sg * (U / 16) + uh * 4) * GA + row) * 16;   // this agent's 16 floats of unit block 4 uh; + GA * 16 per block
+            const long long tile0 = kPool ? (live ? (state_row(agent(row)) + uh * 4 * GA) * 16 : 0)
+                                          : ((sg * (U / 16) + uh * 4) * GA + row) * 16;   // this agent's 16 floats of unit block 4 uh; + GA * 16 per block
             float4 cn[4];   // the next 16 units of c, fetched one iteration ahead
 #pragma unroll
             for (int e = 0; e < 4; ++e) cn[e] = live ? __ldcs(reinterpret_cast<const float4*>(c_in + tile0) + e) : make_float4(0.f, 0.f, 0.f, 0.f);
@@ -216,7 +245,7 @@ lstm_heads_kernel(const float* __restrict__ feat, const float* h_in, const float
             tmem_ld16(tmem + (static_cast<uint32_t>(warp * 32) << 16), y);
             tmem_ld_wait();
             if (row < rem) {
-                const long long m = (a0 + row) * np + pol;
+                const long long m = kPool ? agent(row) : (a0 + row) * np + pol;
                 const float* hb = s_bias + NG;
                 float best = -3.0e38f;
                 int arg = 0;
@@ -267,10 +296,20 @@ extern "C" {
 
 int ssd_policy_set_head_n(ssd_policy_t p, int num_policies, int units, int num_outputs, const float* lstm_w, const float* lstm_u,
                           const float* lstm_b, const float* logits_w, const float* logits_b, const float* value_w, const float* value_b) {
-    using namespace ssd::policy_head;
-    if (!p || !lstm_w || !lstm_u || !lstm_b || !logits_w || !logits_b || !value_w || !value_b) return ssd::set_error(SSD_ERR_INVALID, "null argument");
+    if (!p) return ssd::set_error(SSD_ERR_INVALID, "null argument");
     if (num_policies < 1 || num_policies > SSD_MAX_AGENTS) return ssd::set_error(SSD_ERR_INVALID, "num_policies must be 1..SSD_MAX_AGENTS");
     if (num_policies != p->num_policies) return ssd::set_error(SSD_ERR_INVALID, "the head must have as many weight sets as the trunk");
+    if (p->pool) return ssd::set_error(SSD_ERR_INVALID, "a policy pool's head is loaded by ssd_policy_create_pool");
+    return ssd::policy_head::set_head(p, units, num_outputs, lstm_w, lstm_u, lstm_b, logits_w, logits_b, value_w, value_b);
+}
+#pragma GCC visibility pop
+}  // extern "C"
+
+int ssd::policy_head::set_head(SsdPolicy* p, int units, int num_outputs, const float* lstm_w, const float* lstm_u, const float* lstm_b,
+                               const float* logits_w, const float* logits_b, const float* value_w, const float* value_b) {
+    using namespace ssd::policy_head;
+    if (!lstm_w || !lstm_u || !lstm_b || !logits_w || !logits_b || !value_w || !value_b) return ssd::set_error(SSD_ERR_INVALID, "null argument");
+    const int num_policies = p->num_policies;
     if (units != U) return ssd::set_error(SSD_ERR_UNSUPPORTED, "the fused LSTM kernel is built for cell_size 128 (conv_to_fcnet_v2.py's custom_options)");
     if (num_outputs < 1 || num_outputs > NH - 1) return ssd::set_error(SSD_ERR_UNSUPPORTED, "1..15 policy outputs");
     const size_t blob_bytes = static_cast<size_t>(num_policies) * kBlobBytes;
@@ -303,13 +342,17 @@ int ssd_policy_set_head_n(ssd_policy_t p, int num_policies, int units, int num_o
     cudaError_t e = cudaSetDevice(p->device);
     if (e == cudaSuccess && !p->d_head_blob) e = cudaMalloc(&p->d_head_blob, blob_bytes);
     if (e == cudaSuccess) e = cudaMemcpy(p->d_head_blob, blobs.data(), blob_bytes, cudaMemcpyHostToDevice);
-    if (e == cudaSuccess && num_policies == 1) e = cudaFuncSetAttribute(lstm_heads_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
-    if (e == cudaSuccess && num_policies > 1) e = cudaFuncSetAttribute(lstm_heads_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
+    if (e == cudaSuccess && p->pool) e = cudaFuncSetAttribute(lstm_heads_kernel<WeightMap::Pool>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
+    else if (e == cudaSuccess && num_policies == 1) e = cudaFuncSetAttribute(lstm_heads_kernel<WeightMap::Shared>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
+    else if (e == cudaSuccess) e = cudaFuncSetAttribute(lstm_heads_kernel<WeightMap::PerAgent>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
     if (e != cudaSuccess) return ssd::set_error(SSD_ERR_CUDA, cudaGetErrorString(e));
     p->units = units;
     p->num_outputs = num_outputs;
     return SSD_OK;
 }
+
+#pragma GCC visibility push(default)
+extern "C" {
 
 int ssd_policy_set_head(ssd_policy_t p, int units, int num_outputs, const float* lstm_w, const float* lstm_u, const float* lstm_b,
                         const float* logits_w, const float* logits_b, const float* value_w, const float* value_b) {
@@ -320,6 +363,7 @@ int ssd_policy_lstm_heads(ssd_policy_t p, const float* features, const float* h_
                           float* value, int8_t* actions, int64_t num_agents, uint64_t seed, uint32_t counter, void* stream) {
     using namespace ssd::policy_head;
     if (!p || !features || !h_in || !c_in || !h_out || !c_out || !logits || !value || num_agents < 0) return ssd::set_error(SSD_ERR_INVALID, "bad argument");
+    if (p->pool) return ssd::set_error(SSD_ERR_INVALID, "a policy pool handle takes ssd_policy_pool_lstm_heads");
     if (!p->d_head_blob) return ssd::set_error(SSD_ERR_INVALID, "ssd_policy_set_head has not been called");
     const void* ptrs[5] = {features, h_in, c_in, h_out, c_out};
     for (const void* q : ptrs)
@@ -333,14 +377,39 @@ int ssd_policy_lstm_heads(ssd_policy_t p, const float* features, const float* h_
     if (np == 1) {
         const long long groups = (num_agents + GA - 1) / GA;
         const int grid = static_cast<int>(groups < p->sms ? groups : p->sms);
-        lstm_heads_kernel<false><<<grid, kThreads, kSmemBytes, st>>>(features, h_in, c_in, h_out, c_out, logits, value, actions, num_agents,
-                                                                    p->num_outputs, p->d_head_blob, s_lo, s_hi, counter, 1, grid);
+        lstm_heads_kernel<WeightMap::Shared><<<grid, kThreads, kSmemBytes, st>>>(features, h_in, c_in, h_out, c_out, logits, value, actions, num_agents,
+                                                                                p->num_outputs, p->d_head_blob, s_lo, s_hi, counter, 1, grid,
+                                                                                nullptr, nullptr, nullptr);
     } else {  // P * floor(#SMs / P) CTAs at most, each serving one policy
         const long long groups = (num_agents / np + GA - 1) / GA;
         const int per = static_cast<int>(groups < p->sms / np ? groups : p->sms / np);
-        lstm_heads_kernel<true><<<np * per, kThreads, kSmemBytes, st>>>(features, h_in, c_in, h_out, c_out, logits, value, actions, num_agents,
-                                                                       p->num_outputs, p->d_head_blob, s_lo, s_hi, counter, np, per);
+        lstm_heads_kernel<WeightMap::PerAgent><<<np * per, kThreads, kSmemBytes, st>>>(features, h_in, c_in, h_out, c_out, logits, value, actions,
+                                                                                      num_agents, p->num_outputs, p->d_head_blob, s_lo, s_hi, counter,
+                                                                                      np, per, nullptr, nullptr, nullptr);
     }
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return ssd::set_error(SSD_ERR_CUDA, cudaGetErrorString(e));
+    return SSD_OK;
+}
+
+int ssd_policy_pool_lstm_heads(ssd_policy_t p, const float* features, const uint8_t* policy_ids, const float* h_in, const float* c_in, float* h_out,
+                               float* c_out, float* logits, float* value, int8_t* actions, int64_t num_agents, uint64_t seed, uint32_t counter,
+                               void* stream) {
+    using namespace ssd::policy_head;
+    if (!p || !features || !policy_ids || !h_in || !c_in || !h_out || !c_out || !logits || !value || num_agents < 0)
+        return ssd::set_error(SSD_ERR_INVALID, "bad argument");
+    if (!p->pool) return ssd::set_error(SSD_ERR_INVALID, "not a policy pool handle (ssd_policy_create_pool)");
+    const void* ptrs[5] = {features, h_in, c_in, h_out, c_out};
+    for (const void* q : ptrs)
+        if (reinterpret_cast<uintptr_t>(q) % 16 != 0) return ssd::set_error(SSD_ERR_INVALID, "features and state pointers must be 16-byte aligned");
+    if (num_agents == 0) return SSD_OK;
+    const int rc = ssd::policy_pool::assign(p, policy_ids, num_agents, stream);   // sets the device
+    if (rc != SSD_OK) return rc;
+    const long long tiles = ssd::policy_pool::max_tiles(num_agents, p->num_policies);
+    const int grid = static_cast<int>(tiles < p->sms ? tiles : p->sms);
+    lstm_heads_kernel<WeightMap::Pool><<<grid, kThreads, kSmemBytes, static_cast<cudaStream_t>(stream)>>>(
+        features, h_in, c_in, h_out, c_out, logits, value, actions, num_agents, p->num_outputs, p->d_head_blob, static_cast<uint32_t>(seed),
+        static_cast<uint32_t>(seed >> 32), counter, p->num_policies, grid, p->d_perm, p->d_tiles, p->d_counts + 512);
     const cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return ssd::set_error(SSD_ERR_CUDA, cudaGetErrorString(e));
     return SSD_OK;

@@ -19,7 +19,15 @@ it as opaque between steps (as RLlib does with state_out -> state_in); `state_ro
 One network per agent id -- the reference's training scripts (run_scripts/train_baseline.py, train_moa.py) build a policy per
 'agent-i' and map agent i to it -- is `ConvToFCNet([weights_0, ..., weights_{P-1}])`: agent (b, p) of a [B, P, 15, 15, 3]
 observation tensor is evaluated with weights_p by the same two kernels (one CTA serves one policy), outputs stay agent-major,
-and the tiled state is grouped per policy, [P * ceil(B/128), 8, 128, 16].  Weights are numpy fp32 arrays in the Keras layouts (conv kernel [kh, kw, in, out], dense kernels [in, out], LSTM kernel
+and the tiled state is grouped per policy, [P * ceil(B/128), 8, 128, 16].
+
+A policy pool -- K <= 255 weight sets loaded once, and a uint8 policy id per agent with every call, as RLlib's
+policy_mapping_fn may assign them per agent and per episode -- is `PolicyPool([weights_0, ..., weights_{K-1}])`: several runs
+or seeds on one GPU, cross-play teams, population play.  The kernels group the agents by id on the device; an id >= K leaves
+the agent to the caller's own code (scripted agents).  Its state is the shared network's agent-major tiled layout, so the ids
+may change while a state is alive.
+
+Weights are numpy fp32 arrays in the Keras layouts (conv kernel [kh, kw, in, out], dense kernels [in, out], LSTM kernel
 [in, 4u] / recurrent kernel [u, 4u] / bias [4u] with gates ordered i, f, c, o), so a checkpoint of the reference model
 loads without transposition.  There is no CPU path: the trunk raises without the CUDA library.
 """
@@ -61,6 +69,50 @@ def random_weights(num_outputs, cell_size=128, seed=0):
     }
 
 
+def _cuda_device(device):
+    device = torch.device(device)
+    if device.type != "cuda":
+        raise _lib.SsdError("the policy trunk runs on a CUDA device only")
+    if device.index is None:  # 'cuda' means the current device, not device 0
+        device = torch.device("cuda", torch.cuda.current_device())
+    return device
+
+
+def _weight_sets(weights):
+    """One dict or a list of dicts -> the list of weight sets as contiguous fp32 arrays, checked to share names and shapes."""
+    sets = list(weights) if isinstance(weights, (list, tuple)) else [weights]
+    if not sets:
+        raise ValueError("no weight sets")
+    sets = [{k: np.ascontiguousarray(v, dtype=np.float32) for k, v in ws.items()} for ws in sets]
+    w = sets[0]
+    for name, shape in (("conv_w", (3, 3, 3, CONV_FILTERS)), ("conv_b", (CONV_FILTERS,)), ("fc1_w", (FLAT, FEATURES)),
+                        ("fc1_b", (FEATURES,)), ("fc2_w", (FEATURES, FEATURES)), ("fc2_b", (FEATURES,))):
+        if w[name].shape != shape:
+            raise ValueError("%s has shape %s, expected %s" % (name, w[name].shape, shape))
+    for p, ws in enumerate(sets[1:], 1):
+        if sorted(ws) != sorted(w) or any(ws[k].shape != w[k].shape for k in w):
+            raise ValueError("weights[%d] does not have the names and shapes of weights[0]" % p)
+    return sets
+
+
+def _state_rows(state, m, P):
+    """Tiled state [G, 8, 128, 16] (grouped per policy for P > 1) -> agent-major [m, cell_size] (a copy)."""
+    g, b, r, e = state.shape
+    rows = state.permute(0, 2, 1, 3).reshape(g * r, b * e)
+    if P == 1:
+        return rows[:m].contiguous()
+    return rows.reshape(P, g // P * r, b * e)[:, :m // P].transpose(0, 1).reshape(m, b * e)   # (p, b) -> agent b * P + p
+
+
+def _state_from_rows(rows, P):
+    """Agent-major [m, cell_size] -> tiled state [P * ceil(m / P / 128), cell_size/16, 128, 16], zero padded."""
+    m, u = rows.shape
+    g = (m // P + 127) // 128
+    full = torch.zeros((P, g * 128, u), dtype=rows.dtype, device=rows.device)
+    full[:, :m // P] = rows.reshape(m // P, P, u).transpose(0, 1)
+    return full.reshape(P * g, 128, u // 16, 16).permute(0, 2, 1, 3).contiguous()
+
+
 class ConvToFCNet(object):
     """Forward pass of ConvToFCNetv2 for a batch of agents; `obs` is the uint8 tensor of the step path.
 
@@ -69,23 +121,9 @@ class ConvToFCNet(object):
     (cell_size 128, 1..15 outputs)."""
 
     def __init__(self, weights, device="cuda:0"):
-        self.device = torch.device(device)
-        if self.device.type != "cuda":
-            raise _lib.SsdError("the policy trunk runs on a CUDA device only")
-        if self.device.index is None:  # 'cuda' means the current device, not device 0
-            self.device = torch.device("cuda", torch.cuda.current_device())
-        sets = list(weights) if isinstance(weights, (list, tuple)) else [weights]
-        if not sets:
-            raise ValueError("no weight sets")
-        sets = [{k: np.ascontiguousarray(v, dtype=np.float32) for k, v in ws.items()} for ws in sets]
+        self.device = _cuda_device(device)
+        sets = _weight_sets(weights)
         w = sets[0]
-        for name, shape in (("conv_w", (3, 3, 3, CONV_FILTERS)), ("conv_b", (CONV_FILTERS,)), ("fc1_w", (FLAT, FEATURES)),
-                            ("fc1_b", (FEATURES,)), ("fc2_w", (FEATURES, FEATURES)), ("fc2_b", (FEATURES,))):
-            if w[name].shape != shape:
-                raise ValueError("%s has shape %s, expected %s" % (name, w[name].shape, shape))
-        for p, ws in enumerate(sets[1:], 1):
-            if sorted(ws) != sorted(w) or any(ws[k].shape != w[k].shape for k in w):
-                raise ValueError("weights[%d] does not have the names and shapes of weights[0]" % p)
         self.num_policies = P = len(sets)
         self.weights = w if P == 1 and not isinstance(weights, (list, tuple)) else sets
         self.cell_size = w["lstm_u"].shape[0] if "lstm_u" in w else 0
@@ -161,22 +199,13 @@ class ConvToFCNet(object):
         """Tiled state [G, 8, 128, 16] -> agent-major [m, cell_size] (a copy)."""
         if state.dim() == 2:
             return state[:m]
-        g, b, r, e = state.shape
-        rows = state.permute(0, 2, 1, 3).reshape(g * r, b * e)
-        P = self.num_policies
-        if P == 1:
-            return rows[:m].contiguous()
         self._groups(m)
-        return rows.reshape(P, g // P * r, b * e)[:, :m // P].transpose(0, 1).reshape(m, b * e)   # (p, b) -> agent b * P + p
+        return _state_rows(state, m, self.num_policies)
 
     def state_from_rows(self, rows):
         """Agent-major [m, cell_size] -> tiled state [G, cell_size/16, 128, 16] (G = ceil(m/128), per policy for P > 1), zero padded."""
-        m, u = rows.shape
-        P = self.num_policies
-        g = self._groups(m) // P
-        full = torch.zeros((P, g * 128, u), dtype=rows.dtype, device=rows.device)
-        full[:, :m // P] = rows.reshape(m // P, P, u).transpose(0, 1)
-        return full.reshape(P * g, 128, u // 16, 16).permute(0, 2, 1, 3).contiguous()
+        self._groups(rows.shape[0])
+        return _state_from_rows(rows, self.num_policies)
 
     def seed_sampling(self, seed):
         """Key of the Philox streams `act` samples from (counter = number of `act` calls since)."""
@@ -233,4 +262,108 @@ class ConvToFCNet(object):
             return a, value, h, c
         logits, value, h, c = self.forward(obs, h, c)
         a = torch.multinomial(torch.softmax(logits, dim=1), 1, generator=generator).squeeze(1).to(torch.int8)
+        return a, value, h, c
+
+
+class PolicyPool(object):
+    """K weight sets (1 <= K <= 255, each a dict as for ConvToFCNet) loaded once; every call takes `policy_ids`, a uint8 tensor
+    on the device of shape obs.shape[:-3]: agent m is evaluated with weight_sets[policy_ids[m]], and the ids may differ from
+    call to call.  An id >= K means "no pool policy": nothing is written for that agent (its rows of features, logits, value,
+    h' and c' are left as they were in the output buffers, which `forward` allocates uninitialised) and `act` returns -1
+    for it, so the caller drives it with its own code.  The recurrent state is the shared network's tiled layout
+    [ceil(M/128), 8, 128, 16], independent of the ids; an agent that was skipped wants a fresh state row (state_from_rows)
+    before it returns to a pool policy.  Needs the fused head (cell_size 128, 1..15 outputs).  The id values are checked on
+    the device only (a host check would synchronise).  Calls on one pool must be ordered on one stream: the grouping of the
+    agents by id uses scratch that belongs to the pool."""
+
+    def __init__(self, weight_sets, device="cuda:0"):
+        self.device = _cuda_device(device)
+        sets = _weight_sets(weight_sets if isinstance(weight_sets, (list, tuple)) else [weight_sets])
+        w = sets[0]
+        self.num_policies = len(sets)
+        self.cell_size = w["lstm_u"].shape[0] if "lstm_u" in w else 0
+        self.num_outputs = w["logits_w"].shape[1] if "logits_w" in w else 0
+        if self.cell_size != 128 or not 1 <= self.num_outputs <= 15:
+            raise ValueError("a policy pool needs the fused head: cell_size 128 and 1..15 outputs (got %d, %d)" % (self.cell_size, self.num_outputs))
+        w = {k: np.ascontiguousarray(np.stack([ws[k] for ws in sets])) for k in w}   # K consecutive arrays behind every pointer
+        ptr = lambda a: a.ctypes.data_as(C.c_void_p)
+        names = ("conv_w", "conv_b", "fc1_w", "fc1_b", "fc2_w", "fc2_b", "lstm_w", "lstm_u", "lstm_b", "logits_w", "logits_b", "value_w", "value_b")
+        self._h = C.c_void_p()
+        _lib.check(_lib.lib.ssd_policy_create_pool(VIEW_RADIUS, self.device.index, self.num_policies, self.cell_size, self.num_outputs,
+                                                   *[ptr(w[k]) for k in names], C.byref(self._h)))
+        self._sample_seed, self._sample_counter = 0, 0
+
+    def close(self):
+        if self._h:
+            _lib.lib.ssd_policy_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def _ids(self, obs, policy_ids):
+        if obs.dtype != torch.uint8 or obs.device != self.device or obs.dim() < 4 or tuple(obs.shape[-3:]) != (OBS_SIDE, OBS_SIDE, 3):
+            raise ValueError("obs must be a uint8 [..., %d, %d, 3] tensor on %s" % (OBS_SIDE, OBS_SIDE, self.device))
+        if not isinstance(policy_ids, torch.Tensor) or policy_ids.dtype != torch.uint8 or policy_ids.device != self.device \
+                or tuple(policy_ids.shape) != tuple(obs.shape[:-3]):
+            raise ValueError("policy_ids must be a uint8 tensor of shape %s on %s" % (tuple(obs.shape[:-3]), self.device))
+        return obs.contiguous(), policy_ids.contiguous()
+
+    def features(self, obs, policy_ids, out=None):
+        """uint8 [..., 15, 15, 3] + uint8 ids [...] on the device -> float32 [M, 32], agent-major."""
+        obs, ids = self._ids(obs, policy_ids)
+        m = ids.numel()
+        if out is None:
+            out = torch.empty((m, FEATURES), dtype=torch.float32, device=self.device)
+        stream = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+        _lib.check(_lib.lib.ssd_policy_pool_features(self._h, C.c_void_p(obs.data_ptr()), C.c_void_p(ids.data_ptr()), m,
+                                                     C.c_void_p(out.data_ptr()), stream))
+        return out
+
+    def initial_state(self, m):
+        """Zero (h, c) for m agents in the tiled layout [ceil(m/128), 8, 128, 16]."""
+        z = torch.zeros(((m + 127) // 128, self.cell_size // 16, 128, 16), dtype=torch.float32, device=self.device)
+        return z, z.clone()
+
+    def state_rows(self, state, m):
+        """Tiled state -> agent-major [m, 128] (a copy)."""
+        return _state_rows(state, m, 1)
+
+    def state_from_rows(self, rows):
+        """Agent-major [m, 128] -> tiled state [ceil(m/128), 8, 128, 16], zero padded."""
+        return _state_from_rows(rows, 1)
+
+    def seed_sampling(self, seed):
+        """Key of the Philox streams `act` samples from (counter = number of `act` calls since)."""
+        self._sample_seed, self._sample_counter = int(seed) & (2 ** 64 - 1), 0
+
+    def _run(self, obs, policy_ids, h, c, sample):
+        obs, ids = self._ids(obs, policy_ids)
+        x = self.features(obs, ids)
+        m = x.shape[0]
+        if h.dim() != 4 or h.shape[0] * 128 < m or h.shape != c.shape:
+            raise ValueError("(h, c) must be in the tiled layout of initial_state / state_from_rows")
+        h, c = h.contiguous(), c.contiguous()
+        h_new, c_new = torch.empty_like(h), torch.empty_like(c)
+        logits = torch.empty((m, self.num_outputs), dtype=torch.float32, device=self.device)
+        value = torch.empty((m,), dtype=torch.float32, device=self.device)
+        actions = torch.full((m,), -1, dtype=torch.int8, device=self.device) if sample else None
+        stream = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+        p = lambda t: C.c_void_p(t.data_ptr() if t is not None else None)
+        _lib.check(_lib.lib.ssd_policy_pool_lstm_heads(self._h, p(x), p(ids), p(h), p(c), p(h_new), p(c_new), p(logits), p(value), p(actions),
+                                                       m, self._sample_seed, self._sample_counter & 0xFFFFFFFF, stream))
+        if sample:
+            self._sample_counter += 1
+        return logits, value, h_new, c_new, actions
+
+    def forward(self, obs, policy_ids, h, c):
+        """-> (logits [M, A], value [M], h', c'), all float32; rows of skipped agents are not written."""
+        return self._run(obs, policy_ids, h, c, sample=False)[:4]
+
+    def act(self, obs, policy_ids, h, c):
+        """Sample int8 actions [M] on the device (Philox streams, see `seed_sampling`); -1 for skipped agents."""
+        logits, value, h, c, a = self._run(obs, policy_ids, h, c, sample=True)
         return a, value, h, c
