@@ -78,6 +78,13 @@ def _cuda_device(device):
     return device
 
 
+def _aligned(t):
+    """`t` contiguous and starting on a 16-byte boundary, as the C ABI requires: a view such as obs[1:] is contiguous but starts
+    inside its allocation (675 bytes in), so it is copied."""
+    t = t.contiguous()
+    return t if t.data_ptr() % 16 == 0 else t.clone()
+
+
 def _weight_sets(weights):
     """One dict or a list of dicts -> the list of weight sets as contiguous fp32 arrays, checked to share names and shapes."""
     sets = list(weights) if isinstance(weights, (list, tuple)) else [weights]
@@ -181,7 +188,7 @@ class ConvToFCNet(object):
         if P > 1 and not (obs.dim() == 4 and obs.shape[0] % P == 0 or obs.dim() == 5 and obs.shape[1] == P):
             raise ValueError("a network of %d per-agent policies takes obs [B, %d, %d, %d, 3] or [B * %d, %d, %d, 3], not %s"
                              % (P, P, OBS_SIDE, OBS_SIDE, P, OBS_SIDE, OBS_SIDE, tuple(obs.shape)))
-        obs = obs.contiguous()
+        obs = _aligned(obs)
         m = obs.numel() // (OBS_SIDE * OBS_SIDE * 3)
         if out is None:
             out = torch.empty((m, FEATURES), dtype=torch.float32, device=self.device)
@@ -216,7 +223,7 @@ class ConvToFCNet(object):
         m = x.shape[0]
         if h.dim() != 4 or (h.shape[0] * 128 < m if self.num_policies == 1 else h.shape[0] != self._groups(m)):
             raise ValueError("the fused route carries (h, c) in the tiled layout of initial_state / state_from_rows")
-        h, c = h.contiguous(), c.contiguous()
+        h, c = _aligned(h), _aligned(c)
         h_new, c_new = torch.empty_like(h), torch.empty_like(c)
         logits = torch.empty((m, self.num_outputs), dtype=torch.float32, device=self.device)
         value = torch.empty((m,), dtype=torch.float32, device=self.device)
@@ -249,7 +256,7 @@ class ConvToFCNet(object):
         h16 = torch.empty((m, u), dtype=torch.bfloat16, device=self.device)
         stream = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
         p = lambda t: C.c_void_p(t.data_ptr())
-        _lib.check(_lib.lib.ssd_policy_lstm_cell(p(gates), p(hd["lstm_b"]), p(c.contiguous()), p(c_new), p(h_new), p(h16), m, u, stream))
+        _lib.check(_lib.lib.ssd_policy_lstm_cell(p(gates), p(hd["lstm_b"]), p(_aligned(c)), p(c_new), p(h_new), p(h16), m, u, stream))
         logits = torch.mm(h16, hd["logits_w"]).float() + hd["logits_b"]
         value = (torch.mm(h16, hd["value_w"]).float() + hd["value_b"]).squeeze(1)
         return logits, value, h_new, c_new
@@ -310,7 +317,7 @@ class PolicyPool(object):
         if not isinstance(policy_ids, torch.Tensor) or policy_ids.dtype != torch.uint8 or policy_ids.device != self.device \
                 or tuple(policy_ids.shape) != tuple(obs.shape[:-3]):
             raise ValueError("policy_ids must be a uint8 tensor of shape %s on %s" % (tuple(obs.shape[:-3]), self.device))
-        return obs.contiguous(), policy_ids.contiguous()
+        return _aligned(obs), policy_ids.contiguous()
 
     def features(self, obs, policy_ids, out=None):
         """uint8 [..., 15, 15, 3] + uint8 ids [...] on the device -> float32 [M, 32], agent-major."""
@@ -346,7 +353,7 @@ class PolicyPool(object):
         m = x.shape[0]
         if h.dim() != 4 or h.shape[0] * 128 < m or h.shape != c.shape:
             raise ValueError("(h, c) must be in the tiled layout of initial_state / state_from_rows")
-        h, c = h.contiguous(), c.contiguous()
+        h, c = _aligned(h), _aligned(c)
         h_new, c_new = torch.empty_like(h), torch.empty_like(c)
         logits = torch.empty((m, self.num_outputs), dtype=torch.float32, device=self.device)
         value = torch.empty((m,), dtype=torch.float32, device=self.device)

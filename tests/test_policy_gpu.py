@@ -60,38 +60,59 @@ def _reference_forward(w, obs, h, c):
     return h @ t("logits_w") + t("logits_b"), (h @ t("value_w") + t("value_b")).squeeze(1), h, c
 
 
-def test_forward_matches_fp32_reference_over_steps():
-    """Three recurrent steps: bf16 GEMM operands and the fused cell update against the fp32 reference carried alongside."""
+def _check_forward_over_steps(cell_size, num_outputs):
+    """Three recurrent steps against the fp32 reference and the float64 oracle carried alongside.  cell_size 128 with 1..15
+    outputs takes the fused kernel (fp16 operands, tanh.approx) -- 15 outputs put the value in the last of its 16 head columns,
+    1 output in column 1 -- and is also run through forward_unfused; every other shape takes the unfused route only (bf16
+    GEMM operands around the one-pass cell update)."""
     from sequential_social_dilemma_games_b200 import policy
     torch.backends.cuda.matmul.allow_tf32 = False
     torch.backends.cudnn.allow_tf32 = False
-    m = 1000
-    w = policy.random_weights(num_outputs=9, cell_size=128, seed=11)
+    m, u = 1000, cell_size
+    fused = cell_size == 128 and num_outputs <= 15
+    w = policy.random_weights(num_outputs=num_outputs, cell_size=cell_size, seed=11)
     net = policy.ConvToFCNet(w)
+    assert net._fused_head == fused
     g = torch.Generator(device="cuda").manual_seed(5)
-    h, c = net.initial_state(m)                                 # tiled layout of the fused kernel
-    assert h.shape == (8, 8, 128, 16)
-    hr, cr = torch.zeros((m, 128), device="cuda"), torch.zeros((m, 128), device="cuda")
+    h, c = net.initial_state(m)                                 # tiled layout of the fused kernel, [m, u] rows otherwise
+    assert h.shape == ((8, 8, 128, 16) if fused else (m, u))
+    hr, cr = torch.zeros((m, u), device="cuda"), torch.zeros((m, u), device="cuda")
     hu, cu = hr.clone(), cr.clone()
     from oracle import policy_ref
-    h64, c64 = np.zeros((m, 128)), np.zeros((m, 128))
-    assert torch.equal(net.state_rows(net.state_from_rows(torch.arange(m * 128.0, device="cuda").reshape(m, 128)), m),
-                       torch.arange(m * 128.0, device="cuda").reshape(m, 128))
+    h64, c64 = np.zeros((m, u)), np.zeros((m, u))
+    if fused:
+        assert torch.equal(net.state_rows(net.state_from_rows(torch.arange(m * 128.0, device="cuda").reshape(m, 128)), m),
+                           torch.arange(m * 128.0, device="cuda").reshape(m, 128))
     for _ in range(3):
         obs = torch.randint(0, 256, (m, 15, 15, 3), dtype=torch.uint8, device="cuda", generator=g)
-        logits, value, h, c = net.forward(obs, h, c)            # fused tcgen05 LSTM + heads (cell_size 128)
+        logits, value, h, c = net.forward(obs, h, c)            # fused tcgen05 LSTM + heads, or the unfused route
         l2, v2, h2, c2 = net.forward_unfused(obs, hu, cu)       # library GEMMs + one-pass cell update
         hu, cu = h2, c2
         lr, vr, hr, cr = _reference_forward(w, obs, hr, cr)
         l64, v64, h64, c64 = policy_ref.forward(w, obs.cpu().numpy(), h64, c64)   # float64 numpy oracle carried alongside
-        assert logits.shape == (m, 9) and value.shape == (m,)
+        assert logits.shape == (m, num_outputs) and value.shape == (m,)
         for got, want, w64 in ((logits, lr, l64), (value, vr, v64), (net.state_rows(h, m), hr, h64), (net.state_rows(c, m), cr, c64)):
-            assert (got - want).abs().max().item() < FWD_TOL, (got - want).abs().max().item()   # fp16 operands, fp32 accumulation, tanh.approx
-            assert np.abs(got.cpu().numpy().astype(np.float64) - w64).max() < FWD_TOL
             assert np.abs(want.cpu().numpy().astype(np.float64) - w64).max() < 2e-4           # torch fp32 vs float64: the checkers agree
+            if fused:   # fp16 operands, fp32 accumulation, tanh.approx
+                assert (got - want).abs().max().item() < FWD_TOL, (got - want).abs().max().item()
+                assert np.abs(got.cpu().numpy().astype(np.float64) - w64).max() < FWD_TOL
+            else:       # the unfused route: bf16 operands, 8 significant bits
+                assert torch.allclose(got, want, atol=3e-2, rtol=3e-2), (got - want).abs().max().item()
+                assert np.allclose(got.cpu().numpy().astype(np.float64), w64, atol=3e-2, rtol=3e-2)
         for got, want in ((l2, lr), (v2, vr), (h2, hr), (c2, cr)):
             assert torch.allclose(got, want, atol=3e-2, rtol=3e-2), (got - want).abs().max().item()   # bf16 operands: 8 significant bits
+    assert lr.abs().max().item() > 0.01 and vr.abs().max().item() > 0.01   # not vacuous
     net.close()
+
+
+def test_forward_matches_fp32_reference_over_steps():
+    _check_forward_over_steps(cell_size=128, num_outputs=9)
+
+
+@pytest.mark.parametrize("cell_size,num_outputs", [(128, 1), (128, 15), (128, 16), (8, 3), (24, 5), (64, 8), (256, 8)])
+def test_forward_matches_fp32_reference_every_head_width(cell_size, num_outputs):
+    """1 and 15 outputs on the fused head, 16 outputs (the unfused fallback), and cell sizes 8, 24, 64, 256 (unfused)."""
+    _check_forward_over_steps(cell_size, num_outputs)
 
 
 def test_fused_sampling_follows_softmax():

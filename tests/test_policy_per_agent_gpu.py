@@ -93,19 +93,21 @@ def test_state_rows_round_trip():
     per.close()
 
 
-def _distinct(P=5):
+def _distinct(P=5, num_outputs=NUM_OUTPUTS):
     policy = _policy()
-    return [policy.random_weights(num_outputs=NUM_OUTPUTS, seed=100 + p) for p in range(P)]
+    return [policy.random_weights(num_outputs=num_outputs, seed=100 + p) for p in range(P)]
 
 
-@pytest.mark.parametrize("B", [1, 129, 1000])
-def test_distinct_weights_match_separate_nets(B):
+@pytest.mark.parametrize("B,num_outputs", [pytest.param(B, NUM_OUTPUTS, id=str(B)) for B in (1, 129, 1000)]
+                         + [pytest.param(B, A, id="%d-outputs%d" % (B, A)) for A in (1, 15) for B in (1, 129, 1000)])
+def test_distinct_weights_match_separate_nets(B, num_outputs):
     """Column p of a P = 5 network == ConvToFCNet(weights[p]) on obs[:, p], bitwise (features, three recurrent steps), and
-    within the kernels' tolerances of the float64 oracle with weights[p]."""
+    within the kernels' tolerances of the float64 oracle with weights[p].  1 and 15 outputs put the value in head column 1 and
+    15, which the per-agent head selects with code of its own."""
     from oracle import policy_ref
     policy = _policy()
     P, M = 5, B * 5
-    ws = _distinct(P)
+    ws = _distinct(P, num_outputs)
     per = policy.ConvToFCNet(ws)
     singles = [policy.ConvToFCNet(w) for w in ws]
     steps = _obs_steps("random", B, P, None, seed=B)
@@ -122,7 +124,7 @@ def test_distinct_weights_match_separate_nets(B):
         logits, value, hp2, cp2 = per.forward(obs, hp, cp)
         hp, cp = hp2, cp2
         rows_h, rows_c = per.state_rows(hp2, M).reshape(B, P, 128), per.state_rows(cp2, M).reshape(B, P, 128)
-        logits, value = logits.reshape(B, P, NUM_OUTPUTS), value.reshape(B, P)
+        logits, value = logits.reshape(B, P, num_outputs), value.reshape(B, P)
         for p in range(P):
             col = obs[:, p].clone()
             l1, v1, h1, c1 = singles[p].forward(col, *hs[p])

@@ -21,9 +21,9 @@ def _policy():
     return policy
 
 
-def _sets(K, seed=300):
+def _sets(K, seed=300, num_outputs=NUM_OUTPUTS):
     policy = _policy()
-    return [policy.random_weights(num_outputs=NUM_OUTPUTS, seed=seed + k) for k in range(K)]
+    return [policy.random_weights(num_outputs=num_outputs, seed=seed + k) for k in range(K)]
 
 
 @pytest.fixture(scope="module")
@@ -50,8 +50,8 @@ def env_obs():
 
 
 def _obs_steps(source, M, env_obs, seed):
-    if source == "env":
-        return [o[:M].contiguous() for o in env_obs]
+    if source == "env":   # beyond the recorded agents, the recorded observations again
+        return [o.repeat((M + o.shape[0] - 1) // o.shape[0], 1, 1, 1)[:M].contiguous() for o in env_obs]
     g = torch.Generator(device="cuda").manual_seed(seed)
     return [torch.randint(0, 256, (M, 15, 15, 3), dtype=torch.uint8, device="cuda", generator=g) for _ in range(3)]
 
@@ -99,7 +99,8 @@ def _run_pool(pool, steps, ids_per_step, seed, h=None, c=None):
         f = pool.features(obs, ids)
         lg, v, h2, c2 = pool.forward(obs, ids, h, c)
         a, v2, h, c = pool.act(obs, ids, h, c)
-        assert torch.equal(v2, v)
+        live = ids.reshape(-1).long() < pool.num_policies   # the value of a skipped agent is not written
+        assert torch.equal(v2[live], v[live])
         res.append((f, lg, v, pool.state_rows(h2, m), pool.state_rows(c2, m), a, h, c))
     return res
 
@@ -113,10 +114,11 @@ def _check_against_reference(sets, steps, ids_per_step, seed=77):
     got = _run_pool(pool, steps, ids_per_step, seed)
     h, c = pool.initial_state(m)
     for t, (obs, ids) in enumerate(zip(steps, ids_per_step)):
-        assert int(ids.max()) < len(sets)
+        live = ids.reshape(-1).long() < len(sets)   # the pool writes nothing but action -1 for the other agents
         want = ref.step(obs, ids, h, c)
-        for name, g, w in zip(("features", "logits", "value", "h", "c", "actions"), got[t][:6], want):
-            assert torch.equal(g, w), (t, name)
+        for name, g, w in zip(("features", "logits", "value", "h", "c"), got[t][:5], want):
+            assert torch.equal(g[live], w[live]), (t, name)
+        assert torch.equal(got[t][5], want[5]), (t, "actions")
         h, c = pool.state_from_rows(want[3]), pool.state_from_rows(want[4])
     pool.close()
     ref.close()
@@ -180,30 +182,41 @@ def test_identity_mapping_equals_per_agent_net(N, source, env_obs):
     pool.close()
 
 
-def _ids_with_sizes(M, K, sizes, seed):
-    """uint8 [M]: policy k holds exactly sizes[k] agents for the policies in `sizes`, the others share the rest at random."""
+def _ids_with_sizes(M, K, sizes, seed, skipped=0):
+    """uint8 [M]: policy k holds exactly sizes[k] agents for the policies in `sizes`, `skipped` agents have an id >= K, the
+    other policies share the rest at random."""
     rng = np.random.RandomState(seed)
-    fixed = np.concatenate([np.full(n, k) for k, n in sizes.items()]) if sizes else np.zeros(0)
+    fixed = np.concatenate([np.full(n, k) for k, n in sizes.items()] + [rng.randint(K, 256, skipped)])
     others = np.array([k for k in range(K) if k not in sizes])
     ids = np.concatenate([fixed, rng.choice(others, M - len(fixed))])
     rng.shuffle(ids)
     return torch.from_numpy(ids.astype(np.uint8)).cuda()
 
 
-@pytest.mark.parametrize("K,sizes", [
-    (3, {0: 129, 1: 0}),                                # policy 2 takes the rest
-    (3, {1: 1, 2: 127}),
-    (40, {0: 0, 1: 1, 2: 127, 3: 128, 4: 129}),
-    (255, {7: 127, 8: 128, 9: 129, 10: 1, 11: 0}),
+SCALE_M = 65536 * 5   # 65 536 Harvest envs x 5 agents: a CTA of the trunk and head runs many tiles, the assignment 80 chunks
+
+
+@pytest.mark.parametrize("K,sizes,M", [
+    pytest.param(3, {0: 129, 1: 0}, 5123, id="3-sizes0"),                               # policy 2 takes the rest
+    pytest.param(3, {1: 1, 2: 127}, 5123, id="3-sizes1"),
+    pytest.param(40, {0: 0, 1: 1, 2: 127, 3: 128, 4: 129}, 5123, id="40-sizes2"),
+    pytest.param(255, {7: 127, 8: 128, 9: 129, 10: 1, 11: 0}, 5123, id="255-sizes3"),
+    pytest.param(3, {0: 129, 1: 0}, SCALE_M, id="3-sizes0-M327680"),                     # long same-policy segments
+    pytest.param(255, {7: 127, 8: 128, 9: 129, 10: 1, 11: 0}, SCALE_M, id="255-sizes3-M327680"),   # many switches per CTA
 ])
 @pytest.mark.parametrize("source", ["random", "env"])
-def test_random_ids_match_rowwise_reference(K, sizes, source, env_obs):
-    M = 5123
+def test_random_ids_match_rowwise_reference(K, sizes, M, source, env_obs):
+    """At 327 680 agents about 1 % of the ids are >= K (skipped)."""
+    skipped = M // 100 if M == SCALE_M else 0
     steps = _obs_steps(source, M, env_obs, seed=K)
-    ids = _ids_with_sizes(M, K, sizes, seed=K)
-    counts = torch.bincount(ids.long(), minlength=K).cpu().numpy()
+    ids = _ids_with_sizes(M, K, sizes, seed=K, skipped=skipped)
+    counts = torch.bincount(ids.long(), minlength=256).cpu().numpy()
+    assert counts[K:].sum() == skipped
     for k, n in sizes.items():
         assert counts[k] == n
+    sms = torch.cuda.get_device_properties(torch.cuda.current_device()).multi_processor_count
+    if M == SCALE_M:   # every CTA of the trunk and the head runs at least four tiles
+        assert sum((int(n) + 127) // 128 for n in counts[:K]) >= 4 * sms
     _check_against_reference(_sets(K), steps, [ids] * 3)
 
 
@@ -271,10 +284,20 @@ def test_skipped_agents_are_not_written():
 
 
 def test_matches_float64_oracle():
+    _check_float64_oracle(NUM_OUTPUTS)
+
+
+@pytest.mark.parametrize("num_outputs", [1, 15])
+def test_matches_float64_oracle_head_widths(num_outputs):
+    """The value in head column 1 and 15: the pool head selects it with code of its own."""
+    _check_float64_oracle(num_outputs)
+
+
+def _check_float64_oracle(num_outputs):
     from oracle import policy_ref
     policy = _policy()
     K, M = 3, 600
-    sets = _sets(K)
+    sets = _sets(K, num_outputs=num_outputs)
     pool = policy.PolicyPool(sets)
     steps = _obs_steps("random", M, None, seed=12)
     ids = torch.randint(0, K, (M,), dtype=torch.uint8, device="cuda", generator=torch.Generator(device="cuda").manual_seed(12))
