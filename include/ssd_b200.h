@@ -257,6 +257,32 @@ int ssd_policy_pool_features(ssd_policy_t p, const uint8_t* obs, const uint8_t* 
 int ssd_policy_pool_lstm_heads(ssd_policy_t p, const float* features, const uint8_t* policy_ids, const float* h_in, const float* c_in, float* h_out,
                                float* c_out, float* logits, float* value, int8_t* actions, int64_t num_agents, uint64_t seed, uint32_t counter,
                                void* stream);
+/* The policy's distribution at the chosen action, in the same kernel: ssd_policy_lstm_heads / ssd_policy_pool_lstm_heads (same
+ * handles, state layouts and rules; the _dist form of each rejects the other kind of handle) that also return, per agent,
+ *   logp    dev f32[M] or NULL: log softmax(logits)[a] = l[a] - logsumexp(l) of the agent's action a, computed from the fp32
+ *           logits the call writes (max subtracted first, accurate expf / logf);
+ *   entropy dev f32[M] or NULL: -sum_i softmax(l)_i log softmax(l)_i.
+ * `mode` chooses the action a:
+ *   SSD_ACT_SAMPLE  the Gumbel-max sampler of ssd_policy_lstm_heads: with the same seed and counter the actions are bitwise those
+ *                   of the plain entry point; written to actions dev i8[M];
+ *   SSD_ACT_GREEDY  the first index of the maximum of the fp32 logits as written (np.argmax of them where they are
+ *                   finite; a NaN logit is passed over unless it is the first); written to actions;
+ *   SSD_ACT_GIVEN   actions dev i8[M] is an INPUT and is not written (a scripted agent, another policy's action, a recorded
+ *                   trajectory: the pi(a) of an importance ratio); a value outside 0..num_outputs-1 (-1 included) gives logp NaN
+ *                   for that agent and changes nothing else.
+ * logits, value, h_out and c_out are exactly what the plain entry point writes; a pool's agents with an id >= K get nothing
+ * written, logp and entropy included.  logp is the model's probability of the action; in SSD_ACT_SAMPLE it is not the
+ * sampler's realised frequency, which deviates where the sampler's fast -log(u) is inexact for u close to 1.  A mode outside
+ * the three, NULL actions, or a handle of the other kind returns SSD_ERR_INVALID before anything is launched. */
+#define SSD_ACT_SAMPLE 0
+#define SSD_ACT_GREEDY 1
+#define SSD_ACT_GIVEN 2
+int ssd_policy_lstm_heads_dist(ssd_policy_t p, const float* features, const float* h_in, const float* c_in, float* h_out, float* c_out,
+                               float* logits, float* value, int mode, int8_t* actions, float* logp, float* entropy, int64_t num_agents,
+                               uint64_t seed, uint32_t counter, void* stream);
+int ssd_policy_pool_lstm_heads_dist(ssd_policy_t p, const float* features, const uint8_t* policy_ids, const float* h_in, const float* c_in,
+                                    float* h_out, float* c_out, float* logits, float* value, int mode, int8_t* actions, float* logp,
+                                    float* entropy, int64_t num_agents, uint64_t seed, uint32_t counter, void* stream);
 /* The unfused alternative for other cell sizes: LSTM cell update after the gate GEMM (conv_to_fcnet_v2.py:68-80; Keras gate order i, f, c~, o; sigmoid recurrent
  * activation): gates dev bf16[num_agents][4*units] = x W + h U without the bias, bias dev f32[4*units],
  * c_prev / c_out / h_out dev f32[num_agents][units] (c_out may alias c_prev), h_bf16_out dev bf16[num_agents][units]

@@ -74,12 +74,18 @@ __device__ __forceinline__ float sigmoid_fast(float x) { return fmaf(tanh_fast(0
 // CTA c takes tiles [c T / G, (c + 1) T / G) and reloads the resident weights when the policy changes (the tiles are in
 // policy order).  Feature rows are gathered by perm, h and c are read and written per agent in the agent-major tiled layout
 // (64-byte pieces, one per 16 units), outputs go to row m.
-template <WeightMap kMap>
+//
+// kDist (ssd_policy_lstm_heads_dist): the action is chosen by `mode` (SSD_ACT_SAMPLE: the sampler above; SSD_ACT_GREEDY: the
+// first argmax of the logits; SSD_ACT_GIVEN: read from `actions`, which is then not written), and the epilogue adds
+// logp = l[a] - logsumexp(l) of that action and the entropy of softmax(l), from the fp32 logits it writes (accurate expf /
+// logf, at most 15 of each per agent).  Without kDist these parameters are unused and the code is that of the plain head.
+template <WeightMap kMap, bool kDist>
 __global__ void __launch_bounds__(kThreads, 1)
 lstm_heads_kernel(const float* __restrict__ feat, const float* h_in, const float* c_in, float* h_out, float* c_out, float* __restrict__ logits,
                   float* __restrict__ value, int8_t* __restrict__ actions, long long M, int num_outputs, const uint8_t* __restrict__ blob,
                   uint32_t seed_lo, uint32_t seed_hi, uint32_t counter, int num_policies, int ctas_per_policy, const uint32_t* __restrict__ perm,
-                  const PoolTile* __restrict__ tiles, const uint32_t* __restrict__ num_tiles) {
+                  const PoolTile* __restrict__ tiles, const uint32_t* __restrict__ num_tiles, int mode, float* __restrict__ logp,
+                  float* __restrict__ entropy) {
     constexpr bool kPerAgent = kMap != WeightMap::Shared, kPool = kMap == WeightMap::Pool;
     extern __shared__ __align__(128) uint8_t smem[];
     __shared__ uint32_t s_tmem;
@@ -250,12 +256,14 @@ lstm_heads_kernel(const float* __restrict__ feat, const float* h_in, const float
                 float best = -3.0e38f;
                 int arg = 0;
                 uint4 rnd = make_uint4(0, 0, 0, 0);
+                float lv[NH - 1];   // kDist: the logits as written
 #pragma unroll
                 for (int a = 0; a < NH - 1; ++a) {
                     if (a < num_outputs) {
                         const float l = __uint_as_float(y[a]) + hb[a];
                         logits[m * num_outputs + a] = l;
-                        if (actions != nullptr) {  // Gumbel-max: argmax(l - log(-log u)), u uniform in (0, 1)
+                        if (kDist) lv[a] = l;
+                        if (kDist ? mode == SSD_ACT_SAMPLE : actions != nullptr) {  // Gumbel-max: argmax(l - log(-log u)), u uniform in (0, 1)
                             if ((a & 3) == 0) rnd = philox4x32_10(static_cast<uint32_t>(m), static_cast<uint32_t>(m >> 32), counter, a >> 2, seed_lo, seed_hi);
                             const float u = (static_cast<float>(pick_word(rnd, a & 3) >> 8) + 0.5f) * (1.0f / 16777216.0f);
                             const float s = l - __logf(-__logf(u));
@@ -275,7 +283,30 @@ lstm_heads_kernel(const float* __restrict__ feat, const float* h_in, const float
                     }
                 }
                 value[m] = v;
-                if (actions != nullptr) actions[m] = static_cast<int8_t>(arg);
+                if (kDist) {
+                    float mx = lv[0];   // first argmax: the greedy action, and the shift of the logsumexp
+                    int am = 0;
+#pragma unroll
+                    for (int a = 1; a < NH - 1; ++a)
+                        if (a < num_outputs && lv[a] > mx) { mx = lv[a]; am = a; }
+                    const int act = mode == SSD_ACT_SAMPLE ? arg : mode == SSD_ACT_GREEDY ? am : static_cast<int>(actions[m]);
+                    float se = 0.f, sed = 0.f, la = __int_as_float(0x7fc00000);   // la: NaN unless act is in 0..A-1
+#pragma unroll
+                    for (int a = 0; a < NH - 1; ++a) {
+                        if (a < num_outputs) {
+                            const float d = lv[a] - mx, e = expf(d);
+                            se += e;
+                            sed = fmaf(e, d, sed);
+                            if (a == act) la = d;
+                        }
+                    }
+                    const float lse = logf(se);   // logsumexp(l) - mx; se >= 1
+                    if (logp != nullptr) logp[m] = la - lse;
+                    if (entropy != nullptr) entropy[m] = lse - sed / se;   // -sum p (d - lse)
+                    if (mode != SSD_ACT_GIVEN) actions[m] = static_cast<int8_t>(act);
+                } else if (actions != nullptr) {
+                    actions[m] = static_cast<int8_t>(arg);
+                }
             }
         }
         tc_fence_before();
@@ -286,6 +317,89 @@ lstm_heads_kernel(const float* __restrict__ feat, const float* h_in, const float
     SSD_HT_FLUSH;
     __syncthreads();
     if (warp == 0) tmem_free(tmem, 512);
+}
+
+// both instantiations of a weight map (plain head and ssd_policy_lstm_heads_dist) take the whole of shared memory
+template <WeightMap kMap>
+cudaError_t allow_smem() {
+    const cudaError_t e = cudaFuncSetAttribute(lstm_heads_kernel<kMap, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
+    return e != cudaSuccess ? e : cudaFuncSetAttribute(lstm_heads_kernel<kMap, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
+}
+
+// the arguments only ssd_policy_lstm_heads_dist / ssd_policy_pool_lstm_heads_dist take
+bool bad_dist_args(int mode, const int8_t* actions) {
+    if (mode != SSD_ACT_SAMPLE && mode != SSD_ACT_GREEDY && mode != SSD_ACT_GIVEN) {
+        ssd::set_error(SSD_ERR_INVALID, "mode must be SSD_ACT_SAMPLE, SSD_ACT_GREEDY or SSD_ACT_GIVEN");
+        return true;
+    }
+    if (!actions) {
+        ssd::set_error(SSD_ERR_INVALID, "the _dist entry points need actions (output, or input for SSD_ACT_GIVEN)");
+        return true;
+    }
+    return false;
+}
+
+// ssd_policy_lstm_heads (kDist false: mode, logp and entropy unused) and ssd_policy_lstm_heads_dist
+template <bool kDist>
+int heads(ssd_policy_t p, const float* features, const float* h_in, const float* c_in, float* h_out, float* c_out, float* logits, float* value,
+          int mode, int8_t* actions, float* logp, float* entropy, int64_t num_agents, uint64_t seed, uint32_t counter, void* stream) {
+    if (!p || !features || !h_in || !c_in || !h_out || !c_out || !logits || !value || num_agents < 0) return ssd::set_error(SSD_ERR_INVALID, "bad argument");
+    if (kDist && bad_dist_args(mode, actions)) return SSD_ERR_INVALID;
+    if (p->pool)
+        return ssd::set_error(SSD_ERR_INVALID, kDist ? "a policy pool handle takes ssd_policy_pool_lstm_heads_dist"
+                                                     : "a policy pool handle takes ssd_policy_pool_lstm_heads");
+    if (!p->d_head_blob) return ssd::set_error(SSD_ERR_INVALID, "ssd_policy_set_head has not been called");
+    const void* ptrs[5] = {features, h_in, c_in, h_out, c_out};
+    for (const void* q : ptrs)
+        if (reinterpret_cast<uintptr_t>(q) % 16 != 0) return ssd::set_error(SSD_ERR_INVALID, "features and state pointers must be 16-byte aligned");
+    const int np = p->num_policies;
+    if (num_agents % np != 0) return ssd::set_error(SSD_ERR_INVALID, "num_agents must be a multiple of num_policies");
+    if (num_agents == 0) return SSD_OK;
+    if (cudaSetDevice(p->device) != cudaSuccess) return ssd::set_error(SSD_ERR_CUDA, "cudaSetDevice failed");  // the blob and the stream live there
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const uint32_t s_lo = static_cast<uint32_t>(seed), s_hi = static_cast<uint32_t>(seed >> 32);
+    if (np == 1) {
+        const long long groups = (num_agents + GA - 1) / GA;
+        const int grid = static_cast<int>(groups < p->sms ? groups : p->sms);
+        lstm_heads_kernel<WeightMap::Shared, kDist><<<grid, kThreads, kSmemBytes, st>>>(features, h_in, c_in, h_out, c_out, logits, value, actions,
+                                                                                       num_agents, p->num_outputs, p->d_head_blob, s_lo, s_hi, counter,
+                                                                                       1, grid, nullptr, nullptr, nullptr, mode, logp, entropy);
+    } else {  // P * floor(#SMs / P) CTAs at most, each serving one policy
+        const long long groups = (num_agents / np + GA - 1) / GA;
+        const int per = static_cast<int>(groups < p->sms / np ? groups : p->sms / np);
+        lstm_heads_kernel<WeightMap::PerAgent, kDist><<<np * per, kThreads, kSmemBytes, st>>>(features, h_in, c_in, h_out, c_out, logits, value, actions,
+                                                                                             num_agents, p->num_outputs, p->d_head_blob, s_lo, s_hi,
+                                                                                             counter, np, per, nullptr, nullptr, nullptr, mode, logp,
+                                                                                             entropy);
+    }
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return ssd::set_error(SSD_ERR_CUDA, cudaGetErrorString(e));
+    return SSD_OK;
+}
+
+// ssd_policy_pool_lstm_heads and ssd_policy_pool_lstm_heads_dist
+template <bool kDist>
+int pool_heads(ssd_policy_t p, const float* features, const uint8_t* policy_ids, const float* h_in, const float* c_in, float* h_out, float* c_out,
+               float* logits, float* value, int mode, int8_t* actions, float* logp, float* entropy, int64_t num_agents, uint64_t seed,
+               uint32_t counter, void* stream) {
+    if (!p || !features || !policy_ids || !h_in || !c_in || !h_out || !c_out || !logits || !value || num_agents < 0)
+        return ssd::set_error(SSD_ERR_INVALID, "bad argument");
+    if (kDist && bad_dist_args(mode, actions)) return SSD_ERR_INVALID;
+    if (!p->pool) return ssd::set_error(SSD_ERR_INVALID, "not a policy pool handle (ssd_policy_create_pool)");
+    const void* ptrs[5] = {features, h_in, c_in, h_out, c_out};
+    for (const void* q : ptrs)
+        if (reinterpret_cast<uintptr_t>(q) % 16 != 0) return ssd::set_error(SSD_ERR_INVALID, "features and state pointers must be 16-byte aligned");
+    if (num_agents == 0) return SSD_OK;
+    const int rc = ssd::policy_pool::assign(p, policy_ids, num_agents, stream);   // sets the device
+    if (rc != SSD_OK) return rc;
+    const long long tiles = ssd::policy_pool::max_tiles(num_agents, p->num_policies);
+    const int grid = static_cast<int>(tiles < p->sms ? tiles : p->sms);
+    lstm_heads_kernel<WeightMap::Pool, kDist><<<grid, kThreads, kSmemBytes, static_cast<cudaStream_t>(stream)>>>(
+        features, h_in, c_in, h_out, c_out, logits, value, actions, num_agents, p->num_outputs, p->d_head_blob, static_cast<uint32_t>(seed),
+        static_cast<uint32_t>(seed >> 32), counter, p->num_policies, grid, p->d_perm, p->d_tiles, p->d_counts + 512, mode, logp, entropy);
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return ssd::set_error(SSD_ERR_CUDA, cudaGetErrorString(e));
+    return SSD_OK;
 }
 
 }  // namespace policy_head
@@ -342,9 +456,9 @@ int ssd::policy_head::set_head(SsdPolicy* p, int units, int num_outputs, const f
     cudaError_t e = cudaSetDevice(p->device);
     if (e == cudaSuccess && !p->d_head_blob) e = cudaMalloc(&p->d_head_blob, blob_bytes);
     if (e == cudaSuccess) e = cudaMemcpy(p->d_head_blob, blobs.data(), blob_bytes, cudaMemcpyHostToDevice);
-    if (e == cudaSuccess && p->pool) e = cudaFuncSetAttribute(lstm_heads_kernel<WeightMap::Pool>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
-    else if (e == cudaSuccess && num_policies == 1) e = cudaFuncSetAttribute(lstm_heads_kernel<WeightMap::Shared>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
-    else if (e == cudaSuccess) e = cudaFuncSetAttribute(lstm_heads_kernel<WeightMap::PerAgent>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
+    if (e == cudaSuccess && p->pool) e = allow_smem<WeightMap::Pool>();
+    else if (e == cudaSuccess && num_policies == 1) e = allow_smem<WeightMap::Shared>();
+    else if (e == cudaSuccess) e = allow_smem<WeightMap::PerAgent>();
     if (e != cudaSuccess) return ssd::set_error(SSD_ERR_CUDA, cudaGetErrorString(e));
     p->units = units;
     p->num_outputs = num_outputs;
@@ -361,58 +475,29 @@ int ssd_policy_set_head(ssd_policy_t p, int units, int num_outputs, const float*
 
 int ssd_policy_lstm_heads(ssd_policy_t p, const float* features, const float* h_in, const float* c_in, float* h_out, float* c_out, float* logits,
                           float* value, int8_t* actions, int64_t num_agents, uint64_t seed, uint32_t counter, void* stream) {
-    using namespace ssd::policy_head;
-    if (!p || !features || !h_in || !c_in || !h_out || !c_out || !logits || !value || num_agents < 0) return ssd::set_error(SSD_ERR_INVALID, "bad argument");
-    if (p->pool) return ssd::set_error(SSD_ERR_INVALID, "a policy pool handle takes ssd_policy_pool_lstm_heads");
-    if (!p->d_head_blob) return ssd::set_error(SSD_ERR_INVALID, "ssd_policy_set_head has not been called");
-    const void* ptrs[5] = {features, h_in, c_in, h_out, c_out};
-    for (const void* q : ptrs)
-        if (reinterpret_cast<uintptr_t>(q) % 16 != 0) return ssd::set_error(SSD_ERR_INVALID, "features and state pointers must be 16-byte aligned");
-    const int np = p->num_policies;
-    if (num_agents % np != 0) return ssd::set_error(SSD_ERR_INVALID, "num_agents must be a multiple of num_policies");
-    if (num_agents == 0) return SSD_OK;
-    if (cudaSetDevice(p->device) != cudaSuccess) return ssd::set_error(SSD_ERR_CUDA, "cudaSetDevice failed");  // the blob and the stream live there
-    const cudaStream_t st = static_cast<cudaStream_t>(stream);
-    const uint32_t s_lo = static_cast<uint32_t>(seed), s_hi = static_cast<uint32_t>(seed >> 32);
-    if (np == 1) {
-        const long long groups = (num_agents + GA - 1) / GA;
-        const int grid = static_cast<int>(groups < p->sms ? groups : p->sms);
-        lstm_heads_kernel<WeightMap::Shared><<<grid, kThreads, kSmemBytes, st>>>(features, h_in, c_in, h_out, c_out, logits, value, actions, num_agents,
-                                                                                p->num_outputs, p->d_head_blob, s_lo, s_hi, counter, 1, grid,
-                                                                                nullptr, nullptr, nullptr);
-    } else {  // P * floor(#SMs / P) CTAs at most, each serving one policy
-        const long long groups = (num_agents / np + GA - 1) / GA;
-        const int per = static_cast<int>(groups < p->sms / np ? groups : p->sms / np);
-        lstm_heads_kernel<WeightMap::PerAgent><<<np * per, kThreads, kSmemBytes, st>>>(features, h_in, c_in, h_out, c_out, logits, value, actions,
-                                                                                      num_agents, p->num_outputs, p->d_head_blob, s_lo, s_hi, counter,
-                                                                                      np, per, nullptr, nullptr, nullptr);
-    }
-    const cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return ssd::set_error(SSD_ERR_CUDA, cudaGetErrorString(e));
-    return SSD_OK;
+    return ssd::policy_head::heads<false>(p, features, h_in, c_in, h_out, c_out, logits, value, 0, actions, nullptr, nullptr, num_agents, seed,
+                                          counter, stream);
+}
+
+int ssd_policy_lstm_heads_dist(ssd_policy_t p, const float* features, const float* h_in, const float* c_in, float* h_out, float* c_out,
+                               float* logits, float* value, int mode, int8_t* actions, float* logp, float* entropy, int64_t num_agents,
+                               uint64_t seed, uint32_t counter, void* stream) {
+    return ssd::policy_head::heads<true>(p, features, h_in, c_in, h_out, c_out, logits, value, mode, actions, logp, entropy, num_agents, seed,
+                                         counter, stream);
 }
 
 int ssd_policy_pool_lstm_heads(ssd_policy_t p, const float* features, const uint8_t* policy_ids, const float* h_in, const float* c_in, float* h_out,
                                float* c_out, float* logits, float* value, int8_t* actions, int64_t num_agents, uint64_t seed, uint32_t counter,
                                void* stream) {
-    using namespace ssd::policy_head;
-    if (!p || !features || !policy_ids || !h_in || !c_in || !h_out || !c_out || !logits || !value || num_agents < 0)
-        return ssd::set_error(SSD_ERR_INVALID, "bad argument");
-    if (!p->pool) return ssd::set_error(SSD_ERR_INVALID, "not a policy pool handle (ssd_policy_create_pool)");
-    const void* ptrs[5] = {features, h_in, c_in, h_out, c_out};
-    for (const void* q : ptrs)
-        if (reinterpret_cast<uintptr_t>(q) % 16 != 0) return ssd::set_error(SSD_ERR_INVALID, "features and state pointers must be 16-byte aligned");
-    if (num_agents == 0) return SSD_OK;
-    const int rc = ssd::policy_pool::assign(p, policy_ids, num_agents, stream);   // sets the device
-    if (rc != SSD_OK) return rc;
-    const long long tiles = ssd::policy_pool::max_tiles(num_agents, p->num_policies);
-    const int grid = static_cast<int>(tiles < p->sms ? tiles : p->sms);
-    lstm_heads_kernel<WeightMap::Pool><<<grid, kThreads, kSmemBytes, static_cast<cudaStream_t>(stream)>>>(
-        features, h_in, c_in, h_out, c_out, logits, value, actions, num_agents, p->num_outputs, p->d_head_blob, static_cast<uint32_t>(seed),
-        static_cast<uint32_t>(seed >> 32), counter, p->num_policies, grid, p->d_perm, p->d_tiles, p->d_counts + 512);
-    const cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return ssd::set_error(SSD_ERR_CUDA, cudaGetErrorString(e));
-    return SSD_OK;
+    return ssd::policy_head::pool_heads<false>(p, features, policy_ids, h_in, c_in, h_out, c_out, logits, value, 0, actions, nullptr, nullptr,
+                                               num_agents, seed, counter, stream);
+}
+
+int ssd_policy_pool_lstm_heads_dist(ssd_policy_t p, const float* features, const uint8_t* policy_ids, const float* h_in, const float* c_in,
+                                    float* h_out, float* c_out, float* logits, float* value, int mode, int8_t* actions, float* logp,
+                                    float* entropy, int64_t num_agents, uint64_t seed, uint32_t counter, void* stream) {
+    return ssd::policy_head::pool_heads<true>(p, features, policy_ids, h_in, c_in, h_out, c_out, logits, value, mode, actions, logp, entropy,
+                                              num_agents, seed, counter, stream);
 }
 
 }  // extern "C"

@@ -30,7 +30,12 @@ may change while a state is alive.
 Weights are numpy fp32 arrays in the Keras layouts (conv kernel [kh, kw, in, out], dense kernels [in, out], LSTM kernel
 [in, 4u] / recurrent kernel [u, 4u] / bias [4u] with gates ordered i, f, c, o), so a checkpoint of the reference model
 loads without transposition.  There is no CPU path: the trunk raises without the CUDA library.
+
+`policy_step` returns what a sampler records per step -- the action, its log-probability, the entropy, the logits, the value and
+the next state (a `PolicyStep`) -- for a sampled, a greedy or a caller-given action, from the same fused head kernel
+(`ssd_policy_lstm_heads_dist`).
 """
+import collections
 import ctypes as C
 
 import numpy as np
@@ -43,6 +48,13 @@ OBS_SIDE = 2 * VIEW_RADIUS + 1
 CONV_FILTERS = 6
 FEATURES = 32
 FLAT = (OBS_SIDE - 2) * (OBS_SIDE - 2) * CONV_FILTERS   # 1014
+
+
+PolicyStep = collections.namedtuple("PolicyStep", "actions logp entropy logits value h c")
+PolicyStep.__doc__ = """One step of the policy for M agents: actions int8 [M], logp float32 [M] (log softmax(logits) at the action), entropy
+float32 [M] (of softmax(logits)), logits float32 [M, A], value float32 [M], and the next recurrent state (h, c)."""
+
+_MODES = {"sample": _lib.ACT_SAMPLE, "greedy": _lib.ACT_GREEDY, "given": _lib.ACT_GIVEN}
 
 
 def random_weights(num_outputs, cell_size=128, seed=0):
@@ -100,6 +112,40 @@ def _weight_sets(weights):
         if sorted(ws) != sorted(w) or any(ws[k].shape != w[k].shape for k in w):
             raise ValueError("weights[%d] does not have the names and shapes of weights[0]" % p)
     return sets
+
+
+def _step_mode(mode, actions, m, num_outputs, device):
+    """-> (SSD_ACT_* code, the given actions as a contiguous int8 [m] tensor or None).  Integer actions outside 0..A-1 become
+    -1 or A before the narrowing to int8, so every one of them gets logp NaN (none wraps onto a valid action).  They are
+    widened to int64 first: clamped in an unsigned dtype, the bound -1 would itself wrap to the dtype's maximum."""
+    if mode not in _MODES:
+        raise ValueError("mode must be 'sample', 'greedy' or 'given', not %r" % (mode,))
+    if mode != "given":
+        if actions is not None:
+            raise ValueError("actions are an input of mode 'given' only")
+        return _MODES[mode], None
+    if not isinstance(actions, torch.Tensor) or actions.device != device or actions.numel() != m \
+            or actions.dtype.is_floating_point or actions.dtype.is_complex or actions.dtype == torch.bool:
+        raise ValueError("mode 'given' takes actions, an integer tensor of %d elements on %s" % (m, device))
+    a = actions.reshape(-1)
+    if a.dtype != torch.int8:
+        a = a.long().clamp(-1, num_outputs).to(torch.int8)
+    return _MODES[mode], a.contiguous()
+
+
+def _torch_step(logits, value, h, c, code, given, generator):
+    """PolicyStep of the unfused route: log_softmax, argmax and torch.multinomial over the logits `forward` returned."""
+    logp_all = torch.log_softmax(logits, dim=1)
+    if code == _lib.ACT_SAMPLE:
+        a = torch.multinomial(torch.softmax(logits, dim=1), 1, generator=generator).squeeze(1)
+    elif code == _lib.ACT_GREEDY:
+        a = logits.argmax(dim=1)   # the first maximum
+    else:
+        a = given.long()
+    valid = (a >= 0) & (a < logits.shape[1])
+    logp = logp_all.gather(1, torch.where(valid, a, 0)[:, None]).squeeze(1).masked_fill(~valid, float("nan"))
+    entropy = -(logp_all.exp() * logp_all).sum(dim=1)
+    return PolicyStep(given if given is not None else a.to(torch.int8), logp, entropy, logits, value, h, c)
 
 
 def _state_rows(state, m, P):
@@ -215,18 +261,23 @@ class ConvToFCNet(object):
         return _state_from_rows(rows, self.num_policies)
 
     def seed_sampling(self, seed):
-        """Key of the Philox streams `act` samples from (counter = number of `act` calls since)."""
+        """Key of the Philox streams `act` samples from (counter = number of `act` and sampling `policy_step` calls since)."""
         self._sample_seed, self._sample_counter = int(seed) & (2 ** 64 - 1), 0
 
-    def _fused(self, obs, h, c, sample):
+    def _head_io(self, obs, h, c):
+        """Features of obs, the checked (h, c) and fresh output buffers (h', c', logits, value) of the fused head."""
         x = self.features(obs)
         m = x.shape[0]
         if h.dim() != 4 or (h.shape[0] * 128 < m if self.num_policies == 1 else h.shape[0] != self._groups(m)):
             raise ValueError("the fused route carries (h, c) in the tiled layout of initial_state / state_from_rows")
         h, c = _aligned(h), _aligned(c)
-        h_new, c_new = torch.empty_like(h), torch.empty_like(c)
         logits = torch.empty((m, self.num_outputs), dtype=torch.float32, device=self.device)
         value = torch.empty((m,), dtype=torch.float32, device=self.device)
+        return x, h, c, (torch.empty_like(h), torch.empty_like(c), logits, value)
+
+    def _fused(self, obs, h, c, sample):
+        x, h, c, (h_new, c_new, logits, value) = self._head_io(obs, h, c)
+        m = x.shape[0]
         actions = torch.empty((m,), dtype=torch.int8, device=self.device) if sample else None
         stream = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
         p = lambda t: C.c_void_p(t.data_ptr() if t is not None else None)
@@ -270,6 +321,30 @@ class ConvToFCNet(object):
         logits, value, h, c = self.forward(obs, h, c)
         a = torch.multinomial(torch.softmax(logits, dim=1), 1, generator=generator).squeeze(1).to(torch.int8)
         return a, value, h, c
+
+    def policy_step(self, obs, h, c, mode="sample", actions=None, generator=None):
+        """-> PolicyStep(actions, logp, entropy, logits, value, h', c') for the M agents of obs; (h, c) as for `forward`.
+
+        mode 'sample': the action `act` draws -- the same Philox stream, and the call advances its counter, so `act` and
+        `policy_step` calls may be interleaved; with `generator` (or on the unfused route) torch.multinomial as in `act`.
+        mode 'greedy': the first argmax of the logits (np.argmax of them where they are finite).  mode 'given': `actions` (integers, M of them) are the caller's, e.g. a
+        recorded trajectory or another policy's choice, and are returned as int8; logp is NaN where one is outside 0..A-1.
+        logp and entropy are those of softmax(logits), computed from the float32 logits returned: on the fused route in the head
+        kernel itself (ssd_policy_lstm_heads_dist), on the unfused route with torch.log_softmax."""
+        m = obs.numel() // (OBS_SIDE * OBS_SIDE * 3)
+        code, given = _step_mode(mode, actions, m, self.num_outputs, self.device)
+        if not self._fused_head or (code == _lib.ACT_SAMPLE and generator is not None):
+            return _torch_step(*self.forward(obs, h, c), code, given, generator)
+        x, h, c, (h_new, c_new, logits, value) = self._head_io(obs, h, c)
+        a = given if given is not None else torch.empty((m,), dtype=torch.int8, device=self.device)
+        logp, entropy = torch.empty_like(value), torch.empty_like(value)
+        stream = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+        p = lambda t: C.c_void_p(t.data_ptr())
+        _lib.check(_lib.lib.ssd_policy_lstm_heads_dist(self._h, p(x), p(h), p(c), p(h_new), p(c_new), p(logits), p(value), code, p(a), p(logp),
+                                                       p(entropy), m, self._sample_seed, self._sample_counter & 0xFFFFFFFF, stream))
+        if code == _lib.ACT_SAMPLE:
+            self._sample_counter += 1
+        return PolicyStep(a, logp, entropy, logits, value, h_new, c_new)
 
 
 class PolicyPool(object):
@@ -344,19 +419,25 @@ class PolicyPool(object):
         return _state_from_rows(rows, 1)
 
     def seed_sampling(self, seed):
-        """Key of the Philox streams `act` samples from (counter = number of `act` calls since)."""
+        """Key of the Philox streams `act` samples from (counter = number of `act` and sampling `policy_step` calls since)."""
         self._sample_seed, self._sample_counter = int(seed) & (2 ** 64 - 1), 0
 
-    def _run(self, obs, policy_ids, h, c, sample):
-        obs, ids = self._ids(obs, policy_ids)
+    def _head_io(self, obs, ids, h, c):
+        """Features of obs (obs and ids as `_ids` returns them), the checked (h, c) and fresh output buffers (h', c', logits,
+        value) of the head."""
         x = self.features(obs, ids)
         m = x.shape[0]
         if h.dim() != 4 or h.shape[0] * 128 < m or h.shape != c.shape:
             raise ValueError("(h, c) must be in the tiled layout of initial_state / state_from_rows")
         h, c = _aligned(h), _aligned(c)
-        h_new, c_new = torch.empty_like(h), torch.empty_like(c)
         logits = torch.empty((m, self.num_outputs), dtype=torch.float32, device=self.device)
         value = torch.empty((m,), dtype=torch.float32, device=self.device)
+        return x, h, c, (torch.empty_like(h), torch.empty_like(c), logits, value)
+
+    def _run(self, obs, policy_ids, h, c, sample):
+        obs, ids = self._ids(obs, policy_ids)
+        x, h, c, (h_new, c_new, logits, value) = self._head_io(obs, ids, h, c)
+        m = x.shape[0]
         actions = torch.full((m,), -1, dtype=torch.int8, device=self.device) if sample else None
         stream = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
         p = lambda t: C.c_void_p(t.data_ptr() if t is not None else None)
@@ -374,3 +455,23 @@ class PolicyPool(object):
         """Sample int8 actions [M] on the device (Philox streams, see `seed_sampling`); -1 for skipped agents."""
         logits, value, h, c, a = self._run(obs, policy_ids, h, c, sample=True)
         return a, value, h, c
+
+    def policy_step(self, obs, policy_ids, h, c, mode="sample", actions=None):
+        """-> PolicyStep(actions, logp, entropy, logits, value, h', c'), as ConvToFCNet.policy_step on the pool's kernels:
+        'sample' draws what `act` draws and advances the same counter, 'greedy' takes the first argmax of the logits, 'given'
+        scores the caller's `actions` (returned as int8).  Skipped agents (id >= K) get action -1 in 'sample' and 'greedy'; their
+        rows of logp and entropy, like those of logits, value, h' and c', are not written."""
+        obs, ids = self._ids(obs, policy_ids)
+        m = ids.numel()
+        code, given = _step_mode(mode, actions, m, self.num_outputs, self.device)
+        x, h, c, (h_new, c_new, logits, value) = self._head_io(obs, ids, h, c)
+        a = given if given is not None else torch.full((m,), -1, dtype=torch.int8, device=self.device)
+        logp, entropy = torch.empty_like(value), torch.empty_like(value)
+        stream = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+        p = lambda t: C.c_void_p(t.data_ptr())
+        _lib.check(_lib.lib.ssd_policy_pool_lstm_heads_dist(self._h, p(x), p(ids), p(h), p(c), p(h_new), p(c_new), p(logits), p(value), code,
+                                                            p(a), p(logp), p(entropy), m, self._sample_seed, self._sample_counter & 0xFFFFFFFF,
+                                                            stream))
+        if code == _lib.ACT_SAMPLE:
+            self._sample_counter += 1
+        return PolicyStep(a, logp, entropy, logits, value, h_new, c_new)
