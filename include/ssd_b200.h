@@ -283,6 +283,38 @@ int ssd_policy_lstm_heads_dist(ssd_policy_t p, const float* features, const floa
 int ssd_policy_pool_lstm_heads_dist(ssd_policy_t p, const float* features, const uint8_t* policy_ids, const float* h_in, const float* c_in,
                                     float* h_out, float* c_out, float* logits, float* value, int mode, int8_t* actions, float* logp,
                                     float* entropy, int64_t num_agents, uint64_t seed, uint32_t counter, void* stream);
+/* Model of other agents (MOA) and social-influence reward of the causal-influence models (models/moa_model.py MOA_LSTM,
+ * common_funcs.py compute_influence_reward), forward only, in ONE kernel.  For agent m = b*N + i (env b, agent i):
+ *   input(a') = [features(32) | onehot(a') | onehot(a_{b,j}) for j != i, increasing j], width 32 + N*A; an action outside 0..A-1
+ *   is a zero one-hot row.  LSTM(128) (Keras gate order i, f, c~, o, as ssd_policy_set_head), then Dense((N-1)*A), columns
+ *   (other k in the same order, action).
+ * ssd_moa_create packs HOST fp32 weights in the Keras layouts: lstm_w [32 + N*A][512], lstm_u [128][512], lstm_b [512],
+ * logits_w [128][(N-1)*A], logits_b [(N-1)*A]; num_policies 1 (shared) or N (agent i uses weight set i, the pointers then point
+ * to N consecutive arrays, as ssd_policy_create_n).  N = num_agents 2..SSD_MAX_AGENTS, A = num_actions 1..15, (N-1)*A <= 64.
+ * ssd_moa_step, M = num_agents a multiple of N:
+ *   features dev f32[M][32] (ssd_policy_features), joint_actions dev i8[M] ([B][N], the actions the step took),
+ *   policy_logits dev f32[M][A] (the policy's logits of that step); h_in / c_in / h_out / c_out the MOA's recurrent state in the
+ *   TILED layout of ssd_policy_lstm_heads (grouped per weight set for num_policies = N, as ssd_policy_create_n), out must not
+ *   alias in; all five 16-byte aligned.
+ *   pred dev f32[M][N-1][A]: the MOA logits at the actual joint action; h_out / c_out: the next state at the actual action.
+ *   counterfactual dev f32[M][A][N-1][A] or NULL: the logits with the own action replaced by a' (equal to pred at a' = a_{b,i}).
+ *   influence_per_agent dev f32[M][N-1]: D(p_k(.|a_{b,i}) || q_k), p_k(.|a') = softmax(counterfactual[m][a'][k]),
+ *     q_k = sum_{a'} softmax(policy_logits[m])[a'] p_k(.|a') renormalised to sum 1; D = KL (SSD_DIV_KL, terms with p = 0
+ *     skipped) or the Jensen-Shannon divergence (SSD_DIV_JSD).
+ *   influence dev f32[M]: clamp(sum_k influence_per_agent[m][k], -clip, clip); clip >= 0, +inf disables the clamp.
+ *   An action outside 0..A-1 anywhere in env b sets influence and influence_per_agent of every agent of b to NaN; pred,
+ *   h_out and c_out are still written.
+ * Bad arguments return SSD_ERR_INVALID before anything is launched, as do policy handles here and MOA handles at the policy
+ * entry points.  fp16 gate GEMM operands; one-hot rows, Dense((N-1)*A) and the influence in fp32. */
+typedef struct SsdPolicy* ssd_moa_t;
+#define SSD_DIV_KL 0
+#define SSD_DIV_JSD 1
+int ssd_moa_create(int device, int num_policies, int num_agents, int num_actions, const float* lstm_w, const float* lstm_u, const float* lstm_b,
+                   const float* logits_w, const float* logits_b, ssd_moa_t* out);
+void ssd_moa_destroy(ssd_moa_t p);
+int ssd_moa_step(ssd_moa_t p, const float* features, const int8_t* joint_actions, const float* policy_logits, const float* h_in, const float* c_in,
+                 float* h_out, float* c_out, float* pred, float* counterfactual, float* influence_per_agent, float* influence, int64_t num_agents,
+                 int divergence, float clip, void* stream);
 /* The unfused alternative for other cell sizes: LSTM cell update after the gate GEMM (conv_to_fcnet_v2.py:68-80; Keras gate order i, f, c~, o; sigmoid recurrent
  * activation): gates dev bf16[num_agents][4*units] = x W + h U without the bias, bias dev f32[4*units],
  * c_prev / c_out / h_out dev f32[num_agents][units] (c_out may alias c_prev), h_bf16_out dev bf16[num_agents][units]

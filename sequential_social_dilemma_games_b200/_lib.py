@@ -15,6 +15,7 @@ OPT_CHAIN_STEPS = 1
 OPT_GENERAL_KERNEL = 2
 PHASE_MOVES, PHASE_CONSUME, PHASE_BEAMS, PHASE_SPAWN, PHASE_RENDER, PHASE_ALL = 1, 2, 4, 8, 16, 31
 ACT_SAMPLE, ACT_GREEDY, ACT_GIVEN = 0, 1, 2
+DIV_KL, DIV_JSD = 0, 1
 
 # every symbol include/ssd_b200.h declares (tests/test_cabi.py checks the list against the header)
 SYMBOLS = ("ssd_last_error", "ssd_abi_version", "ssd_create", "ssd_destroy", "ssd_num_apple_points",
@@ -25,7 +26,7 @@ SYMBOLS = ("ssd_last_error", "ssd_abi_version", "ssd_create", "ssd_destroy", "ss
            "ssd_policy_create", "ssd_policy_features", "ssd_policy_destroy", "ssd_policy_lstm_cell",
            "ssd_policy_set_head", "ssd_policy_lstm_heads", "ssd_policy_create_n", "ssd_policy_set_head_n",
            "ssd_policy_create_pool", "ssd_policy_pool_features", "ssd_policy_pool_lstm_heads", "ssd_policy_lstm_heads_dist",
-           "ssd_policy_pool_lstm_heads_dist")
+           "ssd_policy_pool_lstm_heads_dist", "ssd_moa_create", "ssd_moa_destroy", "ssd_moa_step")
 
 
 class SsdConfig(C.Structure):
@@ -99,6 +100,9 @@ def _load():
         "ssd_policy_pool_lstm_heads": (i32, [vp] + [vp] * 9 + [i64, C.c_uint64, C.c_uint32, vp]),
         "ssd_policy_lstm_heads_dist": (i32, [vp] * 8 + [i32] + [vp] * 3 + [i64, C.c_uint64, C.c_uint32, vp]),
         "ssd_policy_pool_lstm_heads_dist": (i32, [vp] * 9 + [i32] + [vp] * 3 + [i64, C.c_uint64, C.c_uint32, vp]),
+        "ssd_moa_create": (i32, [i32, i32, i32, i32] + [vp] * 5 + [C.POINTER(vp)]),
+        "ssd_moa_destroy": (None, [vp]),
+        "ssd_moa_step": (i32, [vp] * 12 + [i64, i32, C.c_float, vp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)

@@ -669,6 +669,7 @@ int ssd_policy_features(ssd_policy_t p, const uint8_t* obs, int64_t num_agents, 
     if (reinterpret_cast<uintptr_t>(obs) % 16 != 0 || reinterpret_cast<uintptr_t>(features) % 16 != 0)
         return ssd::set_error(SSD_ERR_INVALID, "obs and features must be 16-byte aligned");
     if (p->pool) return ssd::set_error(SSD_ERR_INVALID, "a policy pool handle takes ssd_policy_pool_features");
+    if (p->moa) return ssd::set_error(SSD_ERR_INVALID, "an MOA handle takes ssd_moa_step");
     const int np = p->num_policies;
     if (num_agents % np != 0) return ssd::set_error(SSD_ERR_INVALID, "num_agents must be a multiple of num_policies");
     if (num_agents == 0) return SSD_OK;
@@ -735,6 +736,7 @@ void ssd_policy_destroy(ssd_policy_t p) {
     if (p->d_counts) cudaFree(p->d_counts);
     if (p->d_perm) cudaFree(p->d_perm);
     if (p->d_tiles) cudaFree(p->d_tiles);
+    if (p->d_moa_rows) cudaFree(p->d_moa_rows);
     delete p;
 }
 

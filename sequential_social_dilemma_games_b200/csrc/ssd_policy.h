@@ -21,6 +21,11 @@ struct SsdPolicy {
     int units = 0, num_outputs = 0;
     int num_policies = 1;            // weight sets: agent m = b * P + p uses set p (ssd_policy_create_n), or set ids[m] (pool)
     bool pool = false;               // made by ssd_policy_create_pool
+    // made by ssd_moa_create: d_head_blob holds the MOA's resident weights, d_moa_rows its one-hot rows and moa_logits_w,
+    // num_outputs its A, moa_agents its N
+    bool moa = false;
+    int moa_agents = 0;
+    float* d_moa_rows = nullptr;
     // pool scratch, grown on demand: per-policy counts [256] and cursors [256], the tile count, perm [M], tiles [M / 128 + K]
     uint32_t* d_counts = nullptr;
     uint32_t* d_perm = nullptr;

@@ -348,6 +348,7 @@ int heads(ssd_policy_t p, const float* features, const float* h_in, const float*
     if (p->pool)
         return ssd::set_error(SSD_ERR_INVALID, kDist ? "a policy pool handle takes ssd_policy_pool_lstm_heads_dist"
                                                      : "a policy pool handle takes ssd_policy_pool_lstm_heads");
+    if (p->moa) return ssd::set_error(SSD_ERR_INVALID, "an MOA handle takes ssd_moa_step");
     if (!p->d_head_blob) return ssd::set_error(SSD_ERR_INVALID, "ssd_policy_set_head has not been called");
     const void* ptrs[5] = {features, h_in, c_in, h_out, c_out};
     for (const void* q : ptrs)
@@ -414,6 +415,7 @@ int ssd_policy_set_head_n(ssd_policy_t p, int num_policies, int units, int num_o
     if (num_policies < 1 || num_policies > SSD_MAX_AGENTS) return ssd::set_error(SSD_ERR_INVALID, "num_policies must be 1..SSD_MAX_AGENTS");
     if (num_policies != p->num_policies) return ssd::set_error(SSD_ERR_INVALID, "the head must have as many weight sets as the trunk");
     if (p->pool) return ssd::set_error(SSD_ERR_INVALID, "a policy pool's head is loaded by ssd_policy_create_pool");
+    if (p->moa) return ssd::set_error(SSD_ERR_INVALID, "an MOA handle is loaded by ssd_moa_create");
     return ssd::policy_head::set_head(p, units, num_outputs, lstm_w, lstm_u, lstm_b, logits_w, logits_b, value_w, value_b);
 }
 #pragma GCC visibility pop

@@ -34,6 +34,10 @@ loads without transposition.  There is no CPU path: the trunk raises without the
 `policy_step` returns what a sampler records per step -- the action, its log-probability, the entropy, the logits, the value and
 the next state (a `PolicyStep`) -- for a sampled, a greedy or a caller-given action, from the same fused head kernel
 (`ssd_policy_lstm_heads_dist`).
+
+`MOANet` is the model of other agents of the causal-influence models (train_moa.py): from the trunk features, the joint action
+and the policy's logits it predicts the others' next actions, for the actual and for every counterfactual own action, and
+returns the social-influence reward (`MOAStep`), all in one kernel (`ssd_moa_step`).
 """
 import collections
 import ctypes as C
@@ -475,3 +479,127 @@ class PolicyPool(object):
         if code == _lib.ACT_SAMPLE:
             self._sample_counter += 1
         return PolicyStep(a, logp, entropy, logits, value, h_new, c_new)
+
+
+MOAStep = collections.namedtuple("MOAStep", "pred influence influence_per_agent h c counterfactual")
+MOAStep.__doc__ = """One step of the model of other agents for M agents: pred float32 [M, N-1, A] (logits of the others' actions at the
+actual joint action), influence float32 [M], influence_per_agent float32 [M, N-1], the next state (h, c), and counterfactual
+float32 [M, A, N-1, A] (the logits with the own action replaced by each a') or None."""
+
+_DIVERGENCES = {"kl": _lib.DIV_KL, "jsd": _lib.DIV_JSD}
+
+
+def random_moa_weights(num_agents, num_actions, seed=0, cell_size=128):
+    """Random-init MOA weights (glorot, unit forget bias) in the Keras layouts `MOANet` takes."""
+    rng = np.random.RandomState(seed)
+    glorot = lambda shape: rng.uniform(-1, 1, size=shape).astype(np.float32) * np.float32(np.sqrt(6.0 / sum(shape)))
+    u, k_in, n_out = cell_size, FEATURES + num_agents * num_actions, (num_agents - 1) * num_actions
+    return {"moa_lstm_w": glorot((k_in, 4 * u)), "moa_lstm_u": glorot((u, 4 * u)),
+            "moa_lstm_b": np.concatenate([np.zeros(u), np.ones(u), np.zeros(2 * u)]).astype(np.float32),
+            "moa_logits_w": glorot((u, n_out)), "moa_logits_b": (0.1 * rng.randn(n_out)).astype(np.float32)}
+
+
+class MOANet(object):
+    """Model of other agents of the causal-influence models (models/moa_model.py MOA_LSTM) and the social-influence reward
+    (common_funcs.py compute_influence_reward), forward only, in one fused kernel (`ssd_moa_step`).
+
+    For agent m = b * N + i the input is [x | onehot(a_{b,i}) | onehot(a_{b,j}) for j != i in increasing j], x the 32 trunk
+    features (ConvToFCNet.features); LSTM(128) then Dense((N-1) * A).  `weights` is one dict (shared by all agents) or a list of
+    N dicts (agent i uses weights[i], as ConvToFCNet([w_0, ..., w_{N-1}])), with keys moa_lstm_w [32 + N A, 512], moa_lstm_u
+    [128, 512], moa_lstm_b [512], moa_logits_w [128, (N-1) A], moa_logits_b [(N-1) A].  The recurrent state has the tiled layout
+    of ConvToFCNet (grouped per weight set for a list of N)."""
+
+    def __init__(self, weights, num_agents, device="cuda:0"):
+        self.device = _cuda_device(device)
+        sets = list(weights) if isinstance(weights, (list, tuple)) else [weights]
+        n = self.num_agents = int(num_agents)
+        if len(sets) not in (1, n):
+            raise ValueError("weights is one dict or a list of num_agents = %d dicts, not %d" % (n, len(sets)))
+        sets = [{k: np.ascontiguousarray(ws[k], dtype=np.float32) for k in
+                 ("moa_lstm_w", "moa_lstm_u", "moa_lstm_b", "moa_logits_w", "moa_logits_b")} for ws in sets]
+        w = sets[0]
+        self.num_policies = P = len(sets)
+        self.cell_size = w["moa_lstm_u"].shape[0]
+        k_in = w["moa_lstm_w"].shape[0] - FEATURES
+        self.num_actions = A = k_in // n if n >= 2 else 0
+        shapes = {"moa_lstm_w": (FEATURES + n * A, 4 * self.cell_size), "moa_lstm_u": (self.cell_size, 4 * self.cell_size),
+                  "moa_lstm_b": (4 * self.cell_size,), "moa_logits_w": (self.cell_size, (n - 1) * A), "moa_logits_b": ((n - 1) * A,)}
+        for q, ws in enumerate(sets):
+            for k, shape in shapes.items():
+                if ws[k].shape != shape:
+                    raise ValueError("weights[%d][%r] has shape %s, expected %s" % (q, k, ws[k].shape, shape))
+        if self.cell_size != 128 or k_in != n * A:
+            raise ValueError("the MOA kernel is built for cell_size 128 and moa_lstm_w [32 + N A, 512]")
+        w = {k: np.ascontiguousarray(np.stack([ws[k] for ws in sets])) for k in w}   # P consecutive arrays behind every pointer
+        ptr = lambda a: a.ctypes.data_as(C.c_void_p)
+        self._h = C.c_void_p()
+        _lib.check(_lib.lib.ssd_moa_create(self.device.index, P, n, A, ptr(w["moa_lstm_w"]), ptr(w["moa_lstm_u"]), ptr(w["moa_lstm_b"]),
+                                           ptr(w["moa_logits_w"]), ptr(w["moa_logits_b"]), C.byref(self._h)))
+
+    def close(self):
+        if self._h:
+            _lib.lib.ssd_moa_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def _groups(self, m):
+        n, P = self.num_agents, self.num_policies
+        if m % n:
+            raise ValueError("%d agents are not a whole number of envs of %d agents" % (m, n))
+        return P * ((m // P + 127) // 128)
+
+    def initial_state(self, m):
+        """Zero (h, c) for m agents in the tiled layout [G, 8, 128, 16]."""
+        z = torch.zeros((self._groups(m), self.cell_size // 16, 128, 16), dtype=torch.float32, device=self.device)
+        return z, z.clone()
+
+    def state_rows(self, state, m):
+        """Tiled state -> agent-major [m, 128] (a copy)."""
+        self._groups(m)
+        return _state_rows(state, m, self.num_policies)
+
+    def state_from_rows(self, rows):
+        """Agent-major [m, 128] -> tiled state, zero padded."""
+        self._groups(rows.shape[0])
+        return _state_from_rows(rows, self.num_policies)
+
+    def step(self, features, joint_actions, policy_logits, h, c, divergence="kl", clip=float("inf"), counterfactuals=False):
+        """-> MOAStep for the M agents of features [M, 32] (float32, ConvToFCNet.features of the step's observations).
+
+        joint_actions: the actions the step took, an integer tensor of M elements ([B, N] or [M], agent-major); a value outside
+        0..A-1 is a zero one-hot input and makes influence NaN for every agent of its env.  policy_logits [M, A]: the policy's
+        logits of that step (PolicyStep.logits).  divergence 'kl' or 'jsd'; influence = clamp(sum over the others, -clip, clip).
+        counterfactuals=True also returns the [M, A, N-1, A] logits of every own action."""
+        if divergence not in _DIVERGENCES:
+            raise ValueError("divergence must be 'kl' or 'jsd', not %r" % (divergence,))
+        clip = float(clip)
+        if not clip >= 0.0:
+            raise ValueError("clip must be >= 0 (inf: no clamp), not %r" % (clip,))
+        n, A = self.num_agents, self.num_actions
+        if not isinstance(features, torch.Tensor) or features.dtype != torch.float32 or features.device != self.device \
+                or features.dim() != 2 or features.shape[1] != FEATURES:
+            raise ValueError("features must be a float32 [M, %d] tensor on %s" % (FEATURES, self.device))
+        m = features.shape[0]
+        g = self._groups(m)
+        _, given = _step_mode("given", joint_actions, m, A, self.device)
+        if not isinstance(policy_logits, torch.Tensor) or policy_logits.dtype != torch.float32 or policy_logits.device != self.device \
+                or tuple(policy_logits.shape) != (m, A):
+            raise ValueError("policy_logits must be a float32 [%d, %d] tensor on %s" % (m, A, self.device))
+        if tuple(h.shape) != (g, self.cell_size // 16, 128, 16) or h.shape != c.shape:
+            raise ValueError("(h, c) must be in the tiled layout of initial_state / state_from_rows")
+        x, h, c, pl = _aligned(features), _aligned(h), _aligned(c), policy_logits.contiguous()
+        h_new, c_new = torch.empty_like(h), torch.empty_like(c)
+        pred = torch.empty((m, n - 1, A), dtype=torch.float32, device=self.device)
+        cf = torch.empty((m, A, n - 1, A), dtype=torch.float32, device=self.device) if counterfactuals else None
+        ipa = torch.empty((m, n - 1), dtype=torch.float32, device=self.device)
+        infl = torch.empty((m,), dtype=torch.float32, device=self.device)
+        stream = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+        p = lambda t: C.c_void_p(t.data_ptr() if t is not None else None)
+        _lib.check(_lib.lib.ssd_moa_step(self._h, p(x), p(given), p(pl), p(h), p(c), p(h_new), p(c_new), p(pred), p(cf), p(ipa), p(infl), m,
+                                         _DIVERGENCES[divergence], clip, stream))
+        return MOAStep(pred, infl, ipa, h_new, c_new, cf)
