@@ -112,9 +112,8 @@ struct TrunkSmem {
 // thread ~40 cycles, five per step were 15 % of the kernel): whoever needs "the first block of step x is complete" waits
 // barrier x % 8 on parity (x / 8) & 1; no waiter is ever more than six steps from the MMA thread, so phases cannot alias.
 //
-// kPerAgent: agent m = b * P + p of the [B, P] batch is evaluated with weight set p (blob + p * kBlobBytes).  A UMMA tile
-// cannot change its B operand per row, so CTA c serves policy c % P only -- groups g = c / P, c / P + cpp, ... of the agents
-// (b, p), b in [128 g, 128 g + 128) -- and loads that policy's resident weights once, as the shared kernel does.
+// kPerAgent: agent m = b * P + p of the [B, P] batch is evaluated with weight set p (blob + p * kBlobBytes); the CTAs take the
+// groups of GroupMap (ssd_policy.h) and load their policy's resident weights once, as the shared kernel does.
 //
 // WeightMap::Pool: a group is one tile of the assignment (ssd_policy_pool.cu): agents perm[first, first + count) of one
 // policy, gathered and written back as the per-agent variant does, at rows perm[i].  CTA c takes tiles
@@ -137,14 +136,10 @@ __global__ void __launch_bounds__(kThreads, 1) policy_features_kernel(const uint
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     uint64_t* bars = reinterpret_cast<uint64_t*>(smem + kOffBar);
     const float* s_const = reinterpret_cast<const float*>(smem + kOffConst);
-    const int np = kPerAgent ? num_policies : 1;
-    const int pol = kPerAgent ? static_cast<int>(blockIdx.x) % np : 0;                       // this CTA's weight set
-    const long long cta = kPerAgent ? blockIdx.x / np : blockIdx.x;                          // its index among the CTAs of that policy
-    const long long stride = kPerAgent ? ctas_per_policy : gridDim.x;
-    const long long rows = kPerAgent ? M / np : M;                                           // agents per policy
+    const GroupMap<kMap> gm(M, num_policies, ctas_per_policy);
+    const long long cta = gm.cta, stride = gm.stride, rows = gm.rows, n_groups = gm.n_groups;
     const uint8_t* const blob0 = blob;
-    if (kPerAgent && !kPool) blob += static_cast<long long>(pol) * kBlobBytes;
-    const long long n_groups = (rows + GA - 1) / GA;
+    if (kPerAgent && !kPool) blob += static_cast<long long>(gm.pol) * kBlobBytes;
     long long seg_end = 0, tile_end = 0;   // pool: the CTA's tiles not yet run are [seg_end, tile_end)
     if (kPool) {
         const long long nt = *num_tiles;
@@ -216,7 +211,7 @@ __global__ void __launch_bounds__(kThreads, 1) policy_features_kernel(const uint
                 const PoolTile tile = tiles[tb + gi];
                 img += t < tile.count ? (perm[tile.first + t] * static_cast<uint32_t>(IMG)) & 15u : 0u;
             } else if (kPerAgent)  // the slot starts at the 16-byte boundary below the agent's row (obs is 16-byte aligned)
-                img += (static_cast<uint32_t>(((cta + gi * stride) * GA + t) * np + pol) * IMG) & 15u;
+                img += (static_cast<uint32_t>(gm.agent((cta + gi * stride) * GA, t)) * IMG) & 15u;
 #pragma unroll 1
             for (int r = 0; r < V; ++r, ++R) {
                 const uint32_t slot = R % RING;
@@ -382,7 +377,7 @@ __global__ void __launch_bounds__(kThreads, 1) policy_features_kernel(const uint
                 } else {  // gather: per agent the 16-byte-aligned span around its row, into its slot; nothing past the tensor's end
                     const long long end = M * IMG, end16 = end & ~15ll;
                     auto span = [&](int t, long long& s0) {
-                        const long long s = (kPool ? static_cast<long long>(perm[tile.first + t]) : (a0 + t) * np + pol) * IMG, s1 = (s + IMG + 15) & ~15ll;
+                        const long long s = (kPool ? static_cast<long long>(perm[tile.first + t]) : gm.agent(a0, t)) * IMG, s1 = (s + IMG + 15) & ~15ll;
                         s0 = s & ~15ll;
                         return static_cast<uint32_t>((s1 < end16 ? s1 : end16) - s0);
                     };
@@ -465,7 +460,7 @@ __global__ void __launch_bounds__(kThreads, 1) policy_features_kernel(const uint
             const long long a0 = (cta + static_cast<long long>(gi) * stride) * GA;
             const PoolTile tile = kPool ? tiles[tb + gi] : PoolTile{};
             if (kPool ? row < tile.count : a0 + row < rows) {
-                float4* dst = reinterpret_cast<float4*>(out + (kPool ? static_cast<long long>(perm[tile.first + row]) : (a0 + row) * np + pol) * FEAT + 16 * half);
+                float4* dst = reinterpret_cast<float4*>(out + (kPool ? static_cast<long long>(perm[tile.first + row]) : gm.agent(a0, row)) * FEAT + 16 * half);
                 const float* b2 = s_const + N1 + N2 + 16 * half;
 #pragma unroll
                 for (int c = 0; c < 16; c += 4)
@@ -574,6 +569,34 @@ __global__ void __launch_bounds__(256) lstm_cell_kernel(const uint4* __restrict_
     h16_out[idx] = make_uint4(p[0], p[1], p[2], p[3]);
 }
 
+inline auto features_kernel(WeightMap m) {
+    return m == WeightMap::Shared ? policy_features_kernel<WeightMap::Shared>
+                                  : m == WeightMap::PerAgent ? policy_features_kernel<WeightMap::PerAgent> : policy_features_kernel<WeightMap::Pool>;
+}
+inline int smem_bytes(WeightMap m) { return m == WeightMap::Shared ? TrunkSmem<false>::kSmemBytes : TrunkSmem<true>::kSmemBytes; }
+
+// ssd_policy_[pool_]features: policy_ids is null for a network handle
+int features(ssd_policy_t p, const uint8_t* obs, const uint8_t* policy_ids, int64_t num_agents, float* features, void* stream) {
+    const bool pool = policy_ids != nullptr;
+    if (!p || !obs || !features || num_agents < 0) return ssd::set_error(SSD_ERR_INVALID, "bad argument");
+    // ssd_policy_features reports misaligned pointers before a wrong kind of handle, ssd_policy_pool_features after it
+    const char* misaligned = "obs and features must be 16-byte aligned";
+    if (!pool && check_aligned({obs, features}, misaligned) != SSD_OK) return SSD_ERR_INVALID;
+    int rc = pool ? check_kind(p, HandleKind::Pool, "not a policy pool handle (ssd_policy_create_pool)")
+                  : check_kind(p, HandleKind::Net, "a policy pool handle takes ssd_policy_pool_features");
+    if (rc == SSD_OK) rc = check_aligned({obs, features}, misaligned);
+    if (rc != SSD_OK) return rc;
+    if (!pool && num_agents % p->num_policies != 0) return ssd::set_error(SSD_ERR_INVALID, "num_agents must be a multiple of num_policies");
+    if (num_agents == 0) return SSD_OK;
+    rc = setup(p, policy_ids, num_agents, stream);
+    if (rc != SSD_OK) return rc;
+    const Grid g = grid(p, num_agents);
+    const WeightMap map = weight_map(p);
+    features_kernel(map)<<<g.ctas, kThreads, smem_bytes(map), static_cast<cudaStream_t>(stream)>>>(
+        obs, num_agents, p->d_blob, features, p->num_policies, g.ctas_per_policy, p->d_perm, p->d_tiles, ssd::policy_pool::num_tiles(p));
+    return launched();
+}
+
 // Packs num_policies trunk weight sets (Keras layouts, consecutive behind each pointer) into a new handle; the caller has
 // checked num_policies against its map's limit.
 int create_trunk(int view_radius, int device, int num_policies, WeightMap map, const float* conv_w, const float* conv_b, const float* fc1_w,
@@ -584,7 +607,6 @@ int create_trunk(int view_radius, int device, int num_policies, WeightMap map, c
     if (2 * view_radius + 1 != V) return ssd::set_error(SSD_ERR_UNSUPPORTED, "the feature kernel is built for 15x15 observations (view radius 7)");
     const size_t blob_bytes = static_cast<size_t>(num_policies) * kBlobBytes;
     std::vector<uint8_t> blobs(blob_bytes, 0);
-    auto at = [](int rows, int n, int k) { return ((k >> 3) * rows + n) * 8 + (k & 7); };  // canonical K-major, no swizzle
     for (int q = 0; q < num_policies; ++q) {  // weight set q: arrays q of the num_policies consecutive ones behind each pointer
         uint8_t* blob = blobs.data() + static_cast<size_t>(q) * kBlobBytes;
         const float* cw = conv_w + q * (9 * 3 * NF);
@@ -605,7 +627,7 @@ int create_trunk(int view_radius, int device, int num_policies, WeightMap map, c
                     for (int dj = 0; dj < 3; ++dj)
                         for (int c = 0; c < 3; ++c) {
                             const __half h = __float2half_rn(cw[((di * 3 + dj) * 3 + c) * NF + f]);
-                            b1[at(N1, j * NF + f, di * ROWK + (j + dj) * 3 + c)] = h;
+                            b1[kmajor(N1, j * NF + f, di * ROWK + (j + dj) * 3 + c)] = h;
                             sum16 += static_cast<double>(__half2float(h));
                         }
                 // relu(conv((x - 128) / 255) + b) with the operand holding 1024 + x
@@ -613,9 +635,9 @@ int create_trunk(int view_radius, int device, int num_policies, WeightMap map, c
             }
         for (int i = 0; i < CO; ++i)  // Dense(32) kernel [1014][32], inputs flattened (i, j, f)
             for (int k = 0; k < CO * NF; ++k)
-                for (int n = 0; n < N2; ++n) b2[i * (K2 * N2) + at(N2, n, k)] = __float2half_rn(w1[(i * CO * NF + k) * N2 + n]);
+                for (int n = 0; n < N2; ++n) b2[i * (K2 * N2) + kmajor(N2, n, k)] = __float2half_rn(w1[(i * CO * NF + k) * N2 + n]);
         for (int k = 0; k < K3; ++k)
-            for (int n = 0; n < N3; ++n) b3[at(N3, n, k)] = __float2half_rn(w2[k * N3 + n]);
+            for (int n = 0; n < N3; ++n) b3[kmajor(N3, n, k)] = __float2half_rn(w2[k * N3 + n]);
         for (int n = 0; n < N2; ++n) cst[N1 + n] = b1v[n];
         for (int n = 0; n < N3; ++n) cst[N1 + N2 + n] = b2v[n];
     }
@@ -624,17 +646,12 @@ int create_trunk(int view_radius, int device, int num_policies, WeightMap map, c
     if (!p) return ssd::set_error(SSD_ERR_INVALID, "out of host memory");
     p->device = device;
     p->num_policies = num_policies;
-    p->pool = map == WeightMap::Pool;
+    p->kind = map == WeightMap::Pool ? HandleKind::Pool : HandleKind::Net;
     cudaError_t e = cudaSetDevice(device);
     if (e == cudaSuccess) e = cudaDeviceGetAttribute(&p->sms, cudaDevAttrMultiProcessorCount, device);
     if (e == cudaSuccess) e = cudaMalloc(&p->d_blob, blob_bytes);
     if (e == cudaSuccess) e = cudaMemcpy(p->d_blob, blobs.data(), blob_bytes, cudaMemcpyHostToDevice);
-    if (e == cudaSuccess && map == WeightMap::Pool)
-        e = cudaFuncSetAttribute(policy_features_kernel<WeightMap::Pool>, cudaFuncAttributeMaxDynamicSharedMemorySize, TrunkSmem<true>::kSmemBytes);
-    else if (e == cudaSuccess && num_policies == 1)
-        e = cudaFuncSetAttribute(policy_features_kernel<WeightMap::Shared>, cudaFuncAttributeMaxDynamicSharedMemorySize, TrunkSmem<false>::kSmemBytes);
-    else if (e == cudaSuccess)
-        e = cudaFuncSetAttribute(policy_features_kernel<WeightMap::PerAgent>, cudaFuncAttributeMaxDynamicSharedMemorySize, TrunkSmem<true>::kSmemBytes);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(features_kernel(weight_map(p)), cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes(weight_map(p)));
     if (e != cudaSuccess) {
         if (p->d_blob) cudaFree(p->d_blob);
         delete p;
@@ -664,50 +681,12 @@ int ssd_policy_create(int view_radius, int device, const float* conv_w, const fl
 }
 
 int ssd_policy_features(ssd_policy_t p, const uint8_t* obs, int64_t num_agents, float* features, void* stream) {
-    using namespace ssd::policy;
-    if (!p || !obs || !features || num_agents < 0) return ssd::set_error(SSD_ERR_INVALID, "bad argument");
-    if (reinterpret_cast<uintptr_t>(obs) % 16 != 0 || reinterpret_cast<uintptr_t>(features) % 16 != 0)
-        return ssd::set_error(SSD_ERR_INVALID, "obs and features must be 16-byte aligned");
-    if (p->pool) return ssd::set_error(SSD_ERR_INVALID, "a policy pool handle takes ssd_policy_pool_features");
-    if (p->moa) return ssd::set_error(SSD_ERR_INVALID, "an MOA handle takes ssd_moa_step");
-    const int np = p->num_policies;
-    if (num_agents % np != 0) return ssd::set_error(SSD_ERR_INVALID, "num_agents must be a multiple of num_policies");
-    if (num_agents == 0) return SSD_OK;
-    if (cudaSetDevice(p->device) != cudaSuccess) return ssd::set_error(SSD_ERR_CUDA, "cudaSetDevice failed");  // the blob and the stream live there
-    const cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (np == 1) {
-        const long long groups = (num_agents + GA - 1) / GA;
-        const int grid = static_cast<int>(groups < p->sms ? groups : p->sms);
-        policy_features_kernel<WeightMap::Shared><<<grid, kThreads, TrunkSmem<false>::kSmemBytes, st>>>(obs, num_agents, p->d_blob, features, 1, grid,
-                                                                                                      nullptr, nullptr, nullptr);
-    } else {  // P * floor(#SMs / P) CTAs at most, each serving one policy
-        const long long groups = (num_agents / np + GA - 1) / GA;
-        const int per = static_cast<int>(groups < p->sms / np ? groups : p->sms / np);
-        policy_features_kernel<WeightMap::PerAgent><<<np * per, kThreads, TrunkSmem<true>::kSmemBytes, st>>>(obs, num_agents, p->d_blob, features, np, per,
-                                                                                                           nullptr, nullptr, nullptr);
-    }
-    const cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return ssd::set_error(SSD_ERR_CUDA, cudaGetErrorString(e));
-    return SSD_OK;
+    return ssd::policy::features(p, obs, nullptr, num_agents, features, stream);
 }
 
 int ssd_policy_pool_features(ssd_policy_t p, const uint8_t* obs, const uint8_t* policy_ids, int64_t num_agents, float* features, void* stream) {
-    using namespace ssd::policy;
-    if (!p || !obs || !policy_ids || !features || num_agents < 0) return ssd::set_error(SSD_ERR_INVALID, "bad argument");
-    if (!p->pool) return ssd::set_error(SSD_ERR_INVALID, "not a policy pool handle (ssd_policy_create_pool)");
-    if (reinterpret_cast<uintptr_t>(obs) % 16 != 0 || reinterpret_cast<uintptr_t>(features) % 16 != 0)
-        return ssd::set_error(SSD_ERR_INVALID, "obs and features must be 16-byte aligned");
-    if (num_agents == 0) return SSD_OK;
-    const int rc = ssd::policy_pool::assign(p, policy_ids, num_agents, stream);   // sets the device
-    if (rc != SSD_OK) return rc;
-    // a persistent grid over the tile table, whose length only the device knows
-    const long long tiles = ssd::policy_pool::max_tiles(num_agents, p->num_policies);
-    const int grid = static_cast<int>(tiles < p->sms ? tiles : p->sms);
-    policy_features_kernel<WeightMap::Pool><<<grid, kThreads, TrunkSmem<true>::kSmemBytes, static_cast<cudaStream_t>(stream)>>>(
-        obs, num_agents, p->d_blob, features, p->num_policies, grid, p->d_perm, p->d_tiles, p->d_counts + 512);
-    const cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return ssd::set_error(SSD_ERR_CUDA, cudaGetErrorString(e));
-    return SSD_OK;
+    if (!policy_ids) return ssd::set_error(SSD_ERR_INVALID, "bad argument");
+    return ssd::policy::features(p, obs, policy_ids, num_agents, features, stream);
 }
 
 int ssd_policy_lstm_cell(const void* gates_bf16, const float* bias, const float* c_prev, float* c_out, float* h_out, void* h_bf16_out,
@@ -715,17 +694,14 @@ int ssd_policy_lstm_cell(const void* gates_bf16, const float* bias, const float*
     using namespace ssd::policy;
     if (!gates_bf16 || !bias || !c_prev || !c_out || !h_out || !h_bf16_out || num_agents < 0) return ssd::set_error(SSD_ERR_INVALID, "bad argument");
     if (units <= 0 || units % 8 != 0) return ssd::set_error(SSD_ERR_INVALID, "units must be a positive multiple of 8");
-    const void* ptrs[6] = {gates_bf16, bias, c_prev, c_out, h_out, h_bf16_out};
-    for (const void* q : ptrs)
-        if (reinterpret_cast<uintptr_t>(q) % 16 != 0) return ssd::set_error(SSD_ERR_INVALID, "pointers must be 16-byte aligned");
+    const int rc = check_aligned({gates_bf16, bias, c_prev, c_out, h_out, h_bf16_out}, "pointers must be 16-byte aligned");
+    if (rc != SSD_OK) return rc;
     if (num_agents == 0) return SSD_OK;
     const long long n = num_agents * (units / 8);
     lstm_cell_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
         static_cast<const uint4*>(gates_bf16), bias, reinterpret_cast<const float4*>(c_prev), reinterpret_cast<float4*>(c_out),
         reinterpret_cast<float4*>(h_out), static_cast<uint4*>(h_bf16_out), num_agents, units);
-    const cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return ssd::set_error(SSD_ERR_CUDA, cudaGetErrorString(e));
-    return SSD_OK;
+    return launched();
 }
 
 void ssd_policy_destroy(ssd_policy_t p) {

@@ -2,27 +2,18 @@
 // as ONE kernel behind ssd_policy_lstm_heads: per group of 128 agents (= UMMA M, one TMEM lane per agent)
 //
 //   A[128 x 160]  = fp16([features | h])                                  built from HBM into shared memory
-//   G[128 x 512]  = A * [W; U]            (Keras gate order i, f, c~, o)   20 MMAs 128 x 256 x 16, all of tensor memory
+//   G[128 x 512]  = A * [W; U]                                            the gate GEMM of ssd_policy_lstm.cuh
 //   c' = sigmoid(f) c + sigmoid(i) tanh(c~),  h' = sigmoid(o) tanh(c')     drain: thread = agent, 8 warps split the units
 //   Y[128 x 16]   = fp16(h') * [logits_w | value_w]                        8 MMAs 128 x 16 x 16 into the freed columns
 //   action        = argmax(logits + Gumbel noise)                          Philox4x32-10 keyed (seed; agent, counter)
 //
-// The recurrent state lives in HBM in a TILED layout chosen for this kernel: [group of 128 agents][block of 16 units (8)]
-// [agent in group (128)][16 floats] -- element (agent m, unit u) at ((m / 128 * 8 + u / 16) * 128 + m % 128) * 16 + u % 16.
-// A thread owns an agent and works through 16 units at a time, so a warp's loads and stores of c / h are 2 KB contiguous
-// (with row-major [M][128] state they were 64-byte pieces 512 bytes apart and the cell update ran at 2.9 TB/s of HBM).
-// HBM traffic per agent: 128 B features + 1 KB (h, c) in, 1 KB (h', c') + logits / value / action out -- one pass, against
-// ~7.5 KB for the unfused gate GEMMs + cell update.  The B operand [W; U] (160 KB as fp16) stays resident in shared memory;
-// the grid is persistent (one CTA per SM).
-#include <cuda_fp16.h>
-
+// The recurrent state lives in HBM in the tiled layout of ssd_policy_lstm.cuh.  HBM traffic per agent: 128 B features + 1 KB
+// (h, c) in, 1 KB (h', c') + logits / value / action out -- one pass, against ~7.5 KB for the unfused gate GEMMs + cell
+// update.  The B operand [W; U] (160 KB as fp16) stays resident in shared memory; the grid is persistent (one CTA per SM).
 #include <cstdio>
-#include <new>
 #include <vector>
 
-#include "ssd_internal.h"
-#include "ssd_policy.h"
-#include "ssd_umma.cuh"
+#include "ssd_policy_lstm.cuh"
 
 #ifdef SSD_POLICY_TIMING  // profiles/micro/policy_head_timing.cu: cycles per phase of thread 0 of CTA 0
 __device__ unsigned long long g_head_cycles[8];
@@ -37,38 +28,70 @@ __device__ unsigned long long g_head_cycles[8];
 
 namespace ssd {
 namespace policy_head {
-using namespace ssd::umma;
+using namespace ssd::lstm;
 
-constexpr int GA = 128, U = 128, KX = 32, K = KX + U, NG = 4 * U, NH = 16;
-constexpr int kThreads = 256;
-constexpr int kBBytes = (K / 8) * NG * 16;         // 163 840: [W; U] K-major, element (n, k) at ((k / 8) * 512 + n) * 16 + (k % 8) * 2
+constexpr int NH = 16;
 constexpr int kBHBytes = (U / 8) * NH * 16;        // 4 096: [logits_w | value_w | 0]
 constexpr int kConstFloats = NG + NH;              // gate bias, head bias
 constexpr int kBlobBytes = kBBytes + kBHBytes + kConstFloats * 4;   // 170 048
 constexpr int kOffB = 0, kOffBH = kBBytes, kOffConst = kOffBH + kBHBytes;
 constexpr int kOffA = (kOffConst + kConstFloats * 4 + 127) & ~127;   // [128 x 160] fp16, later fp16(h') [128 x 128]
-constexpr int kABytes = (K / 8) * GA * 16;         // 40 960
 constexpr int kOffBar = kOffA + kABytes;
 constexpr int kSmemBytes = kOffBar + 16;
 static_assert(kBlobBytes % 16 == 0 && kSmemBytes <= 227 * 1024, "one CTA per SM");
 
-__device__ __forceinline__ uint32_t pack_h2(float lo, float hi) {
-    const __half2 v = __floats2half2_rn(lo, hi);
-    return *reinterpret_cast<const uint32_t*>(&v);
+// Start of a kernel: the mbarrier, all 512 columns of tensor memory and the resident weights (`bytes` of blob) at smem[0].
+// Returns the tensor-memory base.
+__device__ __forceinline__ uint32_t prologue(uint8_t* smem, const uint8_t* blob, int bytes, uint64_t* bar, uint32_t* s_tmem) {
+    if (threadIdx.x == 0) mbar_init(bar, 1);
+    if (threadIdx.x < 32) tmem_alloc(s_tmem, 512);
+    copy_blob(smem, blob, bytes);
+    fence_async_smem();
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+    return *s_tmem;
 }
-// one MUFU op each (tanh.approx.f32, ~2^-11 relative error: below the fp16 rounding of the GEMM operands); the cell update
-// is transcendental-bound: 5 per unit, 640 per agent
-__device__ __forceinline__ float tanh_fast(float x) {
-    float y;
-    asm("tanh.approx.f32 %0, %1;" : "=f"(y) : "f"(x));
-    return y;
-}
-__device__ __forceinline__ float sigmoid_fast(float x) { return fmaf(tanh_fast(0.5f * x), 0.5f, 0.5f); }
 
-// kPerAgent: agent m = b * P + p uses weight set p (blob + p * kBlobBytes).  As in the trunk, CTA c serves policy c % P only
-// (groups g = c / P, c / P + cpp, ... of the agents (b, p), b in [128 g, 128 g + 128)), so its [W; U] is loaded once; features
-// are read as 128-byte rows P * 128 bytes apart, outputs are written to agent-major rows, and the recurrent state of that
-// group is state group p * ceil(B / 128) + g.  The sampler keys Philox by the agent-major index m in all variants.
+// A = fp16([features | h]) of the group's `rem` live rows into `a`, rows past them zero.  agent(r): the feature row of row r;
+// state(r): the offset, in 16-float pieces, of row r's first unit block in the tiled state (block b at + b * 128).  HBM is read
+// in long contiguous runs (features: a 128-byte row per eight lanes; h: the tiled state, 64 bytes per lane, 2 KB per warp -- a
+// thread walking a row-major row in 32-byte steps reached 2.3 TB/s).  All loads before the stores: the compiler keeps a
+// global load below a store through a generic pointer.
+template <class Agent, class State>
+__device__ __forceinline__ void gate_operand(uint8_t* a, const float* __restrict__ feat, const float* h_in, int rem, Agent agent, State state) {
+    const int tid = threadIdx.x;
+    const int seg = tid & 7, r8 = tid >> 3;                  // features: 32 rows per pass, 4 passes, a 128-byte row per eight lanes
+    const int hrow = tid & (GA - 1), hb0 = (tid >> 7) * 4;   // h: thread = (agent, four of the eight 16-unit blocks), 64 bytes per block
+    const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
+    float4 vx[4], vh[4][4];
+#pragma unroll
+    for (int ps = 0; ps < 4; ++ps) {
+        const int row = ps * 32 + r8;
+        vx[ps] = row < rem ? __ldcs(reinterpret_cast<const float4*>(feat + agent(row) * KX) + seg) : z;
+    }
+    const long long hbase = state(hrow);
+#pragma unroll
+    for (int b = 0; b < 4; ++b) {
+        const float4* src = reinterpret_cast<const float4*>(h_in + (hbase + (hb0 + b) * GA) * 16);
+#pragma unroll
+        for (int j = 0; j < 4; ++j) vh[b][j] = hrow < rem ? __ldcs(src + j) : z;
+    }
+#pragma unroll
+    for (int ps = 0; ps < 4; ++ps)   // elements 4 seg .. 4 seg + 3 of the 32 features: half of operand chunk seg / 2
+        *reinterpret_cast<uint2*>(a + (seg >> 1) * (GA * 16) + (ps * 32 + r8) * 16 + (seg & 1) * 8) =
+            make_uint2(pack_h2(vx[ps].x, vx[ps].y), pack_h2(vx[ps].z, vx[ps].w));
+#pragma unroll
+    for (int b = 0; b < 4; ++b)      // units 16 (hb0 + b) .. + 15: operand chunks 4 + 2 (hb0 + b) and the next
+#pragma unroll
+        for (int hf = 0; hf < 2; ++hf)
+            *reinterpret_cast<uint4*>(a + (KX / 8 + 2 * (hb0 + b) + hf) * (GA * 16) + hrow * 16) =
+                make_uint4(pack_h2(vh[b][2 * hf].x, vh[b][2 * hf].y), pack_h2(vh[b][2 * hf].z, vh[b][2 * hf].w),
+                           pack_h2(vh[b][2 * hf + 1].x, vh[b][2 * hf + 1].y), pack_h2(vh[b][2 * hf + 1].z, vh[b][2 * hf + 1].w));
+}
+
+// Shared / PerAgent: the groups of GroupMap (ssd_policy.h); features are read as 128-byte rows P * 128 bytes apart and
+// outputs are written to agent-major rows.  The sampler keys Philox by the agent-major index m in all variants.
 //
 // WeightMap::Pool: a group is one tile of the assignment (ssd_policy_pool.cu), agents perm[first, first + count) of one policy;
 // CTA c takes tiles [c T / G, (c + 1) T / G) and reloads the resident weights when the policy changes (the tiles are in
@@ -92,94 +115,49 @@ lstm_heads_kernel(const float* __restrict__ feat, const float* h_in, const float
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     uint64_t* bar = reinterpret_cast<uint64_t*>(smem + kOffBar);
     const float* s_bias = reinterpret_cast<const float*>(smem + kOffConst);
-    const int np = kPerAgent ? num_policies : 1;
-    const int pol = kPerAgent ? static_cast<int>(blockIdx.x) % np : 0;                       // this CTA's weight set
+    const GroupMap<kMap> gm(M, num_policies, ctas_per_policy);
     const long long nt = kPool ? *num_tiles : 0;
-    const long long cta = kPool ? nt * blockIdx.x / gridDim.x                                // pool: its first tile
-                                : kPerAgent ? blockIdx.x / np : blockIdx.x;                  // its index among the CTAs of that policy
-    const long long stride = kPool ? 1 : kPerAgent ? ctas_per_policy : gridDim.x;
-    const long long rows = kPerAgent ? M / np : M;                                           // agents per policy
+    const long long first = kPool ? nt * blockIdx.x / gridDim.x : gm.cta;                  // pool: its first tile
+    const long long end = kPool ? nt * (blockIdx.x + 1) / gridDim.x : gm.n_groups;          // pool: the end of its tiles
+    const long long stride = kPool ? 1 : gm.stride;
     const uint8_t* const blob0 = blob;
     int cur = 0;   // pool: the weight set in shared memory
     if (kPool) {
-        cur = cta < nt * (blockIdx.x + 1) / gridDim.x ? tiles[cta].policy : 0;
+        cur = first < end ? tiles[first].policy : 0;
         blob += static_cast<long long>(cur) * kBlobBytes;
     } else if (kPerAgent) {
-        blob += static_cast<long long>(pol) * kBlobBytes;
+        blob += static_cast<long long>(gm.pol) * kBlobBytes;
     }
-    if (tid == 0) mbar_init(bar, 1);
-    if (warp == 0) tmem_alloc(&s_tmem, 512);
-    for (int i = tid; i < (kBlobBytes >> 4); i += kThreads) reinterpret_cast<uint4*>(smem)[i] = reinterpret_cast<const uint4*>(blob)[i];
-    fence_async_smem();
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem = s_tmem;
+    const uint32_t tmem = prologue(smem, blob, kBlobBytes, bar, &s_tmem);
     const uint32_t sA = smem_u32(smem + kOffA), sB = smem_u32(smem + kOffB), sBH = smem_u32(smem + kOffBH);
-    constexpr uint32_t kIG = umma_idesc(GA, 256), kIH = umma_idesc(GA, NH);
+    constexpr uint32_t kIH = umma_idesc(GA, NH);
     uint32_t parity = 0;
 
-    const long long n_groups = kPool ? nt * (blockIdx.x + 1) / gridDim.x : (rows + GA - 1) / GA;   // pool: the end of its tiles
     SSD_HT_DECL;
-    for (long long g = cta; g < n_groups; g += stride) {
-        const long long a0 = g * GA, sg = pol * n_groups + g;   // first agent row of the group in its policy; its state group
+    for (long long g = first; g < end; g += stride) {
+        const long long a0 = g * GA, sg = gm.state_group(g);   // first agent row of the group in its policy; its state group
         const PoolTile tile = kPool ? tiles[g] : PoolTile{};
         if (kPool && tile.policy != cur) {   // the previous group is complete (the barrier at the end of the loop)
             cur = tile.policy;
-            const uint4* src = reinterpret_cast<const uint4*>(blob0 + static_cast<long long>(cur) * kBlobBytes);
-            for (int i = tid; i < (kBlobBytes >> 4); i += kThreads) reinterpret_cast<uint4*>(smem)[i] = src[i];
+            copy_blob(smem, blob0 + static_cast<long long>(cur) * kBlobBytes, kBlobBytes);
             fence_async_smem();
             __syncthreads();
         }
-        // pool: agent of row r of the tile, its offset in the agent-major tiled state (element (m, u) at (that + u / 16 * 128) * 16 + u % 16)
-        auto agent = [&](int r) { return static_cast<long long>(perm[tile.first + r]); };
-        auto state_row = [](long long m) { return (m >> 7) * (U / 16) * GA + (m & (GA - 1)); };
-        const int rem = kPool ? tile.count : static_cast<int>(rows - a0 < GA ? rows - a0 : GA);
-        {   // A = fp16([features | h]).  HBM is read in long contiguous runs (features: a 128-byte row per eight lanes; h: the tiled
-            // state, 64 bytes per lane, 2 KB per warp -- a thread walking a row-major row in 32-byte steps reached 2.3 TB/s).
-            // All loads before the stores: the compiler keeps a global load below a store through a generic pointer.
-            const int seg = tid & 7, r8 = tid >> 3;          // features: 32 rows per pass, 4 passes, a 128-byte row per eight lanes
-            const int hrow = tid & (GA - 1), hb0 = (tid >> 7) * 4;   // h: thread = (agent, four of the eight 16-unit blocks), 64 bytes per block
-            const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
-            float4 vx[4], vh[4][4];
-#pragma unroll
-            for (int ps = 0; ps < 4; ++ps) {
-                const int row = ps * 32 + r8;
-                vx[ps] = row < rem ? __ldcs(reinterpret_cast<const float4*>(feat + (kPool ? agent(row) : (a0 + row) * np + pol) * KX) + seg) : z;
-            }
-            const long long hbase = kPool && hrow < rem ? state_row(agent(hrow)) : 0;
-#pragma unroll
-            for (int b = 0; b < 4; ++b) {
-                const float4* src = reinterpret_cast<const float4*>(h_in + (kPool ? (hbase + (hb0 + b) * GA) * 16 : ((sg * (U / 16) + hb0 + b) * GA + hrow) * 16));
-#pragma unroll
-                for (int j = 0; j < 4; ++j) vh[b][j] = hrow < rem ? __ldcs(src + j) : z;
-            }
-#pragma unroll
-            for (int ps = 0; ps < 4; ++ps)   // elements 4 seg .. 4 seg + 3 of the 32 features: half of operand chunk seg / 2
-                *reinterpret_cast<uint2*>(smem + kOffA + (seg >> 1) * (GA * 16) + (ps * 32 + r8) * 16 + (seg & 1) * 8) =
-                    make_uint2(pack_h2(vx[ps].x, vx[ps].y), pack_h2(vx[ps].z, vx[ps].w));
-#pragma unroll
-            for (int b = 0; b < 4; ++b)      // units 16 (hb0 + b) .. + 15: operand chunks 4 + 2 (hb0 + b) and the next
-#pragma unroll
-                for (int hf = 0; hf < 2; ++hf)
-                    *reinterpret_cast<uint4*>(smem + kOffA + (KX / 8 + 2 * (hb0 + b) + hf) * (GA * 16) + hrow * 16) =
-                        make_uint4(pack_h2(vh[b][2 * hf].x, vh[b][2 * hf].y), pack_h2(vh[b][2 * hf].z, vh[b][2 * hf].w),
-                                   pack_h2(vh[b][2 * hf + 1].x, vh[b][2 * hf + 1].y), pack_h2(vh[b][2 * hf + 1].z, vh[b][2 * hf + 1].w));
-        }
+        const int rem = kPool ? tile.count : static_cast<int>(gm.rows - a0 < GA ? gm.rows - a0 : GA);
+        // agent of row r; its offset in the tiled state (pool: agent-major, element (m, u) at (that + u / 16 * 128) * 16 + u % 16)
+        auto agent = [&](int r) { return kPool ? static_cast<long long>(perm[tile.first + r]) : gm.agent(a0, r); };
+        auto state = [&](int r) -> long long {
+            if (!kPool) return sg * (U / 16) * GA + r;
+            if (r >= rem) return 0;   // a pool tile's rows past its count have no perm entry
+            const long long m = agent(r);
+            return (m >> 7) * (U / 16) * GA + (m & (GA - 1));
+        };
+        gate_operand(smem + kOffA, feat, h_in, rem, agent, state);
         fence_async_smem();
         tc_fence_before();
         __syncthreads();
         SSD_HT(0);
-        if (warp == 0 && elect_one()) {  // gates: two column halves of 256, k-steps interleaved
-            tc_fence_after();
-#pragma unroll
-            for (int ks = 0; ks < K / 16; ++ks)
-#pragma unroll
-                for (int half = 0; half < 2; ++half)
-                    umma_f16(tmem + half * 256, umma_desc(sA + ks * 2 * GA * 16, GA * 16, 128),
-                             umma_desc(sB + half * 256 * 16 + ks * 2 * NG * 16, NG * 16, 128), kIG, ks > 0);
-            umma_commit(bar);
-        }
+        if (warp == 0 && elect_one()) gate_gemm(tmem, sA, sB, bar);
         mbar_wait(bar, parity);
         parity ^= 1;
         tc_fence_after();
@@ -188,8 +166,7 @@ lstm_heads_kernel(const float* __restrict__ feat, const float* h_in, const float
             const int q = warp & 3, row = q * 32 + lane, uh = warp >> 2;
             const uint32_t trow = tmem + (static_cast<uint32_t>(q * 32) << 16);
             const bool live = row < rem;
-            const long long tile0 = kPool ? (live ? (state_row(agent(row)) + uh * 4 * GA) * 16 : 0)
-                                          : ((sg * (U / 16) + uh * 4) * GA + row) * 16;   // this agent's 16 floats of unit block 4 uh; + GA * 16 per block
+            const long long tile0 = (state(row) + uh * 4 * GA) * 16;   // this agent's 16 floats of unit block 4 uh; + GA * 16 per block
             float4 cn[4];   // the next 16 units of c, fetched one iteration ahead
 #pragma unroll
             for (int e = 0; e < 4; ++e) cn[e] = live ? __ldcs(reinterpret_cast<const float4*>(c_in + tile0) + e) : make_float4(0.f, 0.f, 0.f, 0.f);
@@ -251,7 +228,7 @@ lstm_heads_kernel(const float* __restrict__ feat, const float* h_in, const float
             tmem_ld16(tmem + (static_cast<uint32_t>(warp * 32) << 16), y);
             tmem_ld_wait();
             if (row < rem) {
-                const long long m = kPool ? agent(row) : (a0 + row) * np + pol;
+                const long long m = agent(row);
                 const float* hb = s_bias + NG;
                 float best = -3.0e38f;
                 int arg = 0;
@@ -319,11 +296,16 @@ lstm_heads_kernel(const float* __restrict__ feat, const float* h_in, const float
     if (warp == 0) tmem_free(tmem, 512);
 }
 
+template <bool kDist>
+auto heads_kernel(WeightMap m) {
+    return m == WeightMap::Shared ? lstm_heads_kernel<WeightMap::Shared, kDist>
+                                  : m == WeightMap::PerAgent ? lstm_heads_kernel<WeightMap::PerAgent, kDist> : lstm_heads_kernel<WeightMap::Pool, kDist>;
+}
+
 // both instantiations of a weight map (plain head and ssd_policy_lstm_heads_dist) take the whole of shared memory
-template <WeightMap kMap>
-cudaError_t allow_smem() {
-    const cudaError_t e = cudaFuncSetAttribute(lstm_heads_kernel<kMap, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
-    return e != cudaSuccess ? e : cudaFuncSetAttribute(lstm_heads_kernel<kMap, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
+cudaError_t allow_smem(WeightMap m) {
+    const cudaError_t e = cudaFuncSetAttribute(heads_kernel<false>(m), cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
+    return e != cudaSuccess ? e : cudaFuncSetAttribute(heads_kernel<true>(m), cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
 }
 
 // the arguments only ssd_policy_lstm_heads_dist / ssd_policy_pool_lstm_heads_dist take
@@ -339,68 +321,32 @@ bool bad_dist_args(int mode, const int8_t* actions) {
     return false;
 }
 
-// ssd_policy_lstm_heads (kDist false: mode, logp and entropy unused) and ssd_policy_lstm_heads_dist
+// ssd_policy_[pool_]lstm_heads[_dist]: policy_ids is null for a network handle (kDist false: mode, logp and entropy unused)
 template <bool kDist>
-int heads(ssd_policy_t p, const float* features, const float* h_in, const float* c_in, float* h_out, float* c_out, float* logits, float* value,
-          int mode, int8_t* actions, float* logp, float* entropy, int64_t num_agents, uint64_t seed, uint32_t counter, void* stream) {
+int heads(ssd_policy_t p, const float* features, const uint8_t* policy_ids, const float* h_in, const float* c_in, float* h_out, float* c_out,
+          float* logits, float* value, int mode, int8_t* actions, float* logp, float* entropy, int64_t num_agents, uint64_t seed,
+          uint32_t counter, void* stream) {
+    using namespace ssd::policy;
+    const bool pool = policy_ids != nullptr;
     if (!p || !features || !h_in || !c_in || !h_out || !c_out || !logits || !value || num_agents < 0) return ssd::set_error(SSD_ERR_INVALID, "bad argument");
     if (kDist && bad_dist_args(mode, actions)) return SSD_ERR_INVALID;
-    if (p->pool)
-        return ssd::set_error(SSD_ERR_INVALID, kDist ? "a policy pool handle takes ssd_policy_pool_lstm_heads_dist"
-                                                     : "a policy pool handle takes ssd_policy_pool_lstm_heads");
-    if (p->moa) return ssd::set_error(SSD_ERR_INVALID, "an MOA handle takes ssd_moa_step");
-    if (!p->d_head_blob) return ssd::set_error(SSD_ERR_INVALID, "ssd_policy_set_head has not been called");
-    const void* ptrs[5] = {features, h_in, c_in, h_out, c_out};
-    for (const void* q : ptrs)
-        if (reinterpret_cast<uintptr_t>(q) % 16 != 0) return ssd::set_error(SSD_ERR_INVALID, "features and state pointers must be 16-byte aligned");
-    const int np = p->num_policies;
-    if (num_agents % np != 0) return ssd::set_error(SSD_ERR_INVALID, "num_agents must be a multiple of num_policies");
-    if (num_agents == 0) return SSD_OK;
-    if (cudaSetDevice(p->device) != cudaSuccess) return ssd::set_error(SSD_ERR_CUDA, "cudaSetDevice failed");  // the blob and the stream live there
-    const cudaStream_t st = static_cast<cudaStream_t>(stream);
-    const uint32_t s_lo = static_cast<uint32_t>(seed), s_hi = static_cast<uint32_t>(seed >> 32);
-    if (np == 1) {
-        const long long groups = (num_agents + GA - 1) / GA;
-        const int grid = static_cast<int>(groups < p->sms ? groups : p->sms);
-        lstm_heads_kernel<WeightMap::Shared, kDist><<<grid, kThreads, kSmemBytes, st>>>(features, h_in, c_in, h_out, c_out, logits, value, actions,
-                                                                                       num_agents, p->num_outputs, p->d_head_blob, s_lo, s_hi, counter,
-                                                                                       1, grid, nullptr, nullptr, nullptr, mode, logp, entropy);
-    } else {  // P * floor(#SMs / P) CTAs at most, each serving one policy
-        const long long groups = (num_agents / np + GA - 1) / GA;
-        const int per = static_cast<int>(groups < p->sms / np ? groups : p->sms / np);
-        lstm_heads_kernel<WeightMap::PerAgent, kDist><<<np * per, kThreads, kSmemBytes, st>>>(features, h_in, c_in, h_out, c_out, logits, value, actions,
-                                                                                             num_agents, p->num_outputs, p->d_head_blob, s_lo, s_hi,
-                                                                                             counter, np, per, nullptr, nullptr, nullptr, mode, logp,
-                                                                                             entropy);
-    }
-    const cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return ssd::set_error(SSD_ERR_CUDA, cudaGetErrorString(e));
-    return SSD_OK;
-}
-
-// ssd_policy_pool_lstm_heads and ssd_policy_pool_lstm_heads_dist
-template <bool kDist>
-int pool_heads(ssd_policy_t p, const float* features, const uint8_t* policy_ids, const float* h_in, const float* c_in, float* h_out, float* c_out,
-               float* logits, float* value, int mode, int8_t* actions, float* logp, float* entropy, int64_t num_agents, uint64_t seed,
-               uint32_t counter, void* stream) {
-    if (!p || !features || !policy_ids || !h_in || !c_in || !h_out || !c_out || !logits || !value || num_agents < 0)
-        return ssd::set_error(SSD_ERR_INVALID, "bad argument");
-    if (kDist && bad_dist_args(mode, actions)) return SSD_ERR_INVALID;
-    if (!p->pool) return ssd::set_error(SSD_ERR_INVALID, "not a policy pool handle (ssd_policy_create_pool)");
-    const void* ptrs[5] = {features, h_in, c_in, h_out, c_out};
-    for (const void* q : ptrs)
-        if (reinterpret_cast<uintptr_t>(q) % 16 != 0) return ssd::set_error(SSD_ERR_INVALID, "features and state pointers must be 16-byte aligned");
-    if (num_agents == 0) return SSD_OK;
-    const int rc = ssd::policy_pool::assign(p, policy_ids, num_agents, stream);   // sets the device
+    int rc = pool ? check_kind(p, HandleKind::Pool, "not a policy pool handle (ssd_policy_create_pool)")
+                  : check_kind(p, HandleKind::Net, kDist ? "a policy pool handle takes ssd_policy_pool_lstm_heads_dist"
+                                                         : "a policy pool handle takes ssd_policy_pool_lstm_heads");
     if (rc != SSD_OK) return rc;
-    const long long tiles = ssd::policy_pool::max_tiles(num_agents, p->num_policies);
-    const int grid = static_cast<int>(tiles < p->sms ? tiles : p->sms);
-    lstm_heads_kernel<WeightMap::Pool, kDist><<<grid, kThreads, kSmemBytes, static_cast<cudaStream_t>(stream)>>>(
+    if (!p->d_head_blob) return ssd::set_error(SSD_ERR_INVALID, "ssd_policy_set_head has not been called");
+    rc = check_aligned({features, h_in, c_in, h_out, c_out}, "features and state pointers must be 16-byte aligned");
+    if (rc != SSD_OK) return rc;
+    if (!pool && num_agents % p->num_policies != 0) return ssd::set_error(SSD_ERR_INVALID, "num_agents must be a multiple of num_policies");
+    if (num_agents == 0) return SSD_OK;
+    rc = setup(p, policy_ids, num_agents, stream);
+    if (rc != SSD_OK) return rc;
+    const Grid g = grid(p, num_agents);
+    heads_kernel<kDist>(weight_map(p))<<<g.ctas, kThreads, kSmemBytes, static_cast<cudaStream_t>(stream)>>>(
         features, h_in, c_in, h_out, c_out, logits, value, actions, num_agents, p->num_outputs, p->d_head_blob, static_cast<uint32_t>(seed),
-        static_cast<uint32_t>(seed >> 32), counter, p->num_policies, grid, p->d_perm, p->d_tiles, p->d_counts + 512, mode, logp, entropy);
-    const cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return ssd::set_error(SSD_ERR_CUDA, cudaGetErrorString(e));
-    return SSD_OK;
+        static_cast<uint32_t>(seed >> 32), counter, p->num_policies, g.ctas_per_policy, p->d_perm, p->d_tiles, ssd::policy_pool::num_tiles(p), mode,
+        logp, entropy);
+    return launched();
 }
 
 }  // namespace policy_head
@@ -414,8 +360,9 @@ int ssd_policy_set_head_n(ssd_policy_t p, int num_policies, int units, int num_o
     if (!p) return ssd::set_error(SSD_ERR_INVALID, "null argument");
     if (num_policies < 1 || num_policies > SSD_MAX_AGENTS) return ssd::set_error(SSD_ERR_INVALID, "num_policies must be 1..SSD_MAX_AGENTS");
     if (num_policies != p->num_policies) return ssd::set_error(SSD_ERR_INVALID, "the head must have as many weight sets as the trunk");
-    if (p->pool) return ssd::set_error(SSD_ERR_INVALID, "a policy pool's head is loaded by ssd_policy_create_pool");
-    if (p->moa) return ssd::set_error(SSD_ERR_INVALID, "an MOA handle is loaded by ssd_moa_create");
+    const int rc = ssd::policy::check_kind(p, HandleKind::Net, "a policy pool's head is loaded by ssd_policy_create_pool",
+                                           "an MOA handle is loaded by ssd_moa_create");
+    if (rc != SSD_OK) return rc;
     return ssd::policy_head::set_head(p, units, num_outputs, lstm_w, lstm_u, lstm_b, logits_w, logits_b, value_w, value_b);
 }
 #pragma GCC visibility pop
@@ -430,27 +377,20 @@ int ssd::policy_head::set_head(SsdPolicy* p, int units, int num_outputs, const f
     if (num_outputs < 1 || num_outputs > NH - 1) return ssd::set_error(SSD_ERR_UNSUPPORTED, "1..15 policy outputs");
     const size_t blob_bytes = static_cast<size_t>(num_policies) * kBlobBytes;
     std::vector<uint8_t> blobs(blob_bytes, 0);
-    auto at = [](int rows, int n, int k) { return ((k >> 3) * rows + n) * 8 + (k & 7); };  // canonical K-major, no swizzle
+    using ssd::policy::kmajor;
     for (int q = 0; q < num_policies; ++q) {  // weight set q: arrays q of the num_policies consecutive ones behind each pointer
         uint8_t* blob = blobs.data() + static_cast<size_t>(q) * kBlobBytes;
-        const float* lw = lstm_w + static_cast<size_t>(q) * KX * NG;
-        const float* lu = lstm_u + static_cast<size_t>(q) * U * NG;
-        const float* lb = lstm_b + q * NG;
         const float* ow = logits_w + q * U * num_outputs;
         const float* ob = logits_b + q * num_outputs;
         const float* vw = value_w + q * U;
         const float* vb = value_b + q;
-        __half* b = reinterpret_cast<__half*>(blob + kOffB);
         __half* bh = reinterpret_cast<__half*>(blob + kOffBH);
         float* cst = reinterpret_cast<float*>(blob + kOffConst);
-        for (int n = 0; n < NG; ++n) {   // Keras LSTM: kernel [32][4u], recurrent kernel [u][4u], gates i, f, c~, o
-            for (int k = 0; k < KX; ++k) b[at(NG, n, k)] = __float2half_rn(lw[k * NG + n]);
-            for (int k = 0; k < U; ++k) b[at(NG, n, KX + k)] = __float2half_rn(lu[k * NG + n]);
-            cst[n] = lb[n];
-        }
+        pack_gates(reinterpret_cast<__half*>(blob + kOffB), cst, lstm_w + static_cast<size_t>(q) * KX * NG, lstm_u + static_cast<size_t>(q) * U * NG,
+                   lstm_b + q * NG);
         for (int k = 0; k < U; ++k) {
-            for (int n = 0; n < num_outputs; ++n) bh[at(NH, n, k)] = __float2half_rn(ow[k * num_outputs + n]);
-            bh[at(NH, num_outputs, k)] = __float2half_rn(vw[k]);
+            for (int n = 0; n < num_outputs; ++n) bh[kmajor(NH, n, k)] = __float2half_rn(ow[k * num_outputs + n]);
+            bh[kmajor(NH, num_outputs, k)] = __float2half_rn(vw[k]);
         }
         for (int n = 0; n < num_outputs; ++n) cst[NG + n] = ob[n];
         cst[NG + num_outputs] = vb[0];
@@ -458,9 +398,7 @@ int ssd::policy_head::set_head(SsdPolicy* p, int units, int num_outputs, const f
     cudaError_t e = cudaSetDevice(p->device);
     if (e == cudaSuccess && !p->d_head_blob) e = cudaMalloc(&p->d_head_blob, blob_bytes);
     if (e == cudaSuccess) e = cudaMemcpy(p->d_head_blob, blobs.data(), blob_bytes, cudaMemcpyHostToDevice);
-    if (e == cudaSuccess && p->pool) e = allow_smem<WeightMap::Pool>();
-    else if (e == cudaSuccess && num_policies == 1) e = allow_smem<WeightMap::Shared>();
-    else if (e == cudaSuccess) e = allow_smem<WeightMap::PerAgent>();
+    if (e == cudaSuccess) e = allow_smem(ssd::policy::weight_map(p));
     if (e != cudaSuccess) return ssd::set_error(SSD_ERR_CUDA, cudaGetErrorString(e));
     p->units = units;
     p->num_outputs = num_outputs;
@@ -477,29 +415,31 @@ int ssd_policy_set_head(ssd_policy_t p, int units, int num_outputs, const float*
 
 int ssd_policy_lstm_heads(ssd_policy_t p, const float* features, const float* h_in, const float* c_in, float* h_out, float* c_out, float* logits,
                           float* value, int8_t* actions, int64_t num_agents, uint64_t seed, uint32_t counter, void* stream) {
-    return ssd::policy_head::heads<false>(p, features, h_in, c_in, h_out, c_out, logits, value, 0, actions, nullptr, nullptr, num_agents, seed,
-                                          counter, stream);
+    return ssd::policy_head::heads<false>(p, features, nullptr, h_in, c_in, h_out, c_out, logits, value, 0, actions, nullptr, nullptr, num_agents,
+                                          seed, counter, stream);
 }
 
 int ssd_policy_lstm_heads_dist(ssd_policy_t p, const float* features, const float* h_in, const float* c_in, float* h_out, float* c_out,
                                float* logits, float* value, int mode, int8_t* actions, float* logp, float* entropy, int64_t num_agents,
                                uint64_t seed, uint32_t counter, void* stream) {
-    return ssd::policy_head::heads<true>(p, features, h_in, c_in, h_out, c_out, logits, value, mode, actions, logp, entropy, num_agents, seed,
-                                         counter, stream);
+    return ssd::policy_head::heads<true>(p, features, nullptr, h_in, c_in, h_out, c_out, logits, value, mode, actions, logp, entropy, num_agents,
+                                         seed, counter, stream);
 }
 
 int ssd_policy_pool_lstm_heads(ssd_policy_t p, const float* features, const uint8_t* policy_ids, const float* h_in, const float* c_in, float* h_out,
                                float* c_out, float* logits, float* value, int8_t* actions, int64_t num_agents, uint64_t seed, uint32_t counter,
                                void* stream) {
-    return ssd::policy_head::pool_heads<false>(p, features, policy_ids, h_in, c_in, h_out, c_out, logits, value, 0, actions, nullptr, nullptr,
-                                               num_agents, seed, counter, stream);
+    if (!policy_ids) return ssd::set_error(SSD_ERR_INVALID, "bad argument");
+    return ssd::policy_head::heads<false>(p, features, policy_ids, h_in, c_in, h_out, c_out, logits, value, 0, actions, nullptr, nullptr,
+                                          num_agents, seed, counter, stream);
 }
 
 int ssd_policy_pool_lstm_heads_dist(ssd_policy_t p, const float* features, const uint8_t* policy_ids, const float* h_in, const float* c_in,
                                     float* h_out, float* c_out, float* logits, float* value, int mode, int8_t* actions, float* logp,
                                     float* entropy, int64_t num_agents, uint64_t seed, uint32_t counter, void* stream) {
-    return ssd::policy_head::pool_heads<true>(p, features, policy_ids, h_in, c_in, h_out, c_out, logits, value, mode, actions, logp, entropy,
-                                              num_agents, seed, counter, stream);
+    if (!policy_ids) return ssd::set_error(SSD_ERR_INVALID, "bad argument");
+    return ssd::policy_head::heads<true>(p, features, policy_ids, h_in, c_in, h_out, c_out, logits, value, mode, actions, logp, entropy, num_agents,
+                                         seed, counter, stream);
 }
 
 }  // extern "C"

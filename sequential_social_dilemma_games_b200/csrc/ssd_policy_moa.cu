@@ -20,29 +20,22 @@
 // Threads: pass 0 as the head's drain (thread = agent, warps 0-3 / 4-7 take units 0-63 / 64-127); pass 1 thread = agent and
 // half of the own actions (warps 0-3 take a' = 0, 2, ..., warps 4-7 a' = 1, 3, ...), each thread owning all 128 units of its
 // agent for its a'.  The counterfactual at the actual action writes pred and (h', c').  An own action outside 0..A-1 runs one
-// more drain with no own row for pred / h' / c'.  Recurrent state: the library's tiled layout (ssd_policy_head.cu).
-#include <cuda_fp16.h>
-
+// more drain with no own row for pred / h' / c'.  Gate operand, gate GEMM and recurrent state: ssd_policy_lstm.cuh.
 #include <cmath>
 #include <new>
 #include <vector>
 
-#include "ssd_internal.h"
-#include "ssd_policy.h"
-#include "ssd_umma.cuh"
+#include "ssd_policy_lstm.cuh"
 
 namespace ssd {
 namespace moa {
-using namespace ssd::umma;
+using namespace ssd::lstm;
 
-constexpr int GA = 128, U = 128, KX = 32, K = KX + U, NG = 4 * U, NJ = 64, AMAX = 15;
-constexpr int kThreads = 256;
-constexpr int kBBytes = (K / 8) * NG * 16;             // 163 840: [Wx; U] K-major, as the policy head
+constexpr int NJ = 64, AMAX = 15;
 constexpr int kConstFloats = NG + NJ;                  // gate bias, moa_logits_b
 constexpr int kBlobBytes = kBBytes + kConstFloats * 4;  // 166 144
 constexpr int kOffB = 0, kOffConst = kBBytes;
 constexpr int kOffS = (kBlobBytes + 127) & ~127;       // A operand [128 x 160] fp16, then the scratch [NJ / 4][256][4] fp32
-constexpr int kABytes = (K / 8) * GA * 16;             // 40 960
 constexpr int kSBytes = NJ * kThreads * 4;             // 65 536
 constexpr int kOffBar = kOffS + kSBytes;
 constexpr int kSmemBytes = kOffBar + 16;
@@ -52,39 +45,23 @@ static_assert(kABytes <= kSBytes && kBlobBytes % 16 == 0 && kSmemBytes <= 227 * 
 // then moa_logits_w [128][NJ] zero padded
 inline long long rows_floats(int n, int a) { return static_cast<long long>(n) * a * NG + U * NJ; }
 
-__device__ __forceinline__ uint32_t pack_h2(float lo, float hi) {
-    const __half2 v = __floats2half2_rn(lo, hi);
-    return *reinterpret_cast<const uint32_t*>(&v);
-}
-__device__ __forceinline__ float tanh_fast(float x) {  // as the policy head: MUFU tanh, below the fp16 rounding of the GEMM operands
-    float y;
-    asm("tanh.approx.f32 %0, %1;" : "=f"(y) : "f"(x));
-    return y;
-}
-__device__ __forceinline__ float sigmoid_fast(float x) { return fmaf(tanh_fast(0.5f * x), 0.5f, 0.5f); }
-
-// kMap Shared: agent m = a0 + row, own index i = m % N.  PerAgent (P = N): CTA c serves weight set c % N, agents (b, c % N) of
-// groups c / N, c / N + cpp, ..., and its state group is p * ceil(B / 128) + g, exactly as the policy head.
+// kMap Shared: agent m = a0 + row, own index i = m % N.  PerAgent (P = N): the groups of GroupMap (ssd_policy.h), as the
+// policy head.
 template <WeightMap kMap>
 __global__ void __launch_bounds__(kThreads, 1)
 moa_kernel(const float* __restrict__ feat, const int8_t* __restrict__ joint, const float* __restrict__ pol_logits, const float* h_in,
            const float* c_in, float* h_out, float* c_out, float* pred, float* __restrict__ cf, float* __restrict__ ipa, float* __restrict__ infl,
            long long M, int N, int A, const uint8_t* __restrict__ blob, const float* __restrict__ rows, long long rows_stride, int divergence,
            float clip, int ctas_per_policy) {
-    constexpr bool kPerAgent = kMap == WeightMap::PerAgent;
     extern __shared__ __align__(128) uint8_t smem[];
     __shared__ uint32_t s_tmem;
     const int tid = threadIdx.x, warp = tid >> 5;
     uint64_t* bar = reinterpret_cast<uint64_t*>(smem + kOffBar);
     const float* s_bias = reinterpret_cast<const float*>(smem + kOffConst);
     float* ys = reinterpret_cast<float*>(smem + kOffS);   // scratch: column j of thread t at ((j / 4) * kThreads + t) * 4 + j % 4
-    const int np = kPerAgent ? N : 1;
-    const int pol = kPerAgent ? static_cast<int>(blockIdx.x) % np : 0;
-    const long long cta = kPerAgent ? blockIdx.x / np : blockIdx.x;
-    const long long stride = kPerAgent ? ctas_per_policy : gridDim.x;
-    const long long nrows = kPerAgent ? M / np : M;
-    blob += static_cast<long long>(pol) * kBlobBytes;
-    rows += pol * rows_stride;
+    const GroupMap<kMap> gm(M, N, ctas_per_policy);
+    blob += static_cast<long long>(gm.pol) * kBlobBytes;
+    rows += gm.pol * rows_stride;
     const float* wl = rows + static_cast<long long>(N) * A * NG;   // moa_logits_w [128][NJ]
     const int nc = (N - 1) * A;
     if (tid == 0) mbar_init(bar, 1);
@@ -96,14 +73,13 @@ moa_kernel(const float* __restrict__ feat, const int8_t* __restrict__ joint, con
     tc_fence_after();
     const uint32_t tmem = s_tmem;
     const uint32_t sA = smem_u32(smem + kOffS), sB = smem_u32(smem + kOffB);
-    constexpr uint32_t kIG = umma_idesc(GA, 256);
     uint32_t parity = 0;
 
-    const long long n_groups = (nrows + GA - 1) / GA;
-    for (long long g = cta; g < n_groups; g += stride) {
-        const long long a0 = g * GA, sg = pol * n_groups + g;
-        const int rem = static_cast<int>(nrows - a0 < GA ? nrows - a0 : GA);
-        {   // A = fp16([features | h]), as the policy head
+    for (long long g = gm.cta; g < gm.n_groups; g += gm.stride) {
+        const long long a0 = g * GA, sg = gm.state_group(g);
+        const int rem = static_cast<int>(gm.rows - a0 < GA ? gm.rows - a0 : GA);
+        {   // A = fp16([features | h]), as the policy head.  Built here rather than by the head's builder: with that builder this
+            // kernel's register allocation and instruction order changed and it measured 0.5 % slower.
             const int seg = tid & 7, r8 = tid >> 3;
             const int hrow = tid & (GA - 1), hb0 = (tid >> 7) * 4;
             const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -111,7 +87,7 @@ moa_kernel(const float* __restrict__ feat, const int8_t* __restrict__ joint, con
 #pragma unroll
             for (int ps = 0; ps < 4; ++ps) {
                 const int row = ps * 32 + r8;
-                vx[ps] = row < rem ? __ldcs(reinterpret_cast<const float4*>(feat + ((a0 + row) * np + pol) * KX) + seg) : z;
+                vx[ps] = row < rem ? __ldcs(reinterpret_cast<const float4*>(feat + gm.agent(a0, row) * KX) + seg) : z;
             }
 #pragma unroll
             for (int b = 0; b < 4; ++b) {
@@ -134,16 +110,7 @@ moa_kernel(const float* __restrict__ feat, const int8_t* __restrict__ joint, con
         fence_async_smem();
         tc_fence_before();
         __syncthreads();
-        if (warp == 0 && elect_one()) {
-            tc_fence_after();
-#pragma unroll
-            for (int ks = 0; ks < K / 16; ++ks)
-#pragma unroll
-                for (int half = 0; half < 2; ++half)
-                    umma_f16(tmem + half * 256, umma_desc(sA + ks * 2 * GA * 16, GA * 16, 128),
-                             umma_desc(sB + half * 256 * 16 + ks * 2 * NG * 16, NG * 16, 128), kIG, ks > 0);
-            umma_commit(bar);
-        }
+        if (warp == 0 && elect_one()) gate_gemm(tmem, sA, sB, bar);
         mbar_wait(bar, parity);
         parity ^= 1;
         tc_fence_after();
@@ -152,7 +119,7 @@ moa_kernel(const float* __restrict__ feat, const int8_t* __restrict__ joint, con
         const int r = tid & (GA - 1), half = warp >> 2;
         const uint32_t trow = tmem + (static_cast<uint32_t>((warp & 3) * 32) << 16);
         const bool live = r < rem;
-        const long long m = (a0 + r) * np + pol, b = m / N;
+        const long long m = gm.agent(a0, r), b = m / N;
         const int i = static_cast<int>(m - b * N);
         const int8_t* ja = joint + b * N;
         const int own = live ? ja[i] : 0;
@@ -344,6 +311,8 @@ moa_kernel(const float* __restrict__ feat, const int8_t* __restrict__ joint, con
     if (warp == 0) tmem_free(tmem, 512);
 }
 
+inline auto moa_kernel_for(WeightMap m) { return m == WeightMap::Shared ? moa_kernel<WeightMap::Shared> : moa_kernel<WeightMap::PerAgent>; }
+
 }  // namespace moa
 }  // namespace ssd
 
@@ -365,20 +334,13 @@ int ssd_moa_create(int device, int num_policies, int num_agents, int num_actions
     const long long rf = rows_floats(n, na);
     std::vector<uint8_t> blobs(static_cast<size_t>(num_policies) * kBlobBytes, 0);
     std::vector<float> rows(static_cast<size_t>(num_policies * rf), 0.f);
-    auto at = [](int nrow, int col, int k) { return ((k >> 3) * nrow + col) * 8 + (k & 7); };  // canonical K-major, no swizzle
     for (int q = 0; q < num_policies; ++q) {   // weight set q: arrays q of the num_policies consecutive ones behind each pointer
         const float* lw = lstm_w + static_cast<size_t>(q) * kin * NG;
-        const float* lu = lstm_u + static_cast<size_t>(q) * U * NG;
-        const float* lb = lstm_b + q * NG;
         const float* ow = logits_w + static_cast<size_t>(q) * U * nc;
         const float* ob = logits_b + q * nc;
-        __half* bw = reinterpret_cast<__half*>(blobs.data() + static_cast<size_t>(q) * kBlobBytes + kOffB);
         float* cst = reinterpret_cast<float*>(blobs.data() + static_cast<size_t>(q) * kBlobBytes + kOffConst);
-        for (int col = 0; col < NG; ++col) {
-            for (int k = 0; k < KX; ++k) bw[at(NG, col, k)] = __float2half_rn(lw[k * NG + col]);
-            for (int k = 0; k < U; ++k) bw[at(NG, col, KX + k)] = __float2half_rn(lu[k * NG + col]);
-            cst[col] = lb[col];
-        }
+        pack_gates(reinterpret_cast<__half*>(blobs.data() + static_cast<size_t>(q) * kBlobBytes + kOffB), cst, lw, lstm_u + static_cast<size_t>(q) * U * NG,
+                   lstm_b + q * NG);   // the features' rows of moa_lstm_w (its first 32) and moa_lstm_u
         for (int j = 0; j < nc; ++j) cst[NG + j] = ob[j];
         float* rq = rows.data() + q * rf;
         for (size_t e = 0; e < static_cast<size_t>(n) * na * NG; ++e) rq[e] = lw[KX * NG + e];   // rows 32 .. 32 + N A of moa_lstm_w
@@ -389,7 +351,7 @@ int ssd_moa_create(int device, int num_policies, int num_agents, int num_actions
     if (!p) return ssd::set_error(SSD_ERR_INVALID, "out of host memory");
     p->device = device;
     p->num_policies = num_policies;
-    p->moa = true;
+    p->kind = HandleKind::Moa;
     p->moa_agents = n;
     p->num_outputs = na;
     cudaError_t e = cudaSetDevice(device);
@@ -399,9 +361,7 @@ int ssd_moa_create(int device, int num_policies, int num_agents, int num_actions
     if (e == cudaSuccess) e = cudaMalloc(&p->d_moa_rows, rows.size() * sizeof(float));
     if (e == cudaSuccess) e = cudaMemcpyAsync(p->d_moa_rows, rows.data(), rows.size() * sizeof(float), cudaMemcpyHostToDevice, 0);
     if (e == cudaSuccess) e = cudaStreamSynchronize(0);   // the host staging buffers go out of scope
-    if (e == cudaSuccess)
-        e = cudaFuncSetAttribute(num_policies == 1 ? moa_kernel<WeightMap::Shared> : moa_kernel<WeightMap::PerAgent>,
-                                 cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(moa_kernel_for(ssd::policy::weight_map(p)), cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
     if (e != cudaSuccess) {
         ssd_policy_destroy(p);
         return ssd::set_error(SSD_ERR_CUDA, cudaGetErrorString(e));
@@ -416,38 +376,27 @@ int ssd_moa_step(ssd_moa_t p, const float* features, const int8_t* joint_actions
                  float* h_out, float* c_out, float* pred, float* counterfactual, float* influence_per_agent, float* influence, int64_t num_agents,
                  int divergence, float clip, void* stream) {
     using namespace ssd::moa;
+    using namespace ssd::policy;
     if (!p || !features || !joint_actions || !policy_logits || !h_in || !c_in || !h_out || !c_out || !pred || !influence_per_agent || !influence ||
         num_agents < 0)
         return ssd::set_error(SSD_ERR_INVALID, "bad argument");
-    if (!p->moa) return ssd::set_error(SSD_ERR_INVALID, "not an MOA handle (ssd_moa_create)");
+    int rc = check_kind(p, HandleKind::Moa, "not an MOA handle (ssd_moa_create)");
+    if (rc != SSD_OK) return rc;
     if (divergence != SSD_DIV_KL && divergence != SSD_DIV_JSD) return ssd::set_error(SSD_ERR_INVALID, "divergence must be SSD_DIV_KL or SSD_DIV_JSD");
     if (!(clip >= 0.f)) return ssd::set_error(SSD_ERR_INVALID, "clip must be >= 0 (+inf: no clamp), not NaN");
-    const void* ptrs[5] = {features, h_in, c_in, h_out, c_out};
-    for (const void* q : ptrs)
-        if (reinterpret_cast<uintptr_t>(q) % 16 != 0) return ssd::set_error(SSD_ERR_INVALID, "features and state pointers must be 16-byte aligned");
+    rc = check_aligned({features, h_in, c_in, h_out, c_out}, "features and state pointers must be 16-byte aligned");
+    if (rc != SSD_OK) return rc;
     if (h_out == h_in || c_out == c_in) return ssd::set_error(SSD_ERR_INVALID, "h_out / c_out must not alias h_in / c_in");
-    const int n = p->moa_agents, np = p->num_policies;
+    const int n = p->moa_agents;
     if (num_agents % n != 0) return ssd::set_error(SSD_ERR_INVALID, "num_agents must be a multiple of the MOA's num_agents");
     if (num_agents == 0) return SSD_OK;
-    if (cudaSetDevice(p->device) != cudaSuccess) return ssd::set_error(SSD_ERR_CUDA, "cudaSetDevice failed");
-    const cudaStream_t st = static_cast<cudaStream_t>(stream);
-    const long long rf = rows_floats(n, p->num_outputs);
-    if (np == 1) {
-        const long long groups = (num_agents + GA - 1) / GA;
-        const int grid = static_cast<int>(groups < p->sms ? groups : p->sms);
-        moa_kernel<WeightMap::Shared><<<grid, kThreads, kSmemBytes, st>>>(features, joint_actions, policy_logits, h_in, c_in, h_out, c_out, pred,
-                                                                         counterfactual, influence_per_agent, influence, num_agents, n,
-                                                                         p->num_outputs, p->d_head_blob, p->d_moa_rows, rf, divergence, clip, grid);
-    } else {   // N * floor(#SMs / N) CTAs at most, each serving one weight set
-        const long long groups = (num_agents / np + GA - 1) / GA;
-        const int per = static_cast<int>(groups < p->sms / np ? groups : p->sms / np);
-        moa_kernel<WeightMap::PerAgent><<<np * per, kThreads, kSmemBytes, st>>>(features, joint_actions, policy_logits, h_in, c_in, h_out, c_out,
-                                                                               pred, counterfactual, influence_per_agent, influence, num_agents, n,
-                                                                               p->num_outputs, p->d_head_blob, p->d_moa_rows, rf, divergence, clip, per);
-    }
-    const cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return ssd::set_error(SSD_ERR_CUDA, cudaGetErrorString(e));
-    return SSD_OK;
+    rc = setup(p, nullptr, num_agents, stream);
+    if (rc != SSD_OK) return rc;
+    const Grid g = grid(p, num_agents);
+    moa_kernel_for(weight_map(p))<<<g.ctas, kThreads, kSmemBytes, static_cast<cudaStream_t>(stream)>>>(
+        features, joint_actions, policy_logits, h_in, c_in, h_out, c_out, pred, counterfactual, influence_per_agent, influence, num_agents, n,
+        p->num_outputs, p->d_head_blob, p->d_moa_rows, rows_floats(n, p->num_outputs), divergence, clip, g.ctas_per_policy);
+    return launched();
 }
 
 }  // extern "C"

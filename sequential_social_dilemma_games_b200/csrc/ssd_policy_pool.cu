@@ -20,8 +20,6 @@ namespace ssd {
 namespace policy_pool {
 
 constexpr int kThreads = 256, kPerThread = 16, kChunk = kThreads * kPerThread;   // agents per CTA of count / scatter
-constexpr int kBins = 256;                                                        // u8 ids
-constexpr int kOffCursor = kBins, kOffNumTiles = 2 * kBins, kCountWords = 2 * kBins + 1;
 constexpr int kGA = 128;                                                          // agents per tile (UMMA M)
 
 // Histogram of the chunk's ids < K into h[kBins] (zeroed by the caller).  Every lane of every warp runs the same iterations.
@@ -125,9 +123,7 @@ int assign(SsdPolicy* p, const uint8_t* policy_ids, long long M, void* stream) {
     pool_count_kernel<<<chunks, kThreads, 0, st>>>(policy_ids, M, K, p->d_counts);
     pool_plan_kernel<<<1, kBins, 0, st>>>(K, p->d_counts, p->d_tiles);
     pool_scatter_kernel<<<chunks, kThreads, 0, st>>>(policy_ids, M, K, p->d_counts + kOffCursor, p->d_perm);
-    e = cudaGetLastError();
-    if (e != cudaSuccess) return ssd::set_error(SSD_ERR_CUDA, cudaGetErrorString(e));
-    return SSD_OK;
+    return ssd::policy::launched();
 }
 
 }  // namespace policy_pool

@@ -170,7 +170,67 @@ def _state_from_rows(rows, P):
     return full.reshape(P * g, 128, u // 16, 16).permute(0, 2, 1, 3).contiguous()
 
 
-class ConvToFCNet(object):
+class _Handle(object):
+    """A library handle on self.device: its lifetime and the stream its calls are ordered on."""
+    _destroy = "ssd_policy_destroy"
+
+    def close(self):
+        if self._h:
+            getattr(_lib.lib, self._destroy)(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def _stream(self):
+        return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+
+
+class _Policy(_Handle):
+    """What ConvToFCNet and PolicyPool share: the Philox key of the fused sampler and the calls of the fused head."""
+    _sample_seed, _sample_counter = 0, 0
+
+    def seed_sampling(self, seed):
+        """Key of the Philox streams `act` samples from (counter = number of `act` and sampling `policy_step` calls since)."""
+        self._sample_seed, self._sample_counter = int(seed) & (2 ** 64 - 1), 0
+
+    def _heads(self, obs, ids, h, c, code=None, given=None, dist=False):
+        """-> PolicyStep of the fused head on the features of obs (ids: the pool's policy ids as `_ids` returns them, None for a
+        network).  dist False: ssd_policy_[pool_]lstm_heads, which samples the actions when code is ACT_SAMPLE and takes none
+        otherwise (logp and entropy None); dist True: ssd_policy_[pool_]lstm_heads_dist in mode `code`, on the `given` actions
+        for ACT_GIVEN.  A sampling call advances the Philox counter."""
+        x = self.features(obs) if ids is None else self.features(obs, ids)
+        m = x.shape[0]
+        self._check_state(h, c, m)
+        h, c = _aligned(h), _aligned(c)
+        h_new, c_new = torch.empty_like(h), torch.empty_like(c)
+        logits = torch.empty((m, self.num_outputs), dtype=torch.float32, device=self.device)
+        value = torch.empty((m,), dtype=torch.float32, device=self.device)
+        a = logp = entropy = None
+        if given is not None:
+            a = given
+        elif dist or code == _lib.ACT_SAMPLE:   # a pool's skipped agents keep -1
+            a = torch.empty((m,), dtype=torch.int8, device=self.device) if ids is None else torch.full((m,), -1, dtype=torch.int8, device=self.device)
+        p = lambda t: C.c_void_p(t.data_ptr() if t is not None else None)
+        lead = (self._h, p(x)) if ids is None else (self._h, p(x), p(ids))
+        state = (p(h), p(c), p(h_new), p(c_new), p(logits), p(value))
+        key = (m, self._sample_seed, self._sample_counter & 0xFFFFFFFF, self._stream())
+        if dist:
+            logp, entropy = torch.empty_like(value), torch.empty_like(value)
+            fn = _lib.lib.ssd_policy_lstm_heads_dist if ids is None else _lib.lib.ssd_policy_pool_lstm_heads_dist
+            _lib.check(fn(*lead, *state, code, p(a), p(logp), p(entropy), *key))
+        else:
+            fn = _lib.lib.ssd_policy_lstm_heads if ids is None else _lib.lib.ssd_policy_pool_lstm_heads
+            _lib.check(fn(*lead, *state, p(a), *key))
+        if code == _lib.ACT_SAMPLE:
+            self._sample_counter += 1
+        return PolicyStep(a, logp, entropy, logits, value, h_new, c_new)
+
+
+class ConvToFCNet(_Policy):
     """Forward pass of ConvToFCNetv2 for a batch of agents; `obs` is the uint8 tensor of the step path.
 
     `weights` is one dict (one network shared by all agents) or a list of P dicts, weights[p] being the policy of 'agent-p':
@@ -197,7 +257,6 @@ class ConvToFCNet(object):
                                                 ptr(w["fc1_b"]), ptr(w["fc2_w"]), ptr(w["fc2_b"]), C.byref(self._h)))
         self._head = {}
         self._fused_head = False
-        self._sample_seed, self._sample_counter = 0, 0
         if fused:
             _lib.check(_lib.lib.ssd_policy_set_head_n(self._h, P, self.cell_size, self.num_outputs, ptr(w["lstm_w"]), ptr(w["lstm_u"]),
                                                       ptr(w["lstm_b"]), ptr(w["logits_w"]), ptr(w["logits_b"]), ptr(w["value_w"]),
@@ -210,17 +269,6 @@ class ConvToFCNet(object):
             self._head = {"lstm_w": dev("lstm_w", torch.bfloat16), "lstm_u": dev("lstm_u", torch.bfloat16), "lstm_b": dev("lstm_b", torch.float32),
                           "logits_w": dev("logits_w", torch.bfloat16), "logits_b": dev("logits_b", torch.float32),
                           "value_w": dev("value_w", torch.bfloat16), "value_b": dev("value_b", torch.float32)}
-
-    def close(self):
-        if self._h:
-            _lib.lib.ssd_policy_destroy(self._h)
-            self._h = C.c_void_p()
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
 
     def _groups(self, m):
         """Number of 128-agent state groups of m agents: P * ceil(m / P / 128)."""
@@ -242,8 +290,7 @@ class ConvToFCNet(object):
         m = obs.numel() // (OBS_SIDE * OBS_SIDE * 3)
         if out is None:
             out = torch.empty((m, FEATURES), dtype=torch.float32, device=self.device)
-        stream = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
-        _lib.check(_lib.lib.ssd_policy_features(self._h, C.c_void_p(obs.data_ptr()), m, C.c_void_p(out.data_ptr()), stream))
+        _lib.check(_lib.lib.ssd_policy_features(self._h, C.c_void_p(obs.data_ptr()), m, C.c_void_p(out.data_ptr()), self._stream()))
         return out
 
     def initial_state(self, m):
@@ -264,32 +311,14 @@ class ConvToFCNet(object):
         self._groups(rows.shape[0])
         return _state_from_rows(rows, self.num_policies)
 
-    def seed_sampling(self, seed):
-        """Key of the Philox streams `act` samples from (counter = number of `act` and sampling `policy_step` calls since)."""
-        self._sample_seed, self._sample_counter = int(seed) & (2 ** 64 - 1), 0
-
-    def _head_io(self, obs, h, c):
-        """Features of obs, the checked (h, c) and fresh output buffers (h', c', logits, value) of the fused head."""
-        x = self.features(obs)
-        m = x.shape[0]
+    def _check_state(self, h, c, m):
         if h.dim() != 4 or (h.shape[0] * 128 < m if self.num_policies == 1 else h.shape[0] != self._groups(m)):
             raise ValueError("the fused route carries (h, c) in the tiled layout of initial_state / state_from_rows")
-        h, c = _aligned(h), _aligned(c)
-        logits = torch.empty((m, self.num_outputs), dtype=torch.float32, device=self.device)
-        value = torch.empty((m,), dtype=torch.float32, device=self.device)
-        return x, h, c, (torch.empty_like(h), torch.empty_like(c), logits, value)
 
     def _fused(self, obs, h, c, sample):
-        x, h, c, (h_new, c_new, logits, value) = self._head_io(obs, h, c)
-        m = x.shape[0]
-        actions = torch.empty((m,), dtype=torch.int8, device=self.device) if sample else None
-        stream = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
-        p = lambda t: C.c_void_p(t.data_ptr() if t is not None else None)
-        _lib.check(_lib.lib.ssd_policy_lstm_heads(self._h, p(x), p(h), p(c), p(h_new), p(c_new), p(logits), p(value), p(actions), m,
-                                                  self._sample_seed, self._sample_counter & 0xFFFFFFFF, stream))
-        if sample:
-            self._sample_counter += 1
-        return logits, value, h_new, c_new, actions
+        """-> (logits, value, h', c', actions) of ssd_policy_lstm_heads; actions None unless `sample`."""
+        s = self._heads(obs, None, h, c, _lib.ACT_SAMPLE if sample else None)
+        return s.logits, s.value, s.h, s.c, s.actions
 
     def forward(self, obs, h, c):
         """-> (logits [M, A], value [M], h', c'), all float32; (h, c) in the layout of `initial_state`."""
@@ -309,9 +338,8 @@ class ConvToFCNet(object):
         m, u = h.shape
         c_new, h_new = torch.empty_like(c), torch.empty_like(h)
         h16 = torch.empty((m, u), dtype=torch.bfloat16, device=self.device)
-        stream = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
         p = lambda t: C.c_void_p(t.data_ptr())
-        _lib.check(_lib.lib.ssd_policy_lstm_cell(p(gates), p(hd["lstm_b"]), p(_aligned(c)), p(c_new), p(h_new), p(h16), m, u, stream))
+        _lib.check(_lib.lib.ssd_policy_lstm_cell(p(gates), p(hd["lstm_b"]), p(_aligned(c)), p(c_new), p(h_new), p(h16), m, u, self._stream()))
         logits = torch.mm(h16, hd["logits_w"]).float() + hd["logits_b"]
         value = (torch.mm(h16, hd["value_w"]).float() + hd["value_b"]).squeeze(1)
         return logits, value, h_new, c_new
@@ -339,19 +367,10 @@ class ConvToFCNet(object):
         code, given = _step_mode(mode, actions, m, self.num_outputs, self.device)
         if not self._fused_head or (code == _lib.ACT_SAMPLE and generator is not None):
             return _torch_step(*self.forward(obs, h, c), code, given, generator)
-        x, h, c, (h_new, c_new, logits, value) = self._head_io(obs, h, c)
-        a = given if given is not None else torch.empty((m,), dtype=torch.int8, device=self.device)
-        logp, entropy = torch.empty_like(value), torch.empty_like(value)
-        stream = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
-        p = lambda t: C.c_void_p(t.data_ptr())
-        _lib.check(_lib.lib.ssd_policy_lstm_heads_dist(self._h, p(x), p(h), p(c), p(h_new), p(c_new), p(logits), p(value), code, p(a), p(logp),
-                                                       p(entropy), m, self._sample_seed, self._sample_counter & 0xFFFFFFFF, stream))
-        if code == _lib.ACT_SAMPLE:
-            self._sample_counter += 1
-        return PolicyStep(a, logp, entropy, logits, value, h_new, c_new)
+        return self._heads(obs, None, h, c, code, given, dist=True)
 
 
-class PolicyPool(object):
+class PolicyPool(_Policy):
     """K weight sets (1 <= K <= 255, each a dict as for ConvToFCNet) loaded once; every call takes `policy_ids`, a uint8 tensor
     on the device of shape obs.shape[:-3]: agent m is evaluated with weight_sets[policy_ids[m]], and the ids may differ from
     call to call.  An id >= K means "no pool policy": nothing is written for that agent (its rows of features, logits, value,
@@ -377,18 +396,6 @@ class PolicyPool(object):
         self._h = C.c_void_p()
         _lib.check(_lib.lib.ssd_policy_create_pool(VIEW_RADIUS, self.device.index, self.num_policies, self.cell_size, self.num_outputs,
                                                    *[ptr(w[k]) for k in names], C.byref(self._h)))
-        self._sample_seed, self._sample_counter = 0, 0
-
-    def close(self):
-        if self._h:
-            _lib.lib.ssd_policy_destroy(self._h)
-            self._h = C.c_void_p()
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
 
     def _ids(self, obs, policy_ids):
         if obs.dtype != torch.uint8 or obs.device != self.device or obs.dim() < 4 or tuple(obs.shape[-3:]) != (OBS_SIDE, OBS_SIDE, 3):
@@ -404,9 +411,8 @@ class PolicyPool(object):
         m = ids.numel()
         if out is None:
             out = torch.empty((m, FEATURES), dtype=torch.float32, device=self.device)
-        stream = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
         _lib.check(_lib.lib.ssd_policy_pool_features(self._h, C.c_void_p(obs.data_ptr()), C.c_void_p(ids.data_ptr()), m,
-                                                     C.c_void_p(out.data_ptr()), stream))
+                                                     C.c_void_p(out.data_ptr()), self._stream()))
         return out
 
     def initial_state(self, m):
@@ -422,34 +428,14 @@ class PolicyPool(object):
         """Agent-major [m, 128] -> tiled state [ceil(m/128), 8, 128, 16], zero padded."""
         return _state_from_rows(rows, 1)
 
-    def seed_sampling(self, seed):
-        """Key of the Philox streams `act` samples from (counter = number of `act` and sampling `policy_step` calls since)."""
-        self._sample_seed, self._sample_counter = int(seed) & (2 ** 64 - 1), 0
-
-    def _head_io(self, obs, ids, h, c):
-        """Features of obs (obs and ids as `_ids` returns them), the checked (h, c) and fresh output buffers (h', c', logits,
-        value) of the head."""
-        x = self.features(obs, ids)
-        m = x.shape[0]
+    def _check_state(self, h, c, m):
         if h.dim() != 4 or h.shape[0] * 128 < m or h.shape != c.shape:
             raise ValueError("(h, c) must be in the tiled layout of initial_state / state_from_rows")
-        h, c = _aligned(h), _aligned(c)
-        logits = torch.empty((m, self.num_outputs), dtype=torch.float32, device=self.device)
-        value = torch.empty((m,), dtype=torch.float32, device=self.device)
-        return x, h, c, (torch.empty_like(h), torch.empty_like(c), logits, value)
 
     def _run(self, obs, policy_ids, h, c, sample):
-        obs, ids = self._ids(obs, policy_ids)
-        x, h, c, (h_new, c_new, logits, value) = self._head_io(obs, ids, h, c)
-        m = x.shape[0]
-        actions = torch.full((m,), -1, dtype=torch.int8, device=self.device) if sample else None
-        stream = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
-        p = lambda t: C.c_void_p(t.data_ptr() if t is not None else None)
-        _lib.check(_lib.lib.ssd_policy_pool_lstm_heads(self._h, p(x), p(ids), p(h), p(c), p(h_new), p(c_new), p(logits), p(value), p(actions),
-                                                       m, self._sample_seed, self._sample_counter & 0xFFFFFFFF, stream))
-        if sample:
-            self._sample_counter += 1
-        return logits, value, h_new, c_new, actions
+        """-> (logits, value, h', c', actions) of ssd_policy_pool_lstm_heads; actions None unless `sample`."""
+        s = self._heads(*self._ids(obs, policy_ids), h, c, _lib.ACT_SAMPLE if sample else None)
+        return s.logits, s.value, s.h, s.c, s.actions
 
     def forward(self, obs, policy_ids, h, c):
         """-> (logits [M, A], value [M], h', c'), all float32; rows of skipped agents are not written."""
@@ -466,19 +452,8 @@ class PolicyPool(object):
         scores the caller's `actions` (returned as int8).  Skipped agents (id >= K) get action -1 in 'sample' and 'greedy'; their
         rows of logp and entropy, like those of logits, value, h' and c', are not written."""
         obs, ids = self._ids(obs, policy_ids)
-        m = ids.numel()
-        code, given = _step_mode(mode, actions, m, self.num_outputs, self.device)
-        x, h, c, (h_new, c_new, logits, value) = self._head_io(obs, ids, h, c)
-        a = given if given is not None else torch.full((m,), -1, dtype=torch.int8, device=self.device)
-        logp, entropy = torch.empty_like(value), torch.empty_like(value)
-        stream = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
-        p = lambda t: C.c_void_p(t.data_ptr())
-        _lib.check(_lib.lib.ssd_policy_pool_lstm_heads_dist(self._h, p(x), p(ids), p(h), p(c), p(h_new), p(c_new), p(logits), p(value), code,
-                                                            p(a), p(logp), p(entropy), m, self._sample_seed, self._sample_counter & 0xFFFFFFFF,
-                                                            stream))
-        if code == _lib.ACT_SAMPLE:
-            self._sample_counter += 1
-        return PolicyStep(a, logp, entropy, logits, value, h_new, c_new)
+        code, given = _step_mode(mode, actions, ids.numel(), self.num_outputs, self.device)
+        return self._heads(obs, ids, h, c, code, given, dist=True)
 
 
 MOAStep = collections.namedtuple("MOAStep", "pred influence influence_per_agent h c counterfactual")
@@ -499,7 +474,7 @@ def random_moa_weights(num_agents, num_actions, seed=0, cell_size=128):
             "moa_logits_w": glorot((u, n_out)), "moa_logits_b": (0.1 * rng.randn(n_out)).astype(np.float32)}
 
 
-class MOANet(object):
+class MOANet(_Handle):
     """Model of other agents of the causal-influence models (models/moa_model.py MOA_LSTM) and the social-influence reward
     (common_funcs.py compute_influence_reward), forward only, in one fused kernel (`ssd_moa_step`).
 
@@ -508,6 +483,7 @@ class MOANet(object):
     N dicts (agent i uses weights[i], as ConvToFCNet([w_0, ..., w_{N-1}])), with keys moa_lstm_w [32 + N A, 512], moa_lstm_u
     [128, 512], moa_lstm_b [512], moa_logits_w [128, (N-1) A], moa_logits_b [(N-1) A].  The recurrent state has the tiled layout
     of ConvToFCNet (grouped per weight set for a list of N)."""
+    _destroy = "ssd_moa_destroy"
 
     def __init__(self, weights, num_agents, device="cuda:0"):
         self.device = _cuda_device(device)
@@ -535,17 +511,6 @@ class MOANet(object):
         self._h = C.c_void_p()
         _lib.check(_lib.lib.ssd_moa_create(self.device.index, P, n, A, ptr(w["moa_lstm_w"]), ptr(w["moa_lstm_u"]), ptr(w["moa_lstm_b"]),
                                            ptr(w["moa_logits_w"]), ptr(w["moa_logits_b"]), C.byref(self._h)))
-
-    def close(self):
-        if self._h:
-            _lib.lib.ssd_moa_destroy(self._h)
-            self._h = C.c_void_p()
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
 
     def _groups(self, m):
         n, P = self.num_agents, self.num_policies
@@ -598,8 +563,7 @@ class MOANet(object):
         cf = torch.empty((m, A, n - 1, A), dtype=torch.float32, device=self.device) if counterfactuals else None
         ipa = torch.empty((m, n - 1), dtype=torch.float32, device=self.device)
         infl = torch.empty((m,), dtype=torch.float32, device=self.device)
-        stream = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
         p = lambda t: C.c_void_p(t.data_ptr() if t is not None else None)
         _lib.check(_lib.lib.ssd_moa_step(self._h, p(x), p(given), p(pl), p(h), p(c), p(h_new), p(c_new), p(pred), p(cf), p(ipa), p(infl), m,
-                                         _DIVERGENCES[divergence], clip, stream))
+                                         _DIVERGENCES[divergence], clip, self._stream()))
         return MOAStep(pred, infl, ipa, h_new, c_new, cf)
