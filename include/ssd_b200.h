@@ -315,6 +315,30 @@ void ssd_moa_destroy(ssd_moa_t p);
 int ssd_moa_step(ssd_moa_t p, const float* features, const int8_t* joint_actions, const float* policy_logits, const float* h_in, const float* c_in,
                  float* h_out, float* c_out, float* pred, float* counterfactual, float* influence_per_agent, float* influence, int64_t num_agents,
                  int divergence, float clip, void* stream);
+/* An MOA pool: num_policies = K MOA weight sets, 1..255, loaded once; every call takes a device u8 policy id per agent, as a policy
+ * pool does (typically the same ids as the ssd_policy_pool_lstm_heads call of that step: K seeds of an MOA experiment, cross-play
+ * teams).  ssd_moa_create_pool packs the weights exactly as ssd_moa_create, every pointer pointing to K consecutive arrays; the
+ * N / A / (N-1)*A limits are the same; K outside 1..255 or a null pointer returns SSD_ERR_INVALID and allocates nothing.
+ * ssd_moa_pool_step takes the arguments of ssd_moa_step plus policy_ids dev u8[num_agents], agent-major like joint_actions:
+ * agent m is evaluated with weight set policy_ids[m].
+ *   - An id >= K means "no MOA for this agent": nothing is written for it -- none of its rows of pred, counterfactual,
+ *     influence_per_agent, influence, h_out or c_out -- and its row of policy_logits is not read.  Its action still enters the
+ *     other agents' inputs as one of theirs, and an action of it outside 0..A-1 still makes influence NaN for every agent of its
+ *     env (a scripted agent next to pool agents).
+ *   - The recurrent state is in the TILED layout of the shared network, [ceil(M/128)][8][128][16] (element (agent m, unit u) at
+ *     ((m / 128 * 8 + u / 16) * 128 + m % 128) * 16 + u % 16), independent of the ids, so they may change between two steps of
+ *     a live state.
+ *   - Everything else is ssd_moa_step's: M a multiple of N, alignment, no aliasing, counterfactual optional, divergence and
+ *     clip, M = 0 a no-op.  At most 2^31 - 1 agents per call.
+ * Each call first groups the agents by id on the device (no host synchronisation) into scratch that belongs to the handle and
+ * grows on demand, so calls on one MOA pool handle must be ordered (one stream).  ssd_moa_step rejects an MOA pool handle,
+ * ssd_moa_pool_step every other handle, and the policy entry points reject it (SSD_ERR_INVALID).  Destroy with
+ * ssd_moa_destroy. */
+int ssd_moa_create_pool(int device, int num_policies, int num_agents, int num_actions, const float* lstm_w, const float* lstm_u,
+                        const float* lstm_b, const float* logits_w, const float* logits_b, ssd_moa_t* out);
+int ssd_moa_pool_step(ssd_moa_t p, const float* features, const uint8_t* policy_ids, const int8_t* joint_actions, const float* policy_logits,
+                      const float* h_in, const float* c_in, float* h_out, float* c_out, float* pred, float* counterfactual, float* influence_per_agent,
+                      float* influence, int64_t num_agents, int divergence, float clip, void* stream);
 /* The unfused alternative for other cell sizes: LSTM cell update after the gate GEMM (conv_to_fcnet_v2.py:68-80; Keras gate order i, f, c~, o; sigmoid recurrent
  * activation): gates dev bf16[num_agents][4*units] = x W + h U without the bias, bias dev f32[4*units],
  * c_prev / c_out / h_out dev f32[num_agents][units] (c_out may alias c_prev), h_bf16_out dev bf16[num_agents][units]

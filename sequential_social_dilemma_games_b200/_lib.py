@@ -26,7 +26,8 @@ SYMBOLS = ("ssd_last_error", "ssd_abi_version", "ssd_create", "ssd_destroy", "ss
            "ssd_policy_create", "ssd_policy_features", "ssd_policy_destroy", "ssd_policy_lstm_cell",
            "ssd_policy_set_head", "ssd_policy_lstm_heads", "ssd_policy_create_n", "ssd_policy_set_head_n",
            "ssd_policy_create_pool", "ssd_policy_pool_features", "ssd_policy_pool_lstm_heads", "ssd_policy_lstm_heads_dist",
-           "ssd_policy_pool_lstm_heads_dist", "ssd_moa_create", "ssd_moa_destroy", "ssd_moa_step")
+           "ssd_policy_pool_lstm_heads_dist", "ssd_moa_create", "ssd_moa_destroy", "ssd_moa_step", "ssd_moa_create_pool",
+           "ssd_moa_pool_step")
 
 
 class SsdConfig(C.Structure):
@@ -103,6 +104,8 @@ def _load():
         "ssd_moa_create": (i32, [i32, i32, i32, i32] + [vp] * 5 + [C.POINTER(vp)]),
         "ssd_moa_destroy": (None, [vp]),
         "ssd_moa_step": (i32, [vp] * 12 + [i64, i32, C.c_float, vp]),
+        "ssd_moa_create_pool": (i32, [i32, i32, i32, i32] + [vp] * 5 + [C.POINTER(vp)]),
+        "ssd_moa_pool_step": (i32, [vp] * 13 + [i64, i32, C.c_float, vp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)

@@ -11,8 +11,9 @@
 // or set policy_ids[m] for agent m (a policy pool; agents grouped by ssd::policy_pool::assign).
 enum class WeightMap { Shared, PerAgent, Pool };
 
-// What made a handle: ssd_policy_create[_n] (Net), ssd_policy_create_pool (Pool) or ssd_moa_create (Moa).
-enum class HandleKind { Net, Pool, Moa };
+// What made a handle: ssd_policy_create[_n] (Net), ssd_policy_create_pool (Pool), ssd_moa_create (Moa) or ssd_moa_create_pool
+// (MoaPool).
+enum class HandleKind { Net, Pool, Moa, MoaPool };
 
 // One tile of a pool's assignment: agents perm[first, first + count), count <= 128, all evaluated with weight set `policy`.
 struct PoolTile {
@@ -28,8 +29,8 @@ struct SsdPolicy {
     uint8_t* d_head_blob = nullptr;  // packed LSTM / head weights (ssd_policy_set_head)
     int units = 0, num_outputs = 0;
     int num_policies = 1;            // weight sets: agent m = b * P + p uses set p (ssd_policy_create_n), or set ids[m] (pool)
-    // Moa: d_head_blob holds the MOA's resident weights, d_moa_rows its one-hot rows and moa_logits_w, num_outputs its A,
-    // moa_agents its N
+    // Moa, MoaPool: d_head_blob holds the MOA's resident weights, d_moa_rows its one-hot rows and moa_logits_w, num_outputs its
+    // A, moa_agents its N
     int moa_agents = 0;
     float* d_moa_rows = nullptr;
     // pool scratch, grown on demand: per-policy counts [256] and cursors [256], the tile count, perm [M], tiles [M / 128 + K]
@@ -68,13 +69,18 @@ int create_trunk(int view_radius, int device, int num_policies, WeightMap map, c
 // Element (n, k) of a [rows x K] B operand in the canonical K-major layout without swizzle (8 x 16-byte core matrices).
 inline int kmajor(int rows, int n, int k) { return ((k >> 3) * rows + n) * 8 + (k & 7); }
 
+// a policy pool or an MOA pool: agents grouped by the policy ids of each call
+inline bool is_pool(const SsdPolicy* p) { return p->kind == HandleKind::Pool || p->kind == HandleKind::MoaPool; }
+
 inline WeightMap weight_map(const SsdPolicy* p) {
-    return p->kind == HandleKind::Pool ? WeightMap::Pool : p->num_policies == 1 ? WeightMap::Shared : WeightMap::PerAgent;
+    return is_pool(p) ? WeightMap::Pool : p->num_policies == 1 ? WeightMap::Shared : WeightMap::PerAgent;
 }
 
-// SSD_OK when p is of kind `want`; else SSD_ERR_INVALID with `msg`, or for a network entry point given an MOA handle `moa_msg`.
+// SSD_OK when p is of kind `want`; else SSD_ERR_INVALID with `msg`, or for a network entry point given an MOA handle `moa_msg`
+// (an MOA pool handle: its own message).
 inline int check_kind(const SsdPolicy* p, HandleKind want, const char* msg, const char* moa_msg = "an MOA handle takes ssd_moa_step") {
     if (p->kind == want) return SSD_OK;
+    if (want == HandleKind::Net && p->kind == HandleKind::MoaPool) msg = "an MOA pool handle takes ssd_moa_pool_step";
     return ssd::set_error(SSD_ERR_INVALID, want == HandleKind::Net && p->kind == HandleKind::Moa ? moa_msg : msg);
 }
 
@@ -117,7 +123,7 @@ struct Grid {
 };
 inline Grid grid(const SsdPolicy* p, long long M) {
     const int np = p->num_policies;
-    if (p->kind == HandleKind::Pool) {
+    if (is_pool(p)) {
         const long long tiles = ssd::policy_pool::max_tiles(M, np);
         const int g = static_cast<int>(tiles < p->sms ? tiles : p->sms);
         return {g, g};

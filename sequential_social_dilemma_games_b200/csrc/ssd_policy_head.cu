@@ -53,43 +53,6 @@ __device__ __forceinline__ uint32_t prologue(uint8_t* smem, const uint8_t* blob,
     return *s_tmem;
 }
 
-// A = fp16([features | h]) of the group's `rem` live rows into `a`, rows past them zero.  agent(r): the feature row of row r;
-// state(r): the offset, in 16-float pieces, of row r's first unit block in the tiled state (block b at + b * 128).  HBM is read
-// in long contiguous runs (features: a 128-byte row per eight lanes; h: the tiled state, 64 bytes per lane, 2 KB per warp -- a
-// thread walking a row-major row in 32-byte steps reached 2.3 TB/s).  All loads before the stores: the compiler keeps a
-// global load below a store through a generic pointer.
-template <class Agent, class State>
-__device__ __forceinline__ void gate_operand(uint8_t* a, const float* __restrict__ feat, const float* h_in, int rem, Agent agent, State state) {
-    const int tid = threadIdx.x;
-    const int seg = tid & 7, r8 = tid >> 3;                  // features: 32 rows per pass, 4 passes, a 128-byte row per eight lanes
-    const int hrow = tid & (GA - 1), hb0 = (tid >> 7) * 4;   // h: thread = (agent, four of the eight 16-unit blocks), 64 bytes per block
-    const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
-    float4 vx[4], vh[4][4];
-#pragma unroll
-    for (int ps = 0; ps < 4; ++ps) {
-        const int row = ps * 32 + r8;
-        vx[ps] = row < rem ? __ldcs(reinterpret_cast<const float4*>(feat + agent(row) * KX) + seg) : z;
-    }
-    const long long hbase = state(hrow);
-#pragma unroll
-    for (int b = 0; b < 4; ++b) {
-        const float4* src = reinterpret_cast<const float4*>(h_in + (hbase + (hb0 + b) * GA) * 16);
-#pragma unroll
-        for (int j = 0; j < 4; ++j) vh[b][j] = hrow < rem ? __ldcs(src + j) : z;
-    }
-#pragma unroll
-    for (int ps = 0; ps < 4; ++ps)   // elements 4 seg .. 4 seg + 3 of the 32 features: half of operand chunk seg / 2
-        *reinterpret_cast<uint2*>(a + (seg >> 1) * (GA * 16) + (ps * 32 + r8) * 16 + (seg & 1) * 8) =
-            make_uint2(pack_h2(vx[ps].x, vx[ps].y), pack_h2(vx[ps].z, vx[ps].w));
-#pragma unroll
-    for (int b = 0; b < 4; ++b)      // units 16 (hb0 + b) .. + 15: operand chunks 4 + 2 (hb0 + b) and the next
-#pragma unroll
-        for (int hf = 0; hf < 2; ++hf)
-            *reinterpret_cast<uint4*>(a + (KX / 8 + 2 * (hb0 + b) + hf) * (GA * 16) + hrow * 16) =
-                make_uint4(pack_h2(vh[b][2 * hf].x, vh[b][2 * hf].y), pack_h2(vh[b][2 * hf].z, vh[b][2 * hf].w),
-                           pack_h2(vh[b][2 * hf + 1].x, vh[b][2 * hf + 1].y), pack_h2(vh[b][2 * hf + 1].z, vh[b][2 * hf + 1].w));
-}
-
 // Shared / PerAgent: the groups of GroupMap (ssd_policy.h); features are read as 128-byte rows P * 128 bytes apart and
 // outputs are written to agent-major rows.  The sampler keys Philox by the agent-major index m in all variants.
 //

@@ -47,12 +47,20 @@ inline long long rows_floats(int n, int a) { return static_cast<long long>(n) * 
 
 // kMap Shared: agent m = a0 + row, own index i = m % N.  PerAgent (P = N): the groups of GroupMap (ssd_policy.h), as the
 // policy head.
+//
+// kMap Pool (ssd_moa_pool_step): as the policy head's pool, a group is one tile of the assignment (ssd_policy_pool.cu), agents
+// perm[first, first + count) of one weight set; CTA c takes tiles [c T / G, (c + 1) T / G) and, when the tile's set differs
+// from the one in shared memory, reloads the resident blob and moves its one-hot rows and moa_logits_w to the tile's set (the
+// tiles are in set order).  Row r is agent m = perm[first + r] (rows past the count have no perm entry and are not live);
+// features are gathered by m, h and c are read and written in the agent-major tiled layout, outputs go to row m.
 template <WeightMap kMap>
 __global__ void __launch_bounds__(kThreads, 1)
 moa_kernel(const float* __restrict__ feat, const int8_t* __restrict__ joint, const float* __restrict__ pol_logits, const float* h_in,
            const float* c_in, float* h_out, float* c_out, float* pred, float* __restrict__ cf, float* __restrict__ ipa, float* __restrict__ infl,
            long long M, int N, int A, const uint8_t* __restrict__ blob, const float* __restrict__ rows, long long rows_stride, int divergence,
-           float clip, int ctas_per_policy) {
+           float clip, int ctas_per_policy, const uint32_t* __restrict__ perm, const PoolTile* __restrict__ tiles,
+           const uint32_t* __restrict__ num_tiles) {
+    constexpr bool kPool = kMap == WeightMap::Pool;
     extern __shared__ __align__(128) uint8_t smem[];
     __shared__ uint32_t s_tmem;
     const int tid = threadIdx.x, warp = tid >> 5;
@@ -60,8 +68,14 @@ moa_kernel(const float* __restrict__ feat, const int8_t* __restrict__ joint, con
     const float* s_bias = reinterpret_cast<const float*>(smem + kOffConst);
     float* ys = reinterpret_cast<float*>(smem + kOffS);   // scratch: column j of thread t at ((j / 4) * kThreads + t) * 4 + j % 4
     const GroupMap<kMap> gm(M, N, ctas_per_policy);
-    blob += static_cast<long long>(gm.pol) * kBlobBytes;
-    rows += gm.pol * rows_stride;
+    const long long nt = kPool ? *num_tiles : 0;
+    const long long g_first = kPool ? nt * blockIdx.x / gridDim.x : gm.cta;          // pool: its first tile
+    const long long g_end = kPool ? nt * (blockIdx.x + 1) / gridDim.x : gm.n_groups;  // pool: the end of its tiles
+    const uint8_t* const blob0 = blob;
+    const float* const rows0 = rows;
+    int cur = kPool ? (g_first < g_end ? tiles[g_first].policy : 0) : gm.pol;   // pool: the weight set in shared memory
+    blob += static_cast<long long>(cur) * kBlobBytes;
+    rows += cur * rows_stride;
     const float* wl = rows + static_cast<long long>(N) * A * NG;   // moa_logits_w [128][NJ]
     const int nc = (N - 1) * A;
     if (tid == 0) mbar_init(bar, 1);
@@ -75,11 +89,28 @@ moa_kernel(const float* __restrict__ feat, const int8_t* __restrict__ joint, con
     const uint32_t sA = smem_u32(smem + kOffS), sB = smem_u32(smem + kOffB);
     uint32_t parity = 0;
 
-    for (long long g = gm.cta; g < gm.n_groups; g += gm.stride) {
+    for (long long g = g_first; g < g_end; g += kPool ? 1 : gm.stride) {
         const long long a0 = g * GA, sg = gm.state_group(g);
-        const int rem = static_cast<int>(gm.rows - a0 < GA ? gm.rows - a0 : GA);
-        {   // A = fp16([features | h]), as the policy head.  Built here rather than by the head's builder: with that builder this
-            // kernel's register allocation and instruction order changed and it measured 0.5 % slower.
+        const PoolTile pt = kPool ? tiles[g] : PoolTile{};
+        if (kPool && pt.policy != cur) {   // the previous group is complete (the barrier at the end of the loop)
+            cur = pt.policy;
+            copy_blob(smem, blob0 + static_cast<long long>(cur) * kBlobBytes, kBlobBytes);
+            rows = rows0 + cur * rows_stride;
+            wl = rows + static_cast<long long>(N) * A * NG;
+            fence_async_smem();
+            __syncthreads();
+        }
+        const int rem = kPool ? pt.count : static_cast<int>(gm.rows - a0 < GA ? gm.rows - a0 : GA);
+        if (kPool) {   // pool: the head's builder, rows gathered by perm
+            auto agent = [&](int r) { return static_cast<long long>(perm[pt.first + r]); };
+            auto state = [&](int r) -> long long {
+                if (r >= rem) return 0;   // rows past the tile's count have no perm entry
+                const long long m = agent(r);
+                return (m >> 7) * (U / 16) * GA + (m & (GA - 1));
+            };
+            gate_operand(smem + kOffS, feat, h_in, rem, agent, state);
+        } else {   // A = fp16([features | h]), as the policy head.  Built here rather than by the head's builder: with that builder
+            // this kernel's register allocation and instruction order changed and it measured 0.5 % slower.
             const int seg = tid & 7, r8 = tid >> 3;
             const int hrow = tid & (GA - 1), hb0 = (tid >> 7) * 4;
             const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -119,7 +150,9 @@ moa_kernel(const float* __restrict__ feat, const int8_t* __restrict__ joint, con
         const int r = tid & (GA - 1), half = warp >> 2;
         const uint32_t trow = tmem + (static_cast<uint32_t>((warp & 3) * 32) << 16);
         const bool live = r < rem;
-        const long long m = gm.agent(a0, r), b = m / N;
+        const long long m = kPool ? (live ? static_cast<long long>(perm[pt.first + r]) : 0) : gm.agent(a0, r), b = m / N;
+        // this agent's first 16-float piece of the tiled state, unit block ub at + ub * GA (pool: agent-major)
+        const long long sbase = kPool ? (m >> 7) * (U / 16) * GA + (m & (GA - 1)) : sg * (U / 16) * GA + r;
         const int i = static_cast<int>(m - b * N);
         const int8_t* ja = joint + b * N;
         const int own = live ? ja[i] : 0;
@@ -189,7 +222,7 @@ moa_kernel(const float* __restrict__ feat, const int8_t* __restrict__ joint, con
                 tmem_ld16(trow + U + u0, gf);
                 tmem_ld16(trow + 2 * U + u0, gg);
                 tmem_ld16(trow + 3 * U + u0, go);
-                const long long tile = ((sg * (U / 16) + ub) * GA + r) * 16;
+                const long long tile = kPool ? (sbase + ub * GA) * 16 : ((sg * (U / 16) + ub) * GA + r) * 16;
                 float c[16];
 #pragma unroll
                 for (int e = 0; e < 4; ++e) {
@@ -311,17 +344,13 @@ moa_kernel(const float* __restrict__ feat, const int8_t* __restrict__ joint, con
     if (warp == 0) tmem_free(tmem, 512);
 }
 
-inline auto moa_kernel_for(WeightMap m) { return m == WeightMap::Shared ? moa_kernel<WeightMap::Shared> : moa_kernel<WeightMap::PerAgent>; }
+inline auto moa_kernel_for(WeightMap m) {
+    return m == WeightMap::Shared ? moa_kernel<WeightMap::Shared> : m == WeightMap::PerAgent ? moa_kernel<WeightMap::PerAgent> : moa_kernel<WeightMap::Pool>;
+}
 
-}  // namespace moa
-}  // namespace ssd
-
-#pragma GCC visibility push(default)
-extern "C" {
-
-int ssd_moa_create(int device, int num_policies, int num_agents, int num_actions, const float* lstm_w, const float* lstm_u, const float* lstm_b,
-                   const float* logits_w, const float* logits_b, ssd_moa_t* out) {
-    using namespace ssd::moa;
+// ssd_moa_create[_pool]: `pool` false takes num_policies 1 or N, true 1..255 and allocates the assignment's scratch
+int create(bool pool, int device, int num_policies, int num_agents, int num_actions, const float* lstm_w, const float* lstm_u,
+           const float* lstm_b, const float* logits_w, const float* logits_b, ssd_moa_t* out) {
     if (!out) return ssd::set_error(SSD_ERR_INVALID, "null argument");
     *out = nullptr;
     if (!lstm_w || !lstm_u || !lstm_b || !logits_w || !logits_b) return ssd::set_error(SSD_ERR_INVALID, "null weight pointer");
@@ -329,7 +358,9 @@ int ssd_moa_create(int device, int num_policies, int num_agents, int num_actions
     if (n < 2 || n > SSD_MAX_AGENTS) return ssd::set_error(SSD_ERR_INVALID, "the MOA needs 2..SSD_MAX_AGENTS agents");
     if (na < 1 || na > AMAX) return ssd::set_error(SSD_ERR_INVALID, "num_actions must be 1..15");
     if ((n - 1) * na > NJ) return ssd::set_error(SSD_ERR_INVALID, "(num_agents - 1) * num_actions must be at most 64");
-    if (num_policies != 1 && num_policies != n) return ssd::set_error(SSD_ERR_INVALID, "num_policies must be 1 or num_agents");
+    if (pool && (num_policies < 1 || num_policies > ssd::policy_pool::kBins - 1))
+        return ssd::set_error(SSD_ERR_INVALID, "an MOA pool holds 1..255 weight sets");
+    if (!pool && num_policies != 1 && num_policies != n) return ssd::set_error(SSD_ERR_INVALID, "num_policies must be 1 or num_agents");
     const int kin = KX + n * na, nc = (n - 1) * na;
     const long long rf = rows_floats(n, na);
     std::vector<uint8_t> blobs(static_cast<size_t>(num_policies) * kBlobBytes, 0);
@@ -351,15 +382,18 @@ int ssd_moa_create(int device, int num_policies, int num_agents, int num_actions
     if (!p) return ssd::set_error(SSD_ERR_INVALID, "out of host memory");
     p->device = device;
     p->num_policies = num_policies;
-    p->kind = HandleKind::Moa;
+    p->kind = pool ? HandleKind::MoaPool : HandleKind::Moa;
     p->moa_agents = n;
     p->num_outputs = na;
+    using ssd::policy_pool::kCountWords;
     cudaError_t e = cudaSetDevice(device);
     if (e == cudaSuccess) e = cudaDeviceGetAttribute(&p->sms, cudaDevAttrMultiProcessorCount, device);
     if (e == cudaSuccess) e = cudaMalloc(&p->d_head_blob, blobs.size());
     if (e == cudaSuccess) e = cudaMemcpyAsync(p->d_head_blob, blobs.data(), blobs.size(), cudaMemcpyHostToDevice, 0);
     if (e == cudaSuccess) e = cudaMalloc(&p->d_moa_rows, rows.size() * sizeof(float));
     if (e == cudaSuccess) e = cudaMemcpyAsync(p->d_moa_rows, rows.data(), rows.size() * sizeof(float), cudaMemcpyHostToDevice, 0);
+    if (e == cudaSuccess && pool) e = cudaMalloc(&p->d_counts, kCountWords * sizeof(uint32_t));
+    if (e == cudaSuccess && pool) e = cudaMemsetAsync(p->d_counts, 0, kCountWords * sizeof(uint32_t), 0);   // the assignment's counts start at zero
     if (e == cudaSuccess) e = cudaStreamSynchronize(0);   // the host staging buffers go out of scope
     if (e == cudaSuccess) e = cudaFuncSetAttribute(moa_kernel_for(ssd::policy::weight_map(p)), cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
     if (e != cudaSuccess) {
@@ -370,17 +404,18 @@ int ssd_moa_create(int device, int num_policies, int num_agents, int num_actions
     return SSD_OK;
 }
 
-void ssd_moa_destroy(ssd_moa_t p) { ssd_policy_destroy(p); }
-
-int ssd_moa_step(ssd_moa_t p, const float* features, const int8_t* joint_actions, const float* policy_logits, const float* h_in, const float* c_in,
-                 float* h_out, float* c_out, float* pred, float* counterfactual, float* influence_per_agent, float* influence, int64_t num_agents,
-                 int divergence, float clip, void* stream) {
-    using namespace ssd::moa;
+// ssd_moa_[pool_]step: policy_ids is null for a plain MOA handle
+int step(ssd_moa_t p, const float* features, const uint8_t* policy_ids, const int8_t* joint_actions, const float* policy_logits, const float* h_in,
+         const float* c_in, float* h_out, float* c_out, float* pred, float* counterfactual, float* influence_per_agent, float* influence,
+         int64_t num_agents, int divergence, float clip, void* stream) {
     using namespace ssd::policy;
+    const bool pool = policy_ids != nullptr;
     if (!p || !features || !joint_actions || !policy_logits || !h_in || !c_in || !h_out || !c_out || !pred || !influence_per_agent || !influence ||
         num_agents < 0)
         return ssd::set_error(SSD_ERR_INVALID, "bad argument");
-    int rc = check_kind(p, HandleKind::Moa, "not an MOA handle (ssd_moa_create)");
+    int rc = pool ? check_kind(p, HandleKind::MoaPool, "not an MOA pool handle (ssd_moa_create_pool)")
+                  : check_kind(p, HandleKind::Moa, p->kind == HandleKind::MoaPool ? "an MOA pool handle takes ssd_moa_pool_step"
+                                                                                   : "not an MOA handle (ssd_moa_create)");
     if (rc != SSD_OK) return rc;
     if (divergence != SSD_DIV_KL && divergence != SSD_DIV_JSD) return ssd::set_error(SSD_ERR_INVALID, "divergence must be SSD_DIV_KL or SSD_DIV_JSD");
     if (!(clip >= 0.f)) return ssd::set_error(SSD_ERR_INVALID, "clip must be >= 0 (+inf: no clamp), not NaN");
@@ -390,13 +425,47 @@ int ssd_moa_step(ssd_moa_t p, const float* features, const int8_t* joint_actions
     const int n = p->moa_agents;
     if (num_agents % n != 0) return ssd::set_error(SSD_ERR_INVALID, "num_agents must be a multiple of the MOA's num_agents");
     if (num_agents == 0) return SSD_OK;
-    rc = setup(p, nullptr, num_agents, stream);
+    rc = setup(p, policy_ids, num_agents, stream);
     if (rc != SSD_OK) return rc;
     const Grid g = grid(p, num_agents);
     moa_kernel_for(weight_map(p))<<<g.ctas, kThreads, kSmemBytes, static_cast<cudaStream_t>(stream)>>>(
         features, joint_actions, policy_logits, h_in, c_in, h_out, c_out, pred, counterfactual, influence_per_agent, influence, num_agents, n,
-        p->num_outputs, p->d_head_blob, p->d_moa_rows, rows_floats(n, p->num_outputs), divergence, clip, g.ctas_per_policy);
+        p->num_outputs, p->d_head_blob, p->d_moa_rows, rows_floats(n, p->num_outputs), divergence, clip, g.ctas_per_policy, p->d_perm, p->d_tiles,
+        ssd::policy_pool::num_tiles(p));
     return launched();
+}
+
+}  // namespace moa
+}  // namespace ssd
+
+#pragma GCC visibility push(default)
+extern "C" {
+
+int ssd_moa_create(int device, int num_policies, int num_agents, int num_actions, const float* lstm_w, const float* lstm_u, const float* lstm_b,
+                   const float* logits_w, const float* logits_b, ssd_moa_t* out) {
+    return ssd::moa::create(false, device, num_policies, num_agents, num_actions, lstm_w, lstm_u, lstm_b, logits_w, logits_b, out);
+}
+
+int ssd_moa_create_pool(int device, int num_policies, int num_agents, int num_actions, const float* lstm_w, const float* lstm_u,
+                        const float* lstm_b, const float* logits_w, const float* logits_b, ssd_moa_t* out) {
+    return ssd::moa::create(true, device, num_policies, num_agents, num_actions, lstm_w, lstm_u, lstm_b, logits_w, logits_b, out);
+}
+
+void ssd_moa_destroy(ssd_moa_t p) { ssd_policy_destroy(p); }
+
+int ssd_moa_step(ssd_moa_t p, const float* features, const int8_t* joint_actions, const float* policy_logits, const float* h_in, const float* c_in,
+                 float* h_out, float* c_out, float* pred, float* counterfactual, float* influence_per_agent, float* influence, int64_t num_agents,
+                 int divergence, float clip, void* stream) {
+    return ssd::moa::step(p, features, nullptr, joint_actions, policy_logits, h_in, c_in, h_out, c_out, pred, counterfactual, influence_per_agent,
+                          influence, num_agents, divergence, clip, stream);
+}
+
+int ssd_moa_pool_step(ssd_moa_t p, const float* features, const uint8_t* policy_ids, const int8_t* joint_actions, const float* policy_logits,
+                      const float* h_in, const float* c_in, float* h_out, float* c_out, float* pred, float* counterfactual, float* influence_per_agent,
+                      float* influence, int64_t num_agents, int divergence, float clip, void* stream) {
+    if (!policy_ids) return ssd::set_error(SSD_ERR_INVALID, "bad argument");
+    return ssd::moa::step(p, features, policy_ids, joint_actions, policy_logits, h_in, c_in, h_out, c_out, pred, counterfactual, influence_per_agent,
+                          influence, num_agents, divergence, clip, stream);
 }
 
 }  // extern "C"

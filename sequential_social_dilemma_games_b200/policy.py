@@ -37,7 +37,9 @@ the next state (a `PolicyStep`) -- for a sampled, a greedy or a caller-given act
 
 `MOANet` is the model of other agents of the causal-influence models (train_moa.py): from the trunk features, the joint action
 and the policy's logits it predicts the others' next actions, for the actual and for every counterfactual own action, and
-returns the social-influence reward (`MOAStep`), all in one kernel (`ssd_moa_step`).
+returns the social-influence reward (`MOAStep`), all in one kernel (`ssd_moa_step`).  `MOAPool` is its policy pool: K <= 255
+MOA weight sets and a policy id per agent with every step (`ssd_moa_pool_step`), typically the ids of the PolicyPool call of
+the same step.  `policy_step(..., features=x)` takes the features already computed for the MOA, so the trunk runs once per step.
 """
 import collections
 import ctypes as C
@@ -197,12 +199,16 @@ class _Policy(_Handle):
         """Key of the Philox streams `act` samples from (counter = number of `act` and sampling `policy_step` calls since)."""
         self._sample_seed, self._sample_counter = int(seed) & (2 ** 64 - 1), 0
 
-    def _heads(self, obs, ids, h, c, code=None, given=None, dist=False):
-        """-> PolicyStep of the fused head on the features of obs (ids: the pool's policy ids as `_ids` returns them, None for a
-        network).  dist False: ssd_policy_[pool_]lstm_heads, which samples the actions when code is ACT_SAMPLE and takes none
-        otherwise (logp and entropy None); dist True: ssd_policy_[pool_]lstm_heads_dist in mode `code`, on the `given` actions
-        for ACT_GIVEN.  A sampling call advances the Philox counter."""
-        x = self.features(obs) if ids is None else self.features(obs, ids)
+    def _heads(self, obs, ids, h, c, code=None, given=None, dist=False, features=None):
+        """-> PolicyStep of the fused head on the features of obs, or on `features` (checked by `_given_features`) without running
+        the trunk (ids: the pool's policy ids as `_ids` returns them, None for a network).  dist False:
+        ssd_policy_[pool_]lstm_heads, which samples the actions when code is ACT_SAMPLE and takes none otherwise (logp and entropy
+        None); dist True: ssd_policy_[pool_]lstm_heads_dist in mode `code`, on the `given` actions for ACT_GIVEN.  A sampling call
+        advances the Philox counter."""
+        if features is not None:
+            x = features
+        else:
+            x = self.features(obs) if ids is None else self.features(obs, ids)
         m = x.shape[0]
         self._check_state(h, c, m)
         h, c = _aligned(h), _aligned(c)
@@ -228,6 +234,15 @@ class _Policy(_Handle):
         if code == _lib.ACT_SAMPLE:
             self._sample_counter += 1
         return PolicyStep(a, logp, entropy, logits, value, h_new, c_new)
+
+    def _given_features(self, features, m):
+        """`features` of a policy_step call: None, or float32 [m, 32] on the device (what `features` returns), made aligned."""
+        if features is None:
+            return None
+        if not isinstance(features, torch.Tensor) or features.dtype != torch.float32 or features.device != self.device \
+                or tuple(features.shape) != (m, FEATURES):
+            raise ValueError("features must be a float32 [%d, %d] tensor on %s" % (m, FEATURES, self.device))
+        return _aligned(features)
 
 
 class ConvToFCNet(_Policy):
@@ -354,7 +369,7 @@ class ConvToFCNet(_Policy):
         a = torch.multinomial(torch.softmax(logits, dim=1), 1, generator=generator).squeeze(1).to(torch.int8)
         return a, value, h, c
 
-    def policy_step(self, obs, h, c, mode="sample", actions=None, generator=None):
+    def policy_step(self, obs, h, c, mode="sample", actions=None, generator=None, features=None):
         """-> PolicyStep(actions, logp, entropy, logits, value, h', c') for the M agents of obs; (h, c) as for `forward`.
 
         mode 'sample': the action `act` draws -- the same Philox stream, and the call advances its counter, so `act` and
@@ -362,12 +377,27 @@ class ConvToFCNet(_Policy):
         mode 'greedy': the first argmax of the logits (np.argmax of them where they are finite).  mode 'given': `actions` (integers, M of them) are the caller's, e.g. a
         recorded trajectory or another policy's choice, and are returned as int8; logp is NaN where one is outside 0..A-1.
         logp and entropy are those of softmax(logits), computed from the float32 logits returned: on the fused route in the head
-        kernel itself (ssd_policy_lstm_heads_dist), on the unfused route with torch.log_softmax."""
-        m = obs.numel() // (OBS_SIDE * OBS_SIDE * 3)
+        kernel itself (ssd_policy_lstm_heads_dist), on the unfused route with torch.log_softmax.
+
+        features: float32 [M, 32] on the device, what `features(obs)` returned for these observations (e.g. computed once
+        for an MOANet / MOAPool of the same step).  The trunk is then not run and the head reads them; the result is bitwise that
+        of the call without them.  obs may then be None (M is features.shape[0]); obs that is given is not read.  Fused route
+        only (no `generator`)."""
+        if features is not None:
+            if not isinstance(features, torch.Tensor) or features.dim() != 2:
+                raise ValueError("features must be a float32 [M, %d] tensor on %s" % (FEATURES, self.device))
+            m = features.shape[0]
+            if obs is not None and obs.numel() // (OBS_SIDE * OBS_SIDE * 3) != m:
+                raise ValueError("features has %d rows, obs %d agents" % (m, obs.numel() // (OBS_SIDE * OBS_SIDE * 3)))
+            if not self._fused_head or generator is not None:
+                raise ValueError("features= runs the fused head kernel: cell_size 128, 1..15 outputs and no generator")
+        else:
+            m = obs.numel() // (OBS_SIDE * OBS_SIDE * 3)
+        x = self._given_features(features, m)
         code, given = _step_mode(mode, actions, m, self.num_outputs, self.device)
         if not self._fused_head or (code == _lib.ACT_SAMPLE and generator is not None):
             return _torch_step(*self.forward(obs, h, c), code, given, generator)
-        return self._heads(obs, None, h, c, code, given, dist=True)
+        return self._heads(obs, None, h, c, code, given, dist=True, features=x)
 
 
 class PolicyPool(_Policy):
@@ -446,14 +476,25 @@ class PolicyPool(_Policy):
         logits, value, h, c, a = self._run(obs, policy_ids, h, c, sample=True)
         return a, value, h, c
 
-    def policy_step(self, obs, policy_ids, h, c, mode="sample", actions=None):
+    def policy_step(self, obs, policy_ids, h, c, mode="sample", actions=None, features=None):
         """-> PolicyStep(actions, logp, entropy, logits, value, h', c'), as ConvToFCNet.policy_step on the pool's kernels:
         'sample' draws what `act` draws and advances the same counter, 'greedy' takes the first argmax of the logits, 'given'
         scores the caller's `actions` (returned as int8).  Skipped agents (id >= K) get action -1 in 'sample' and 'greedy'; their
-        rows of logp and entropy, like those of logits, value, h' and c', are not written."""
-        obs, ids = self._ids(obs, policy_ids)
+        rows of logp and entropy, like those of logits, value, h' and c', are not written.
+
+        features: float32 [M, 32] on the device, what `features(obs, policy_ids)` returned (e.g. computed once for an MOAPool
+        of the same step).  The trunk is then not run; the head still groups the agents by `policy_ids` itself, and the result is
+        bitwise that of the call without features.  obs may then be None (policy_ids is a uint8 tensor of M elements on the
+        device); obs that is given is checked against policy_ids but not read."""
+        if features is None or obs is not None:
+            obs, ids = self._ids(obs, policy_ids)
+        else:
+            if not isinstance(policy_ids, torch.Tensor) or policy_ids.dtype != torch.uint8 or policy_ids.device != self.device:
+                raise ValueError("policy_ids must be a uint8 tensor on %s" % (self.device,))
+            ids = policy_ids.contiguous()
+        x = self._given_features(features, ids.numel())
         code, given = _step_mode(mode, actions, ids.numel(), self.num_outputs, self.device)
-        return self._heads(obs, ids, h, c, code, given, dist=True)
+        return self._heads(obs, ids, h, c, code, given, dist=True, features=x)
 
 
 MOAStep = collections.namedtuple("MOAStep", "pred influence influence_per_agent h c counterfactual")
@@ -486,11 +527,17 @@ class MOANet(_Handle):
     _destroy = "ssd_moa_destroy"
 
     def __init__(self, weights, num_agents, device="cuda:0"):
-        self.device = _cuda_device(device)
         sets = list(weights) if isinstance(weights, (list, tuple)) else [weights]
-        n = self.num_agents = int(num_agents)
+        n = int(num_agents)
         if len(sets) not in (1, n):
             raise ValueError("weights is one dict or a list of num_agents = %d dicts, not %d" % (n, len(sets)))
+        self._create(sets, n, device, _lib.lib.ssd_moa_create)
+        self._state_sets = self.num_policies   # the tiled state is grouped per weight set
+
+    def _create(self, sets, n, device, create):
+        """Checks the weight sets' names and shapes and loads them with `create` (ssd_moa_create[_pool])."""
+        self.device = _cuda_device(device)
+        self.num_agents = n
         sets = [{k: np.ascontiguousarray(ws[k], dtype=np.float32) for k in
                  ("moa_lstm_w", "moa_lstm_u", "moa_lstm_b", "moa_logits_w", "moa_logits_b")} for ws in sets]
         w = sets[0]
@@ -509,11 +556,11 @@ class MOANet(_Handle):
         w = {k: np.ascontiguousarray(np.stack([ws[k] for ws in sets])) for k in w}   # P consecutive arrays behind every pointer
         ptr = lambda a: a.ctypes.data_as(C.c_void_p)
         self._h = C.c_void_p()
-        _lib.check(_lib.lib.ssd_moa_create(self.device.index, P, n, A, ptr(w["moa_lstm_w"]), ptr(w["moa_lstm_u"]), ptr(w["moa_lstm_b"]),
-                                           ptr(w["moa_logits_w"]), ptr(w["moa_logits_b"]), C.byref(self._h)))
+        _lib.check(create(self.device.index, P, n, A, ptr(w["moa_lstm_w"]), ptr(w["moa_lstm_u"]), ptr(w["moa_lstm_b"]),
+                          ptr(w["moa_logits_w"]), ptr(w["moa_logits_b"]), C.byref(self._h)))
 
     def _groups(self, m):
-        n, P = self.num_agents, self.num_policies
+        n, P = self.num_agents, self._state_sets
         if m % n:
             raise ValueError("%d agents are not a whole number of envs of %d agents" % (m, n))
         return P * ((m // P + 127) // 128)
@@ -526,12 +573,12 @@ class MOANet(_Handle):
     def state_rows(self, state, m):
         """Tiled state -> agent-major [m, 128] (a copy)."""
         self._groups(m)
-        return _state_rows(state, m, self.num_policies)
+        return _state_rows(state, m, self._state_sets)
 
     def state_from_rows(self, rows):
         """Agent-major [m, 128] -> tiled state, zero padded."""
         self._groups(rows.shape[0])
-        return _state_from_rows(rows, self.num_policies)
+        return _state_from_rows(rows, self._state_sets)
 
     def step(self, features, joint_actions, policy_logits, h, c, divergence="kl", clip=float("inf"), counterfactuals=False):
         """-> MOAStep for the M agents of features [M, 32] (float32, ConvToFCNet.features of the step's observations).
@@ -540,6 +587,10 @@ class MOANet(_Handle):
         0..A-1 is a zero one-hot input and makes influence NaN for every agent of its env.  policy_logits [M, A]: the policy's
         logits of that step (PolicyStep.logits).  divergence 'kl' or 'jsd'; influence = clamp(sum over the others, -clip, clip).
         counterfactuals=True also returns the [M, A, N-1, A] logits of every own action."""
+        return self._step(features, None, joint_actions, policy_logits, h, c, divergence, clip, counterfactuals)
+
+    def _step(self, features, ids, joint_actions, policy_logits, h, c, divergence, clip, counterfactuals):
+        """ssd_moa_step, or ssd_moa_pool_step on `ids` (None: the former)."""
         if divergence not in _DIVERGENCES:
             raise ValueError("divergence must be 'kl' or 'jsd', not %r" % (divergence,))
         clip = float(clip)
@@ -552,6 +603,9 @@ class MOANet(_Handle):
         m = features.shape[0]
         g = self._groups(m)
         _, given = _step_mode("given", joint_actions, m, A, self.device)
+        if ids is not None and (not isinstance(ids, torch.Tensor) or ids.dtype != torch.uint8 or ids.device != self.device
+                                or tuple(ids.shape) not in ((m,), (m // n, n))):
+            raise ValueError("policy_ids must be a uint8 tensor of shape [%d, %d] or [%d] on %s" % (m // n, n, m, self.device))
         if not isinstance(policy_logits, torch.Tensor) or policy_logits.dtype != torch.float32 or policy_logits.device != self.device \
                 or tuple(policy_logits.shape) != (m, A):
             raise ValueError("policy_logits must be a float32 [%d, %d] tensor on %s" % (m, A, self.device))
@@ -564,6 +618,34 @@ class MOANet(_Handle):
         ipa = torch.empty((m, n - 1), dtype=torch.float32, device=self.device)
         infl = torch.empty((m,), dtype=torch.float32, device=self.device)
         p = lambda t: C.c_void_p(t.data_ptr() if t is not None else None)
-        _lib.check(_lib.lib.ssd_moa_step(self._h, p(x), p(given), p(pl), p(h), p(c), p(h_new), p(c_new), p(pred), p(cf), p(ipa), p(infl), m,
-                                         _DIVERGENCES[divergence], clip, self._stream()))
+        io = (p(pl), p(h), p(c), p(h_new), p(c_new), p(pred), p(cf), p(ipa), p(infl), m, _DIVERGENCES[divergence], clip, self._stream())
+        if ids is None:
+            _lib.check(_lib.lib.ssd_moa_step(self._h, p(x), p(given), *io))
+        else:
+            _lib.check(_lib.lib.ssd_moa_pool_step(self._h, p(x), p(ids.contiguous()), p(given), *io))
         return MOAStep(pred, infl, ipa, h_new, c_new, cf)
+
+
+class MOAPool(MOANet):
+    """K MOA weight sets (1 <= K <= 255, each a dict as for MOANet) loaded once; every `step` takes `policy_ids`, a uint8
+    tensor on the device of M elements ([B, N] or [M], agent-major): agent m is evaluated with weight_sets[policy_ids[m]], and
+    the ids may differ from call to call -- typically the tensor the PolicyPool call of the same step took (K seeds of an MOA
+    experiment on one GPU, cross-play teams).  An id >= K means "no MOA for this agent": nothing is written for it (its rows
+    of pred, influence, influence_per_agent, counterfactual, h' and c' are left as they were in the output buffers, which
+    `step` allocates uninitialised) and its row of policy_logits is not read; its action still enters the other agents'
+    inputs, and an action outside 0..A-1 still makes influence NaN for its whole env.  The recurrent state is the shared
+    network's tiled layout [ceil(M/128), 8, 128, 16], independent of the ids; an agent that was skipped wants a fresh state row
+    (state_from_rows) before it returns to a pool MOA.  The id values are checked on the device only.  Calls on one MOA pool
+    must be ordered on one stream: the grouping of the agents by id uses scratch that belongs to the pool."""
+
+    def __init__(self, weight_sets, num_agents, device="cuda:0"):
+        sets = list(weight_sets) if isinstance(weight_sets, (list, tuple)) else [weight_sets]
+        if not sets:
+            raise ValueError("no weight sets")
+        self._create(sets, int(num_agents), device, _lib.lib.ssd_moa_create_pool)
+        self._state_sets = 1   # agent-major, whatever the ids
+
+    def step(self, features, policy_ids, joint_actions, policy_logits, h, c, divergence="kl", clip=float("inf"), counterfactuals=False):
+        """-> MOAStep as MOANet.step, agent m evaluated with weight set policy_ids[m] (ssd_moa_pool_step); rows of skipped agents
+        (id >= K) are not written."""
+        return self._step(features, policy_ids, joint_actions, policy_logits, h, c, divergence, clip, counterfactuals)
