@@ -19,7 +19,13 @@ pytestmark = pytest.mark.gpu
 
 MOA_TOL = FWD_TOL
 OWN_TOL = 1e-5   # influence vs float64 recomputed from the kernel's own logits (accurate expf / logf in fp32)
-CASES = [(2, 8), (5, 8), (5, 9), (8, 8), (9, 8)]
+# every shape class of the kernel (N = 2..16, A = 1..15, (N - 1) A <= 64)
+SHAPE_CLASSES = [(2, 1), (16, 1),           # A = 1: no counterfactual drain on warps 4-7, the influence is exactly 0
+                 (2, 15), (5, 15),          # A >= 10
+                 (16, 4), (13, 5),          # N >= 10: the pass-0 loop over the others runs past 8
+                 (2, 9), (4, 3), (3, 7),    # (N - 1) A not a multiple of 4: a partial last column block of moa_logits_w
+                 (8, 9)]                    # (N - 1) A = 63
+CASES = [(2, 8), (5, 8), (5, 9), (8, 8), (9, 8)] + SHAPE_CLASSES
 
 
 def _policy():
@@ -93,7 +99,11 @@ def test_against_float64_oracle(n, a, kind):
                                      ("influence", s.influence, ref["influence"], tol_infl)):
             err = np.abs(_np(got) - want).max()
             assert err < tol, (t, name, err)
-        assert np.abs(ref["influence"]).max() > 1e-3 and np.abs(ref["pred"]).max() > 0.1   # not vacuous
+        assert np.abs(ref["pred"]).max() > 0.1   # not vacuous
+        if a == 1:   # one action: every softmax is exactly 1, so is every marginal
+            assert bool((s.influence == 0).all()) and bool((s.influence_per_agent == 0).all())
+        else:
+            assert np.abs(ref["influence"]).max() > 1e-3   # not vacuous
         h, c = s.h, s.c
         hr, cr = ref["h"], ref["c"]
     net.close()
@@ -117,7 +127,7 @@ def test_counterfactual_at_the_actual_action_is_pred(n, a):
 
 
 @pytest.mark.parametrize("divergence", ["kl", "jsd"])
-@pytest.mark.parametrize("n,a", [(2, 8), (5, 9), (9, 8)])
+@pytest.mark.parametrize("n,a", [(2, 8), (5, 9), (9, 8)] + SHAPE_CLASSES)
 def test_influence_against_its_own_logits(n, a, divergence):
     from oracle import moa_ref
     net = _policy().MOANet(_sets(n, a, 1, seed=7), n)
@@ -127,6 +137,10 @@ def test_influence_against_its_own_logits(n, a, divergence):
     ipa, infl = moa_ref.influence_from(_np(s.pred), _np(s.counterfactual), _np(pl), _np(joint).astype(np.int64), a, divergence)
     assert np.abs(_np(s.influence_per_agent) - ipa).max() < OWN_TOL
     assert np.abs(_np(s.influence) - infl).max() < OWN_TOL
+    if a == 1:   # exactly 0; a clip has nothing to act on
+        assert bool((s.influence == 0).all()) and bool((s.influence_per_agent == 0).all())
+        net.close()
+        return
     clip = float(np.float32(np.median(infl)))   # the C ABI takes clip as a float
     s2 = net.step(x, joint, pl, h, c, divergence=divergence, clip=clip, counterfactuals=True)
     _, infl_c = moa_ref.influence_from(_np(s2.pred), _np(s2.counterfactual), _np(pl), _np(joint).astype(np.int64), a, divergence, clip)
@@ -134,6 +148,56 @@ def test_influence_against_its_own_logits(n, a, divergence):
     assert float(s2.influence.max()) <= clip and (infl > clip).any()
     if divergence == "jsd":
         assert float(s.influence_per_agent.max()) <= math.log(2) + 1e-6
+    net.close()
+
+
+@pytest.mark.parametrize("divergence", ["kl", "jsd"])
+@pytest.mark.parametrize("n,a", [(5, 8), (3, 7)])
+def test_sharp_distributions(n, a, divergence):
+    """Trained models are sharper than random init.  Own-action rows x 16 (twice the x 8 of _weights), moa_logits_w x 6 (MOA
+    logits up to about +-7 on these inputs) and policy logits 6 randn (pi nearly one-hot for many agents); every 7th agent
+    took an action of probability ~e^-30.  Every output is finite; the influence matches float64 from the kernel's own logits within
+    OWN_TOL (1 + |v|); a JSD term is at most log 2.  pred and the counterfactual logits are compared with the oracle at 6 MOA_TOL:
+    the error of h' (MOA_TOL, as the own-action rows enter in fp32 and the gate GEMM's operands are unchanged) reaches the logits
+    through moa_logits_w, which is 6 times random init; h' and c' themselves at MOA_TOL."""
+    from oracle import moa_ref
+    policy = _policy()
+    b = 300
+    m = b * n
+    w = policy.random_moa_weights(n, a, seed=60 + a)
+    w["moa_lstm_w"][32:32 + a] *= 16.0
+    w["moa_logits_w"] *= 6.0
+    net = policy.MOANet(w, n)
+    x, joint, _ = _inputs(b, n, a, seed=61, steps=1)[0]
+    g = torch.Generator(device="cuda").manual_seed(62)
+    pl = 6.0 * torch.randn((m, a), device="cuda", generator=g)
+    rare = torch.arange(0, m, 7, device="cuda")
+    own = joint.reshape(-1).long()
+    pl[rare, own[rare]] = pl[rare].scatter(1, own[rare, None], -math.inf).max(dim=1).values - 30.0   # pi(own action) ~ e^-30
+    hr = 0.5 * torch.randn((m, 128), device="cuda", generator=g)
+    cr = 0.5 * torch.randn((m, 128), device="cuda", generator=g)
+    h, c = net.state_from_rows(hr), net.state_from_rows(cr)
+    s = net.step(x, joint, pl, h, c, divergence=divergence, counterfactuals=True)
+    for name, t in (("pred", s.pred), ("influence", s.influence), ("influence_per_agent", s.influence_per_agent),
+                    ("h", net.state_rows(s.h, m)), ("c", net.state_rows(s.c, m)), ("counterfactual", s.counterfactual)):
+        assert bool(torch.isfinite(t).all()), name   # the state as agent rows: the tiled layout's padding rows are not written
+    jn = _np(joint).astype(np.int64)
+    ref = moa_ref.moa_forward(w, _np(x), jn, _np(pl), _np(hr), _np(cr), a, divergence=divergence)
+    assert np.abs(ref["pred"]).max() > 5.0   # sharp: MOA logits of about +-7, softmax probabilities down to ~e^-14
+    lp = torch.log_softmax(pl.double(), dim=1).gather(1, own[:, None])[:, 0]
+    assert float(lp[rare].max()) < -29.0   # rare actions
+    assert float((torch.softmax(pl.double(), dim=1).max(dim=1).values > 0.99).double().mean()) > 0.15   # near one-hot policies
+    for name, got, tol in (("pred", s.pred, 6 * MOA_TOL), ("counterfactual", s.counterfactual, 6 * MOA_TOL),
+                           ("h", net.state_rows(s.h, m), MOA_TOL), ("c", net.state_rows(s.c, m), MOA_TOL)):
+        err = np.abs(_np(got) - ref[name]).max()
+        assert err < tol, (name, err)
+    ipa, infl = moa_ref.influence_from(_np(s.pred), _np(s.counterfactual), _np(pl), jn, a, divergence)
+    for name, got, want in (("influence_per_agent", s.influence_per_agent, ipa), ("influence", s.influence, infl)):
+        err = (np.abs(_np(got) - want) / (1 + np.abs(want))).max()
+        assert err < OWN_TOL, (name, err)
+    if divergence == "jsd":
+        assert float(s.influence_per_agent.max()) <= math.log(2) + 1e-6
+    assert infl.max() > 0.1   # not vacuous
     net.close()
 
 
@@ -186,11 +250,13 @@ def test_per_agent_against_shared():
         net.close()
 
 
-@pytest.mark.parametrize("kind", ["shared", "per_agent"])
-def test_scale_equals_one_group_per_cta_calls(kind):
+@pytest.mark.parametrize("kind,n,a", [pytest.param("shared", 5, 8, id="shared"), pytest.param("per_agent", 5, 8, id="per_agent"),
+                                      pytest.param("shared", 16, 4, id="shared-16-4"), pytest.param("per_agent", 16, 4, id="per_agent-16-4"),
+                                      pytest.param("shared", 5, 15, id="shared-5-15"), pytest.param("per_agent", 5, 15, id="per_agent-5-15")])
+def test_scale_equals_one_group_per_cta_calls(kind, n, a):
     """At least four groups per CTA plus a ragged tail, against calls that each run at most one group per CTA."""
     policy = _policy()
-    n, a, sms = 5, 8, _sms()
+    sms = _sms()
     per_policy = kind == "per_agent"
     ctas = sms // n if per_policy else sms
     rows = 4 * ctas * 128 + 77                     # agents per weight set
@@ -220,29 +286,36 @@ def test_scale_equals_one_group_per_cta_calls(kind):
 
 
 def test_invalid_actions():
+    """Envs 3, 7, 150 and 299 have one action -1, A, 127 or -128; the agent that took it has an invalid own action, whose extra
+    drain (a' = A) runs on warps 0-3 for even A and on warps 4-7 for odd A: (N, A) = (5, 8), (5, 15) and (3, 7)."""
+    for n, a in ((5, 8), (5, 15), (3, 7)):
+        _check_invalid_actions(n, a)
+
+
+def _check_invalid_actions(n, a):
     policy = _policy()
-    n, a, b = 5, 8, 300
+    b = 300
     m = b * n
     w = policy.random_moa_weights(n, a, seed=40)
     net = policy.MOANet(w, n)
     x, joint, pl = _inputs(b, n, a, seed=41, steps=1)[0]
-    joint[3, 0], joint[7, 2], joint[150, 4], joint[299, 1] = -1, a, 127, -128
+    joint[3, 0], joint[7, 2 % n], joint[150, 4 % n], joint[299, 1] = -1, a, 127, -128
     bad = torch.zeros(b, dtype=torch.bool, device="cuda")
     bad[[3, 7, 150, 299]] = True
     bad = bad.repeat_interleave(n)
     h, c = net.initial_state(m)
     s = net.step(x, joint, pl, h, c, counterfactuals=True)
-    assert bool(torch.isnan(s.influence[bad]).all()) and bool(torch.isnan(s.influence_per_agent[bad]).all())
-    assert bool(torch.isfinite(s.influence[~bad]).all()) and bool(torch.isfinite(s.influence_per_agent[~bad]).all())
+    assert bool(torch.isnan(s.influence[bad]).all()) and bool(torch.isnan(s.influence_per_agent[bad]).all()), (n, a)
+    assert bool(torch.isfinite(s.influence[~bad]).all()) and bool(torch.isfinite(s.influence_per_agent[~bad]).all()), (n, a)
     ref = _oracle_rows([w], n, _np(x), _np(joint).astype(np.int64), _np(pl), np.zeros((m, 128)), np.zeros((m, 128)), a)
-    assert np.abs(_np(s.pred) - ref["pred"]).max() < MOA_TOL
-    assert np.abs(_np(net.state_rows(s.h, m)) - ref["h"]).max() < MOA_TOL
-    assert np.abs(_np(net.state_rows(s.c, m)) - ref["c"]).max() < MOA_TOL
+    for name, got in (("pred", s.pred), ("h", net.state_rows(s.h, m)), ("c", net.state_rows(s.c, m))):
+        err = np.abs(_np(got) - ref[name]).max()
+        assert err < MOA_TOL, (n, a, name, err)
     # wider integer dtypes are narrowed without wrapping: 136 is not action 8 - 128 + ...; -200 is not valid
     wide = joint.long()
     wide[3, 0], wide[7, 2] = 136, -200
     s2 = net.step(x, wide, pl, h, c)
-    assert bool(torch.isnan(s2.influence[bad]).all()) and torch.equal(s2.influence[~bad], s.influence[~bad])
+    assert bool(torch.isnan(s2.influence[bad]).all()) and torch.equal(s2.influence[~bad], s.influence[~bad]), (n, a)
     net.close()
 
 

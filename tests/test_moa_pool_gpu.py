@@ -237,11 +237,12 @@ def test_skipped_agents_are_not_written():
 
 
 @pytest.mark.parametrize("divergence,clip", [("kl", math.inf), ("jsd", math.inf), ("kl", 0.02)])
-@pytest.mark.parametrize("a", [8, 9])
-def test_matches_float64_oracle(a, divergence, clip):
+@pytest.mark.parametrize("n,a", [pytest.param(5, 8, id="8"), pytest.param(5, 9, id="9"),
+                                 (2, 1), (16, 4), (2, 9), (5, 15)])   # A = 1, N >= 10, (N - 1) A % 4 != 0, A >= 10
+def test_matches_float64_oracle(n, a, divergence, clip):
     from oracle import moa_ref
     policy = _policy()
-    n, B, K = 5, 157, 3
+    B, K = 157, 3
     m = B * n
     sets = _sets(n, a, K, seed=90 + a)
     pool = policy.MOAPool(sets, n)
@@ -261,7 +262,10 @@ def test_matches_float64_oracle(a, divergence, clip):
                                ("influence", s.influence, tol_infl)):
             err = np.abs(_np(got) - ref[name]).max()
             assert err < tol, (t, name, err)
-        assert np.abs(ref["influence"]).max() > 1e-3   # not vacuous
+        if a == 1:   # one action: the influence is exactly 0
+            assert bool((s.influence == 0).all())
+        else:
+            assert np.abs(ref["influence"]).max() > 1e-3   # not vacuous
         if clip < math.inf:
             assert float(s.influence.max()) <= clip
         h, c, h64, c64 = s.h, s.c, ref["h"], ref["c"]
