@@ -346,6 +346,48 @@ int ssd_moa_pool_step(ssd_moa_t p, const float* features, const uint8_t* policy_
 int ssd_policy_lstm_cell(const void* gates_bf16, const float* bias, const float* c_prev, float* c_out, float* h_out, void* h_bf16_out,
                          int64_t num_agents, int units, void* stream);
 
+/* ---- Advantages and value targets of a trajectory (the rollout worker's postprocess_trajectory) --------------------------------
+ * T >= 1 steps of M = B*N agents, agent-major (m = b*N + n) as everywhere in the library; all arrays dev, time-major [T][M]:
+ *   rewards     [T][M] int32 (SSD_DTYPE_I32, what ssd_step / ssd_rollout write) or float32 (SSD_DTYPE_F32);
+ *   intrinsic   [T][M] f32 or NULL, with intrinsic_weight w: the step reward is r_t = float(rewards_t) + w * intrinsic_t in fp32
+ *               (the curriculum-weighted influence reward of the MOA trainers; the caller aligns it in time);
+ *   values      [T][M] f32, the value predictions (RLlib's vf_preds);
+ *   dones       [T][B] u8: nonzero = the episode of env b ended with step t; agent m reads dones[t][m / num_agents];
+ *   bootstrap   [M] f32: RLlib's last_r, the value of the observation after step T-1.  V_T = bootstrap.
+ * Every mode is the affine recurrence acc_t = x_t + k_t * acc_{t+1}, run backwards in time per agent:
+ *   SSD_ADV_GAE      (compute_advantages, use_gae=True): x_t = (r_t + gamma V_{t+1}) - V_t, k_t = gamma * lambda, acc_T = 0;
+ *                    advantages = acc, value_targets = acc + V_t.
+ *   SSD_ADV_RETURNS  (use_gae=False): x_t = r_t, k_t = gamma, acc_T = bootstrap; advantages = acc (discounted returns).  RLlib
+ *                    writes zeros as value targets; this mode writes none and value_targets must be NULL.
+ *   ssd_vtrace       (from_importance_weights): rho_t = exp(target_logp_t - behaviour_logp_t), rho_bar = min(clip_rho, rho),
+ *                    c = min(1, rho), rho_pg = min(clip_pg_rho, rho); x_t = rho_bar_t ((r_t + gamma V_{t+1}) - V_t), k_t = gamma c_t,
+ *                    acc_T = 0; vs = acc + V_t, pg_advantages = rho_pg_t ((r_t + gamma vs_{t+1}) - V_t) with vs_T = bootstrap.
+ *                    A threshold of +inf disables its clip (None in RLlib).
+ * Episode ends are a select, not a multiply: at a done at t every (t+1) term -- V_{t+1}, acc_{t+1}, vs_{t+1} -- is dropped, not
+ * multiplied by zero, so each episode fragment gets exactly what RLlib computes for it alone with last_r = 0, and nothing of a
+ * later episode (NaN and inf included) or of the bootstrap behind a done at T-1 reaches an earlier one.  Inside an episode a
+ * non-finite input propagates as the arithmetic implies; agents are independent, so garbage in one column (a pool agent whose
+ * value policy_step did not write) affects that column only.  The min of a clip passes a NaN rho on.
+ * All float / int32 arrays 4-byte aligned; outputs [T][M] f32 must not alias an input or each other.  gamma outside [0, 1],
+ * lambda outside [0, 1] in SSD_ADV_GAE (SSD_ADV_RETURNS does not use lambda and accepts any value), a negative or NaN clip
+ * threshold, T or M <= 0, M not a multiple of num_agents, an unknown mode or dtype, a null pointer or a workspace smaller than
+ * ssd_advantages_workspace_bytes(T, M) return SSD_ERR_INVALID before anything is launched.
+ * workspace: dev, 16-byte aligned, of ssd_advantages_workspace_bytes(T, M) bytes (0 -- NULL is fine -- when the call runs one
+ * pass over time); it holds per-chunk carries when the call splits time into chunks to fill the GPU with few agents.  No host
+ * synchronisation and no allocation; runs on `stream` on the current device.  fp32 throughout (accurate expf). */
+#define SSD_ADV_GAE 0
+#define SSD_ADV_RETURNS 1
+#define SSD_DTYPE_I32 0
+#define SSD_DTYPE_F32 1
+int64_t ssd_advantages_workspace_bytes(int64_t T, int64_t M);
+int ssd_advantages(int mode, int64_t T, int64_t M, int num_agents, const void* rewards, int reward_dtype, const float* intrinsic,
+                   float intrinsic_weight, const float* values, const uint8_t* dones, const float* bootstrap, float gamma, float lambda,
+                   float* advantages, float* value_targets, void* workspace, int64_t workspace_bytes, void* stream);
+int ssd_vtrace(int64_t T, int64_t M, int num_agents, const void* rewards, int reward_dtype, const float* intrinsic, float intrinsic_weight,
+               const float* values, const uint8_t* dones, const float* bootstrap, const float* target_logp, const float* behaviour_logp,
+               float gamma, float clip_rho_threshold, float clip_pg_rho_threshold, float* vs, float* pg_advantages, void* workspace,
+               int64_t workspace_bytes, void* stream);
+
 /* Tuning options.
  * SSD_OPT_CHAIN_STEPS (default 0): when 1, consecutive ssd_step calls on the same stream are launched
  * with programmatic dependent launch: the kernel of step t+1 starts filling SMs while the last CTAs of

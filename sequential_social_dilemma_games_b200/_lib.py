@@ -16,6 +16,8 @@ OPT_GENERAL_KERNEL = 2
 PHASE_MOVES, PHASE_CONSUME, PHASE_BEAMS, PHASE_SPAWN, PHASE_RENDER, PHASE_ALL = 1, 2, 4, 8, 16, 31
 ACT_SAMPLE, ACT_GREEDY, ACT_GIVEN = 0, 1, 2
 DIV_KL, DIV_JSD = 0, 1
+ADV_GAE, ADV_RETURNS = 0, 1
+DTYPE_I32, DTYPE_F32 = 0, 1
 
 # every symbol include/ssd_b200.h declares (tests/test_cabi.py checks the list against the header)
 SYMBOLS = ("ssd_last_error", "ssd_abi_version", "ssd_create", "ssd_destroy", "ssd_num_apple_points",
@@ -27,7 +29,7 @@ SYMBOLS = ("ssd_last_error", "ssd_abi_version", "ssd_create", "ssd_destroy", "ss
            "ssd_policy_set_head", "ssd_policy_lstm_heads", "ssd_policy_create_n", "ssd_policy_set_head_n",
            "ssd_policy_create_pool", "ssd_policy_pool_features", "ssd_policy_pool_lstm_heads", "ssd_policy_lstm_heads_dist",
            "ssd_policy_pool_lstm_heads_dist", "ssd_moa_create", "ssd_moa_destroy", "ssd_moa_step", "ssd_moa_create_pool",
-           "ssd_moa_pool_step")
+           "ssd_moa_pool_step", "ssd_advantages_workspace_bytes", "ssd_advantages", "ssd_vtrace")
 
 
 class SsdConfig(C.Structure):
@@ -106,6 +108,10 @@ def _load():
         "ssd_moa_step": (i32, [vp] * 12 + [i64, i32, C.c_float, vp]),
         "ssd_moa_create_pool": (i32, [i32, i32, i32, i32] + [vp] * 5 + [C.POINTER(vp)]),
         "ssd_moa_pool_step": (i32, [vp] * 13 + [i64, i32, C.c_float, vp]),
+        "ssd_advantages_workspace_bytes": (i64, [i64, i64]),
+        "ssd_advantages": (i32, [i32, i64, i64, i32, vp, i32, vp, C.c_float, vp, vp, vp, C.c_float, C.c_float, vp, vp, vp, i64, vp]),
+        "ssd_vtrace": (i32, [i64, i64, i32, vp, i32, vp, C.c_float, vp, vp, vp, vp, vp, C.c_float, C.c_float, C.c_float, vp, vp, vp,
+                             i64, vp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)

@@ -8,7 +8,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libssd_b200.so")
 SOURCES = ["ssd_step_fast.cu", "ssd_step_general.cu", "ssd_aux.cu", "ssd_capi.cu", "ssd_policy.cu", "ssd_policy_head.cu",
-           "ssd_policy_pool.cu", "ssd_policy_moa.cu"]  # compiled in parallel
+           "ssd_policy_pool.cu", "ssd_policy_moa.cu", "ssd_advantages.cu"]  # compiled in parallel
 HEADERS = ["ssd_internal.h", "ssd_device.cuh", "ssd_phases.cuh", "ssd_umma.cuh", "ssd_policy.h", "ssd_policy_lstm.cuh", os.path.join("..", "..", "include", "ssd_b200.h")]
 NVCC_FLAGS = ["-std=c++17", "-O3", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden"]
